@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- 150 bp reads aligned per second through the bwa hot path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c1|c2|c3|c4|c5]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c1|c2|c3|c4|c5] [--dump-outputs DIR]
 
 A step = one pass of the hot path (seed -> chain -> extend -> finalize -> rows in read order with MAPQ) over one batch of
 simulated reads against the resident FM-index.  --config picks a BASELINE.json configuration with BASELINE.md's exact row layout
@@ -76,7 +76,12 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="target CPU seconds of the cpu_baseline sample")
     ap.add_argument("--no-extras", action="store_true", help="skip the tuple / loader / microbenchmark probes after the timed legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the rows of the last timed step (rank 0) to DIR/*.npy for a fixed, seeded sample of reads (dump_sample, "
+                         "dump_outputs); --impl reference writes the oracle's rows for the same reads")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     layout, reads, rlen, err, idx = CONFIGS[args.config]
     args.layout = layout
     args.baseline_index = idx
@@ -239,6 +244,12 @@ def run_reference(args, rank, world):
         r = orc.align_batch(seqs[:int(offs[sample])], offs[:sample + 1], ids[:sample], cores)
         if s >= args.warmup:
             times.append(r["seconds"])
+    if args.dump_outputs:
+        # the timed batch size comes from a timing probe; the dump covers dump_sample's reads, as the GPU arm's does, aligned once more
+        pick = dump_sample(args.reads, args.read_len)
+        lens = (offs[pick + 1] - offs[pick]).astype(np.int64)
+        d = orc.align_batch(seqs[ranges(offs[pick], lens)], np.concatenate(([0], np.cumsum(lens))), ids[pick], cores)
+        dump_outputs(args.dump_outputs, pick, d["row_off"], d["rows"], d["cigar"], at=np.arange(len(pick)))
     total = sum(times)
     value = sample * len(times) / total
     line = {
@@ -254,7 +265,13 @@ def run_reference(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
-# ------------------------------------------------------------------------------------------ our arm
+# ------------------------------------------------------------------------------------------ outputs
+def ranges(starts, counts):
+    """Indices of the concatenated ranges [starts[i], starts[i] + counts[i])."""
+    counts = np.asarray(counts, dtype=np.int64)
+    return np.repeat(np.asarray(starts, dtype=np.int64) - (np.cumsum(counts) - counts), counts) + np.arange(int(counts.sum()), dtype=np.int64)
+
+
 def rows_digest(res):
     """SHA-1 over everything the step produced (row offsets, row fields, CIGAR words): two builds / code paths compare run to run."""
     import hashlib
@@ -266,12 +283,64 @@ def rows_digest(res):
         if name != "cigar_off":            # pool positions depend on the order warps allocate in; the words they point at do not
             dg.update(np.ascontiguousarray(rr[name]).tobytes())
     if total_rows:
-        nc = rr["n_cigar"].astype(np.int64)
-        starts = np.repeat(rr["cigar_off"].astype(np.int64) - np.concatenate(([0], np.cumsum(nc)[:-1])), nc)
-        dg.update(np.ascontiguousarray(res.cigar[starts + np.arange(int(nc.sum()), dtype=np.int64)]).tobytes())
+        dg.update(np.ascontiguousarray(res.cigar[ranges(rr["cigar_off"], rr["n_cigar"])]).tobytes())
     return dg.hexdigest()
 
 
+DUMP_BYTES = 64 << 20
+DUMP_READS = 1 << 16          # sampled 150 bp reads; longer reads are sampled fewer in proportion
+DUMP_SEED = 20261021
+
+
+def dump_sample(n, read_len):
+    """The reads a dump covers, in read order: a seeded choice fixed by the batch size and the read length alone."""
+    k = min(n, max(1, DUMP_READS * 150 // max(read_len, 150)))
+    return np.sort(np.random.Generator(np.random.PCG64(DUMP_SEED)).permutation(n)[:k])
+
+
+def _dump_arrays(read_index, row_off, rows, cigar, at):
+    row_off = np.asarray(row_off, dtype=np.int64)
+    counts = row_off[at + 1] - row_off[at]
+    rr = rows[ranges(row_off[at], counts)]
+    out = {"read_index": read_index.astype(np.float64), "rows_per_read": counts.astype(np.float64)}
+    for name in rr.dtype.names:
+        v = rr[name]
+        if name == "cigar_off":
+            continue
+        if v.dtype.kind in "iu" and v.dtype.itemsize == 8:
+            out["row_%s_hi" % name] = (v >> v.dtype.type(32)).astype(np.float64)
+            out["row_%s_lo" % name] = (v & v.dtype.type(0xFFFFFFFF)).astype(np.float64)
+        else:
+            out["row_" + name] = v.astype(np.float32 if v.dtype.kind == "f" else np.float64)
+    out["cigar"] = np.asarray(cigar)[ranges(rr["cigar_off"], rr["n_cigar"])].astype(np.float64)
+    return out
+
+
+def dump_outputs(out_dir, read_index, row_off, rows, cigar, at=None):
+    """Writes the rows of the reads read_index (from dump_sample) as .npy files in out_dir: read_index, rows_per_read, row_<field> for
+    every row field in read order, and cigar (the CIGAR words of those rows in the same order).  row_off / rows / cigar are a result
+    whose read at[i] (default: read_index[i]) is read read_index[i].  cigar_off is left out for the reason rows_digest gives.  Every
+    array is float64 (frac_rep float32) and exact: each 64-bit integer field goes in two 32-bit halves, row_<field>_hi (signed for a
+    signed field) and row_<field>_lo.  When the arrays would exceed DUMP_BYTES, the longest prefix of the reads that fits is written.
+    Returns the number of bytes written."""
+    at = read_index if at is None else at
+    out = _dump_arrays(read_index, row_off, rows, cigar, at)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_BYTES:
+        counts = out["rows_per_read"].astype(np.int64)
+        words = np.bincount(np.repeat(np.arange(len(counts)), counts), weights=out["row_n_cigar"], minlength=len(counts))
+        row_bytes = sum(a.itemsize for k, a in out.items() if k.startswith("row_"))
+        per_read = 16 + counts * row_bytes + words * 8
+        keep = max(1, int(np.searchsorted(np.cumsum(per_read), DUMP_BYTES, side="right")))
+        out = _dump_arrays(read_index[:keep], row_off, rows, cigar, at[:keep])
+        total = sum(a.nbytes for a in out.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return total
+
+
+# ------------------------------------------------------------------------------------------ our arm
 def run_ours(args, rank, world, local_rank):
     import ctypes as C
     import torch
@@ -352,6 +421,8 @@ def run_ours(args, rank, world, local_rank):
     okk = has & (pr["rid"] == truth[0]) & (pr["is_rev"] == truth[2].astype(np.int32)) & (np.abs(pr["pos"] - truth[1]) <= 16 + args.read_len // 8)
     truth_frac = float(okk.mean())
     digest = rows_digest(res)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dump_sample(n, args.read_len), res.row_off, res.rows, res.cigar)
 
     # ---------------- e2e: host buffers through the C ABI.  The reference-facing form of the call takes the reads as the PG glue holds them
     # (NUCLSEQ datum images, extension.cpp:362) and returns the 64-byte public rows; the ASCII form (bsq_align_batch) is timed beside it.

@@ -2,8 +2,9 @@
 // reference's UNCHANGED sequence.h / sequence.cpp and against the lines of the reference's extension.cpp that use the adapter --
 // bwa_index_from_query (extension.cpp:211-236: BwaIndex returned by value, bwa.options->field writes, build()) and the per-read
 // loop (extension.cpp:362-370: bwa.align_sequence(*nuclseq) on a const-qualified call, rows read field by field).  The excerpt is
-// cut out of /root/reference at test time (tests/test_dropin.py) and #included here as dropin_excerpt.inc: nothing of the
-// reference is stored in this repository.  PostgreSQL is replaced by tests/pg_stub.
+// cut out of the BIOSEQDB_SRC checkout at test time (tests/test_dropin.py) and #included here as dropin_excerpt.inc: nothing of the
+// reference is stored in this repository.  Without a checkout, tests/dropin_src supplies a stand-in for sequence.h, sequence.cpp and
+// the excerpt.  PostgreSQL is replaced by tests/pg_stub.
 #include <algorithm>
 #include <cstdio>
 #include <functional>
