@@ -310,7 +310,6 @@ class BwaIndex:
     def align_tuples_datums(self, data: np.ndarray, off: np.ndarray, ids: np.ndarray | None = None, flags: int = 0):
         """Rows and their materialised columns in one go: bsq_align_batch_datums, then bsq_result_tuples served from the resident batch
         (no re-upload).  Returns (AlignResult, Tuples)."""
-        from ._lib import BsqTuples
         if not getattr(self, "two_chunks", False):
             self.two_chunks = True
             self._apply_flags()
@@ -321,17 +320,8 @@ class BwaIndex:
             ids = np.ascontiguousarray(ids, dtype=np.int64)
         res = C.POINTER(BsqResult)()
         check(self.L.bsq_align_batch_datums(self.h, ptr(data), ptr(off), ptr(ids) if ids is not None else None, n, C.byref(res)))
-        tp = C.POINTER(BsqTuples)()
         try:
-            check(self.L.bsq_result_tuples(self.h, res, None, None, int(flags), C.byref(tp)))
-            t = tp.contents
-            nr = int(t.n_rows)
-            toff = np.ctypeslib.as_array(t.off, shape=(3 * nr + 1,)).copy()
-            ref_match = np.ctypeslib.as_array(t.ref_match, shape=(max(3 * nr, 1),))[:3 * nr].copy().reshape(nr, 3)
-            nb = int(t.n_bytes)
-            tdata = np.ctypeslib.as_array(t.bytes, shape=(max(nb, 1),))[:nb].copy()
-            tup = Tuples(toff, ref_match, tdata, float(t.device_ms))
-            self.L.bsq_tuples_free(tp)
+            tup = self._fetch_tuples(res, None, None, flags)
         except Exception:
             self.L.bsq_result_free(res)
             raise
@@ -360,7 +350,6 @@ class BwaIndex:
     def tuples(self, res: AlignResult, seqs: np.ndarray, offs: np.ndarray, flags: int = 0) -> "Tuples":
         """Row materialisation on the GPU (SURVEY.md 8f-2): for every row of `res` the NUCLSEQ datum images of ref_subseq and
         query_subseq, the CIGAR string and ref_match_* -- what build_tuple_bwa (extension.cpp:282-305) assembles from a BwaMatch."""
-        from ._lib import BsqTuples
         seqs = np.ascontiguousarray(seqs, dtype=np.uint8)
         offs = np.ascontiguousarray(offs, dtype=np.uint64)
         row_off = np.ascontiguousarray(res.row_off, dtype=np.uint64)
@@ -374,8 +363,14 @@ class BwaIndex:
         r.rows = rows.ctypes.data
         r.cigar = cigar.ctypes.data_as(C.POINTER(C.c_uint32))
         r.n_cigar_words = len(cigar)
+        return self._fetch_tuples(C.byref(r), ptr(seqs), ptr(offs), flags)
+
+    def _fetch_tuples(self, res, seqs, offs, flags: int) -> "Tuples":
+        """bsq_result_tuples on `res` (a pointer to a bsq_result; seqs / offs: the reads, or None when the library serves the result
+        from its resident batch), copied out"""
+        from ._lib import BsqTuples
         tp = C.POINTER(BsqTuples)()
-        check(self.L.bsq_result_tuples(self.h, C.byref(r), ptr(seqs), ptr(offs), int(flags), C.byref(tp)))
+        check(self.L.bsq_result_tuples(self.h, res, seqs, offs, int(flags), C.byref(tp)))
         t = tp.contents
         n = int(t.n_rows)
         off = np.ctypeslib.as_array(t.off, shape=(3 * n + 1,)).copy()

@@ -68,12 +68,17 @@ struct Batch {
     DevBuf<uint8_t> ext_scratch, fin_scratch, narrow_z, narrow_jobs; DevBuf<uint64_t> wide_jobs;
     DevBuf<ExtMemo> ext_memo; DevBuf<uint8_t> ext_memo_key; DevBuf<uint32_t> ext_memo_perm, ext_memo_hist, ext_todo, chain_todo, fin_todo, seed_todo, seed_pk, seed_u32;   // thread-per-extension pre-pass (extend_plan.cu)
     DevBuf<uint32_t> ctl;  // [0..3] tickets, [4] overflow, [5] pool_top, [6] cigar_top, [8..23] counters (u64 x 8), [24] narrow_cnt, [25] wide_cnt, [26..27] tickets, [56] reads left for sw_extend, [57] reads left for the warp chain kernel, [58] for regs_finalize
-    size_t device_bytes() const {
-        return seqs.bytes() + offs.bytes() + ids.bytes() + ascii.bytes() + datums.bytes() + datum_off.bytes() + scan_tmp64.bytes() + intv.bytes() + intv_cnt.bytes() + seed_scratch.bytes() + raw.bytes() + seeds.bytes() + ctmp.bytes() +
-               ord.bytes() + chains.bytes() + srt.bytes() + regs.bytes() + rows.bytes() + rows_compact.bytes() + rows_ext.bytes() + reg_cnt.bytes() + row_cnt.bytes() + row_off.bytes() +
-               scan_tmp.bytes() + blocks.bytes() + cigar.bytes() + read_logtab.bytes() + ext_scratch.bytes() + fin_scratch.bytes() + narrow_z.bytes() +
-               narrow_jobs.bytes() + wide_jobs.bytes() + ctl.bytes() + ext_memo.bytes() + ext_memo_key.bytes() + ext_memo_perm.bytes() + ext_memo_hist.bytes() + ext_todo.bytes() + chain_todo.bytes() + fin_todo.bytes() + seed_todo.bytes() + seed_pk.bytes() + seed_u32.bytes();
+    // f(buf) for every DevBuf above: the one list release() frees and device_bytes() counts (BwaIndexCache's eviction budget)
+    template <class B, class F> static void each(B& b, F f) {
+        f(b.seqs); f(b.offs); f(b.ids); f(b.datums); f(b.datum_off); f(b.scan_tmp64); f(b.ascii); f(b.row_off64);
+        f(b.tup_off); f(b.tup_tmp); f(b.tup_row_read); f(b.tup_nholes); f(b.tup_rm); f(b.tup_bytes);
+        f(b.intv); f(b.intv_cnt); f(b.seed_scratch); f(b.raw); f(b.seeds); f(b.ctmp); f(b.ord); f(b.chains); f(b.srt);
+        f(b.regs); f(b.rows); f(b.rows_compact); f(b.rows_ext); f(b.reg_cnt); f(b.row_cnt); f(b.row_off); f(b.scan_tmp); f(b.blocks); f(b.cigar);
+        f(b.read_logtab); f(b.ext_scratch); f(b.fin_scratch); f(b.narrow_z); f(b.narrow_jobs); f(b.wide_jobs);
+        f(b.ext_memo); f(b.ext_memo_key); f(b.ext_memo_perm); f(b.ext_memo_hist); f(b.ext_todo); f(b.chain_todo); f(b.fin_todo); f(b.seed_todo); f(b.seed_pk); f(b.seed_u32);
+        f(b.ctl);
     }
+    size_t device_bytes() const { size_t n = 0; each(*this, [&](const auto& d) { n += d.bytes(); }); return n; }
     bool resident = false, aligned = false;
     // one batch = one lane of the host pipeline: its stream, the host staging that must outlive the async copies,
     // and the state of the attempt in flight (pipeline_enqueue -> pipeline_check)
@@ -81,7 +86,7 @@ struct Batch {
     std::vector<bsq_row_ext> ext_tmp;   // extension records fetched only to finish a MAPQ on the host
     uint32_t* ctl_host = nullptr;       // pinned, 16 words: ctl[0..7], total rows (2 words), host-MAPQ flag
     cudaEvent_t ev[5]; bool ev_ok = false;
-    cudaEvent_t ev_x[5]; bool evx_ok = false;   // chunked mode: upload begin/end, download begin/end, pipeline queued
+    cudaEvent_t ev_x[4]; bool evx_ok = false;   // chunked mode: upload begin/end, download begin/end
     ExtAux ext_aux; bool ext_aux_ok = false;    // side streams of the extension pre-pass
     uint32_t att_rseq_cap = 0; bool idle = true;
     uint64_t out_rows = 0; uint32_t out_cig = 0;
@@ -91,11 +96,7 @@ struct Batch {
         if (ev_ok) { for (auto& e : ev) cudaEventDestroy(e); ev_ok = false; }
         if (evx_ok) { for (auto& e : ev_x) cudaEventDestroy(e); evx_ok = false; }
         if (ext_aux_ok) { for (auto& s_ : ext_aux.st) cudaStreamDestroy(s_); for (auto& e : ext_aux.ev) cudaEventDestroy(e); ext_aux_ok = false; }
-        seqs.release(); offs.release(); ids.release(); ascii.release(); tup_off.release(); tup_tmp.release(); tup_row_read.release(); tup_nholes.release(); tup_rm.release(); tup_bytes.release(); datums.release(); datum_off.release(); scan_tmp64.release(); intv.release(); intv_cnt.release(); seed_scratch.release(); raw.release(); seeds.release();
-        ctmp.release(); ord.release(); chains.release(); srt.release(); regs.release(); rows.release(); rows_compact.release(); rows_ext.release(); reg_cnt.release();
-        row_cnt.release(); row_off.release(); scan_tmp.release(); blocks.release(); cigar.release(); ext_scratch.release(); fin_scratch.release();
-        ctl.release(); narrow_z.release(); narrow_jobs.release(); wide_jobs.release(); read_logtab.release();
-        ext_memo.release(); ext_memo_key.release(); ext_memo_perm.release(); ext_memo_hist.release(); ext_todo.release(); chain_todo.release(); fin_todo.release(); seed_todo.release(); seed_pk.release(); seed_u32.release();
+        each(*this, [](auto& d) { d.release(); });
     }
 };
 
@@ -135,7 +136,9 @@ static void fill_dev_opts(bsq_index* h) {
     o.split_len = (int)(p.min_seed_len * 1.5f + .499);   // (int)(min_seed_len * split_factor + .499), split_factor is a float 1.5
     o.max_chain_gap = 10000; o.max_chain_extend = 1 << 30; o.min_chain_weight = 0;
     o.mask_level = 0.50f; o.drop_ratio = 0.50f; o.mask_level_redun = 0.95f;
-    // bwa_fill_scmat(1, 4): filled once by mem_opt_init and never refreshed (SURVEY.md B#5)
+    // bwa_fill_scmat(1, 4): filled once by mem_opt_init and never refreshed (SURVEY.md B#5).  This is the only matrix DevOpts ever
+    // carries: the register and thread DP kernels (finalize.cu, ksw_thread.cuh) rely on its form -- one match, one mismatch and one
+    // ambiguous-base score.
     for (int i = 0; i < 4; ++i) { for (int j = 0; j < 4; ++j) o.mat[i * 5 + j] = i == j ? 1 : -4; o.mat[i * 5 + 4] = -1; }
     for (int j = 0; j < 5; ++j) o.mat[20 + j] = -1;
     o.mat_max = 1;
@@ -178,10 +181,9 @@ bsq_index* bsq_index_new(const bsq_opts* o, int device) {
     memset(&h->meta, 0, sizeof(h->meta)); memset(&h->timing, 0, sizeof(h->timing));
     fill_dev_opts(h);
     // The main stream (and lane 0 of the chunked pipeline) outranks lane 1: two chunks share the SMs, the earlier one gets free ones
-    // first and is done -- its result on the way to the host -- while the later one still computes.  BSQ_NO_STREAM_PRIO: equal ranks.
+    // first and is done -- its result on the way to the host -- while the later one still computes.
     int prio_lo = 0, prio_hi = 0;
     cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);
-    if (getenv("BSQ_NO_STREAM_PRIO")) prio_hi = prio_lo;
     h->prio_hi = prio_hi; h->prio_lo = prio_lo;
     if (cudaStreamCreateWithPriority(&h->stream, cudaStreamNonBlocking, prio_hi) != cudaSuccess) { bsq_set_error("cudaStreamCreate failed"); delete h; return nullptr; }
     h->batch.st = h->stream;
@@ -721,12 +723,12 @@ int upload_datums(bsq_index* h, Batch& b, const uint8_t* bytes, const uint64_t* 
 // k-mer table of the LAST-like seeding pass: built once per device index (also after a broadcast replica)
 int ensure_kmer_table(bsq_index* h, const DevIndex& ix) {
     if (ix.seq_len >= (1ull << 40)) return BSQ_OK;   // the table packs rows in 40 bits
-    if (!h->d_isa && !getenv("BSQ_NO_ISA")) {
+    if (!h->d_isa) {
         CUDA_CHECK(cudaMalloc(&h->d_isa, (ix.seq_len + 1) * (uint64_t)ix.sa_bytes + 64));
         build_isa(ix, h->d_isa, h->stream, &h->timing.launches);
         CUDA_CHECK(cudaStreamSynchronize(h->stream));
     }
-    if (h->d_kmer || ix.seq_len < (1u << 16) || getenv("BSQ_NO_KMER")) return BSQ_OK;
+    if (h->d_kmer || ix.seq_len < (1u << 16)) return BSQ_OK;
     h->kmer_k = kmer_table_depth(ix.seq_len);
     // One level more than ceil(log4 n) where HBM allows it (23 GB at K = 15): a K-mer of the read's own locus then has a second,
     // chance occurrence three times less often, and every such occurrence costs the seeding kernels real bwt_extend steps
@@ -739,11 +741,10 @@ int ensure_kmer_table(bsq_index* h, const DevIndex& ix) {
         // If the pools do not fit after all, the pipeline drops a level and goes on (kmer_downgrade).
         if (cudaMemGetInfo(&fr, &tot) == cudaSuccess && (ix.sa_bytes == 4 ? fr > 4 * kmer_table_bytes(15) : fr > want + (40ull << 30))) h->kmer_k = 15;
     }
-    if (const char* e = getenv("BSQ_KMER_K")) { const int k = atoi(e); if (k >= 8 && k <= 15) h->kmer_k = k; }
     if (h->kmer_k > h->kmer_k_cap) h->kmer_k = h->kmer_k_cap;
     CUDA_CHECK(cudaMalloc(&h->d_kmer, kmer_table_bytes(h->kmer_k)));
     build_kmer_table(ix, h->d_kmer, h->kmer_k, h->stream, &h->timing.launches);
-    if (!getenv("BSQ_NO_KMER_Z") && cudaMalloc(&h->d_kmer_z, kmer_table_bytes(h->kmer_k) / 4) == cudaSuccess) build_kmer_sizes(h->d_kmer, h->d_kmer_z, h->kmer_k, h->stream, &h->timing.launches);
+    if (cudaMalloc(&h->d_kmer_z, kmer_table_bytes(h->kmer_k) / 4) == cudaSuccess) build_kmer_sizes(h->d_kmer, h->d_kmer_z, h->kmer_k, h->stream, &h->timing.launches);
     else { h->d_kmer_z = nullptr; cudaGetLastError(); }
     CUDA_CHECK(cudaStreamSynchronize(h->stream));
     return BSQ_OK;
@@ -830,19 +831,16 @@ static int pipeline_enqueue_once(bsq_index* h, Batch& b) {
     ENS(b.scan_tmp.ensure(prim::scan_tmp_elems(n + 1) + 16));
     ENS(b.cigar.ensure(b.cigar_cap));
     ENS(b.ext_scratch.ensure((size_t)ext_warps * ext_per_warp)); ENS(b.fin_scratch.ensure((size_t)fin_warps * fin_per_warp));
-    int narrow_warps = 0;
-    const size_t narrow_bytes = narrow_zbuf_bytes(&narrow_warps);
-    ENS(b.narrow_z.ensure(narrow_bytes)); ENS(b.narrow_jobs.ensure((size_t)b.pool_cap * 5 * 24)); ENS(b.wide_jobs.ensure(b.pool_cap));
+    ENS(b.narrow_z.ensure(narrow_zbuf_bytes())); ENS(b.narrow_jobs.ensure((size_t)b.pool_cap * 5 * 24)); ENS(b.wide_jobs.ensure(b.pool_cap));
     ENS(b.ctl.ensure(64)); ENS(b.chain_todo.ensure(n)); ENS(b.fin_todo.ensure(n)); ENS(b.seed_todo.ensure(n + 1));
     if (max_len <= 496) { ENS(b.seed_pk.ensure((size_t)n * seed_thread_words(max_len))); ENS(b.seed_u32.ensure(3 * (size_t)n)); }
     // the thread-per-extension pre-pass packs column scores in 16 bits: every value it stores is <= l_query * (a + 1)
-    static const bool no_memo = getenv("BSQ_NO_EXT_MEMO") != nullptr;
     // Small batches take the warp-cooperative kernels for the DP stages: the thread-per-extension / thread-per-region kernels are built for
     // throughput (one thread runs a whole DP, ~0.5 ms of latency whatever the batch size), which is what a one-read call of
     // nuclseq_search_bwa would wait for.  BSQ_SMALL_BATCH_READS moves the threshold (0 = thread kernels always; the parity tests use that).
     static const long small_n = getenv("BSQ_SMALL_BATCH_READS") ? atol(getenv("BSQ_SMALL_BATCH_READS")) : 40000;   // measured crossover ~50 k reads (scripts/latency.py)
     const bool small_batch = (long)n < small_n;
-    const bool use_memo = !no_memo && !small_batch && max_len <= 512 && (uint64_t)max_len * (uint64_t)(o.a + 1) < 32000 && (uint64_t)n * EXT_MEMO_CHAINS < (1ull << 31);
+    const bool use_memo = !small_batch && max_len <= 512 && (uint64_t)max_len * (uint64_t)(o.a + 1) < 32000 && (uint64_t)n * EXT_MEMO_CHAINS < (1ull << 31);
     if (use_memo) {
         const size_t jobs2 = (size_t)n * EXT_MEMO_CHAINS * 2;
         ENS(b.ext_memo.ensure(jobs2)); ENS(b.ext_memo_key.ensure(jobs2)); ENS(b.ext_memo_perm.ensure(jobs2));
@@ -871,8 +869,7 @@ static int pipeline_enqueue_once(bsq_index* h, Batch& b) {
         P.blocks = b.blocks.p; P.ticket = b.ctl.p + 1; P.overflow = b.ctl.p + 4; P.counters = ctr ? ctr + 1 : nullptr;
         P.logtab = needs_seed_sw(b.max_len) ? b.read_logtab.p : nullptr; P.sw_cells = nullptr;
         // short reads: a thread-per-read pass takes every read with a handful of seed occurrences, the warp kernel the rest
-        static const bool no_thread_chain = getenv("BSQ_NO_CHAIN_THREAD") != nullptr;
-        const bool thread_chain = !no_thread_chain && !P.logtab;
+        const bool thread_chain = !P.logtab;
         P.todo = thread_chain ? b.chain_todo.p : nullptr; P.todo_cnt = b.ctl.p + 57;
         if (thread_chain) { launch_chain_thread(P, ix, o, st); ++T.launches; }
         launch_chain(P, ix, o, st); ++T.launches;
@@ -885,8 +882,7 @@ static int pipeline_enqueue_once(bsq_index* h, Batch& b) {
         P.ticket = b.ctl.p + 2; P.overflow = b.ctl.p + 4; P.need_rseq = b.ctl.p + 7; P.counters = ctr ? ctr + 3 : nullptr;
         P.memo = use_memo ? b.ext_memo.p : nullptr; P.memo_key = b.ext_memo_key.p; P.memo_perm = b.ext_memo_perm.p; P.memo_hist = b.ext_memo_hist.p;
         P.todo = use_memo ? b.ext_todo.p : nullptr; P.todo_cnt = b.ctl.p + 56;
-        static const bool one_stream = getenv("BSQ_EXT_ONE_STREAM") != nullptr;
-        launch_extend_memo(P, ix, o, st, &T.launches, one_stream ? nullptr : &b.ext_aux);
+        launch_extend_memo(P, ix, o, st, &T.launches, b.ext_aux);     // runs only with use_memo, whose !small_batch made the side streams
         if (use_memo) { launch_extend_finish(P, ix, o, st); ++T.launches; }
         launch_extend(P, ix, o, st); ++T.launches;
     }
@@ -897,11 +893,9 @@ static int pipeline_enqueue_once(bsq_index* h, Batch& b) {
         P.rows = b.rows.p; P.row_cnt = b.row_cnt.p; P.cigar_pool = b.cigar.p; P.cigar_cap = b.cigar_cap; P.cigar_top = b.ctl.p + 6;
         P.scratch = b.fin_scratch.p; P.scratch_per_warp = fin_per_warp; P.max_len = max_len; P.z_cap = z_cap; P.ann_id = h->d_ann_id;
         P.narrow_jobs = small_batch ? nullptr : b.narrow_jobs.p; P.narrow_cap = b.pool_cap; P.narrow_cnt = b.ctl.p + 32; P.wide_jobs = b.wide_jobs.p; P.wide_cnt = b.ctl.p + 25;
-        P.narrow_z = b.narrow_z.p; P.narrow_warps = narrow_warps;
-        { static const bool no_tight = getenv("BSQ_FIN_NO_TIGHT") != nullptr; P.narrow_tight = !no_tight; }
+        P.narrow_z = b.narrow_z.p;
         P.ticket = b.ctl.p + 40; P.overflow = b.ctl.p + 4; P.need_rseq = b.ctl.p + 7; P.counters = ctr ? ctr + 6 : nullptr;
-        static const bool no_thread_fin = getenv("BSQ_NO_FIN_THREAD") != nullptr;
-        P.todo = (no_thread_fin || small_batch) ? nullptr : b.fin_todo.p; P.todo_cnt = b.ctl.p + 58;
+        P.todo = small_batch ? nullptr : b.fin_todo.p; P.todo_cnt = b.ctl.p + 58;
         launch_finalize(P, ix, o, st, rseq_cap, fin_warps, &T.launches, b.ext_aux_ok ? &b.ext_aux : nullptr);
     }
     // compact rows: exclusive scan of row_cnt (n + 1 entries, the last one is a zero pad) -> row_off
@@ -1159,9 +1153,7 @@ int download_result(bsq_index* h, Batch& b, bsq_result** out) {
 constexpr uint64_t CHUNK_MIN = 1u << 16, CHUNK_MAX = 1u << 20;
 uint64_t chunk_reads(uint64_t n, bool two = false) {
     if (two) return std::max((n + 1) / 2, CHUNK_MIN);
-    static long long env = -1;
-    if (env < 0) { env = 0; if (const char* e = getenv("BSQ_CHUNK_READS")) { const long long x = atoll(e); if (x >= 1024) env = x; } }
-    if (env > 0) return (uint64_t)env;
+    if (const char* e = getenv("BSQ_CHUNK_READS")) { const long long x = atoll(e); if (x >= 1024) return (uint64_t)x; }   // read per call: tests set it
     const uint64_t k = std::max<uint64_t>(2, (n + CHUNK_MAX - 1) / CHUNK_MAX);     // as few chunks as the cap allows, at least two
     return std::max((n + k - 1) / k, CHUNK_MIN);
 }
@@ -1186,23 +1178,9 @@ int align_chunked(bsq_index* h, const ReadSrc& S, uint64_t n, bsq_result** out, 
     };
     Batch* lane[2] = {&h->batch, &h->batch2};
     for (Batch* b : lane) if (!b->evx_ok) { for (auto& e : b->ev_x) cudaEventCreate(&e); b->evx_ok = true; }
-    // chunk boundaries: uniform chunks, or (BSQ_CHUNK_FRACS="f0,f1,...") fractions of the batch -- the first chunk's upload and the
-    // last chunk's download are the only copies nothing hides, while every chunk pays the fixed cost of ~40 kernel tails
-    std::vector<uint64_t> starts;
-    {
-        static const char* fr = getenv("BSQ_CHUNK_FRACS");
-        if (fr) {
-            double acc = 0; starts.push_back(0);
-            for (const char* q = fr; *q;) { char* e; const double f = strtod(q, &e); if (e == q) break; acc += f; starts.push_back(std::min<uint64_t>(n, (uint64_t)(acc * (double)n))); q = *e ? e + 1 : e; }
-            if (starts.back() != n) starts.push_back(n);
-        } else {
-            const uint64_t CHUNK_READS = chunk_reads(n, (h->flags & BSQ_FLAG_TWO_CHUNKS) != 0);
-            for (uint64_t s0 = 0; s0 < n; s0 += CHUNK_READS) starts.push_back(s0);
-            starts.push_back(n);
-        }
-    }
-    const uint64_t n_chunks = starts.size() - 1;
-    auto start_of = [&](uint64_t c) { return starts[std::min<uint64_t>(c, n_chunks)]; };
+    const uint64_t CHUNK_READS = chunk_reads(n, (h->flags & BSQ_FLAG_TWO_CHUNKS) != 0);
+    const uint64_t n_chunks = (n + CHUNK_READS - 1) / CHUNK_READS;
+    auto start_of = [&](uint64_t c) { return std::min(c * CHUNK_READS, n); };
     auto launch = [&](uint64_t c) -> int {
         Batch& b = *lane[c & 1];
         const uint64_t s0 = start_of(c), cnt = start_of(c + 1) - s0;
@@ -1212,12 +1190,7 @@ int align_chunked(bsq_index* h, const ReadSrc& S, uint64_t n, bsq_result** out, 
         if (upload_src(h, b, S, s0, cnt) != BSQ_OK) return BSQ_ERR;
         mark("upload done (headers back)", c);
         cudaEventRecord(b.ev_x[1], b.st);
-        // BSQ_CHUNK_SERIAL: chunk c's kernels start behind chunk c-1's (its copies still overlap them), so that an earlier chunk is
-        // finished -- and its download under way -- while the later one computes, instead of both sharing the SMs to the end
-        static const bool serial = getenv("BSQ_CHUNK_SERIAL") != nullptr;
-        if (serial && c > 0) cudaStreamWaitEvent(b.st, lane[(c & 1) ^ 1]->ev_x[4], 0);
         const int rc2 = pipeline_enqueue(h, b);
-        cudaEventRecord(b.ev_x[4], b.st);
         mark("pipeline queued", c);
         return rc2;
     };
@@ -1313,7 +1286,7 @@ static int align_batch_src(bsq_index* h, const ReadSrc& S, uint64_t n, bsq_resul
     bsq_timing& T = h->timing;
     T.launches = 0; T.h2d_bytes = T.d2h_bytes = 0; T.h2d = T.d2h = 0; T.notes = 0;
     int rc = BSQ_OK;
-    bool chunked = n >= 2 * CHUNK_MIN && n > chunk_reads(n, (h->flags & BSQ_FLAG_TWO_CHUNKS) != 0) && h->meta.built && !getenv("BSQ_NO_CHUNKS");
+    bool chunked = n >= 2 * CHUNK_MIN && n > chunk_reads(n, (h->flags & BSQ_FLAG_TWO_CHUNKS) != 0) && h->meta.built;
     cudaEventRecord(e0, h->stream);
     if (chunked) {
         // two lanes, copies overlapped with compute; the stage times are sums over chunks of each lane's stream time
@@ -1488,8 +1461,7 @@ int bsq_result_tuples(bsq_index* h, const bsq_result* res, const char* seqs, con
     {   // a result of this library whose batch is still in HBM needs no upload at all
         const ResultImpl* mine = nullptr;
         { std::lock_guard<std::mutex> lk(g_live_mu); for (const ResultImpl* r : g_live) if (&r->pub == res) { mine = r; break; } }
-        static const bool no_res = getenv("BSQ_TUPLES_NO_RESIDENT") != nullptr;
-        if (mine && h->meta.built && !no_res) {
+        if (mine && h->meta.built) {
             if (cudaSetDevice(h->device) != cudaSuccess) { bsq_set_error("cudaSetDevice failed"); return BSQ_ERR; }
             const int rc = tuples_resident(h, mine, flags, out);
             if (rc != 1) return rc;

@@ -203,8 +203,8 @@ void launch_dp(const ExtendParams& p, const DevIndex& ix, const DevOpts& o, cuda
 }  // namespace
 
 // aux: three extra streams + eight events (ExtAux, owned by the batch) so that the four length classes of one side run
-// concurrently -- each class alone leaves most of the chip idle in its tail; nullptr = everything on st.
-void launch_extend_memo(const ExtendParams& p, const DevIndex& ix, const DevOpts& o, cudaStream_t st, uint64_t* launches, const ExtAux* aux) {
+// concurrently -- each class alone leaves most of the chip idle in its tail.
+void launch_extend_memo(const ExtendParams& p, const DevIndex& ix, const DevOpts& o, cudaStream_t st, uint64_t* launches, const ExtAux& aux) {
     if (!p.memo || p.n_reads == 0) return;
     const int sms = cached_sm_count();
     const unsigned blocks = (p.n_reads + PLAN_THREADS - 1) / PLAN_THREADS;
@@ -213,19 +213,15 @@ void launch_extend_memo(const ExtendParams& p, const DevIndex& ix, const DevOpts
     ext_plan_scan<<<1, 32, 0, st>>>(p.memo_hist);
     ext_plan_scatter<<<(p.n_reads * EXT_MEMO_CHAINS + PLAN_THREADS - 1) / PLAN_THREADS, PLAN_THREADS, 0, st>>>(p);
     for (int side = 0; side < 2; ++side) {
-        cudaStream_t s1 = st, s2 = st, s3 = st;
-        if (aux) {   // fork
-            cudaEventRecord(aux->ev[0], st);
-            s1 = aux->st[0]; s2 = aux->st[1]; s3 = aux->st[2];
-            for (int k = 0; k < 3; ++k) cudaStreamWaitEvent(aux->st[k], aux->ev[0], 0);
-        }
+        // fork
+        cudaEventRecord(aux.ev[0], st);
+        for (int k = 0; k < 3; ++k) cudaStreamWaitEvent(aux.st[k], aux.ev[0], 0);
         launch_dp<97>(p, ix, o, st, side, 65, 96, sms);          // the class with most cells keeps the main stream
-        launch_dp<65>(p, ix, o, s1, side, 33, 64, sms);
-        launch_dp<EXT_MEMO_MAXQ + 1>(p, ix, o, s2, side, 97, EXT_MEMO_MAXQ, sms);
-        launch_dp<33>(p, ix, o, s3, side, 1, 32, sms);
-        if (aux) {   // join
-            for (int k = 0; k < 3; ++k) { cudaEventRecord(aux->ev[1 + k], aux->st[k]); cudaStreamWaitEvent(st, aux->ev[1 + k], 0); }
-        }
+        launch_dp<65>(p, ix, o, aux.st[0], side, 33, 64, sms);
+        launch_dp<EXT_MEMO_MAXQ + 1>(p, ix, o, aux.st[1], side, 97, EXT_MEMO_MAXQ, sms);
+        launch_dp<33>(p, ix, o, aux.st[2], side, 1, 32, sms);
+        // join
+        for (int k = 0; k < 3; ++k) { cudaEventRecord(aux.ev[1 + k], aux.st[k]); cudaStreamWaitEvent(st, aux.ev[1 + k], 0); }
     }
     if (launches) *launches += 11;
 }

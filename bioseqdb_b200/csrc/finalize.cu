@@ -6,6 +6,7 @@
 // The DP rows run on the whole warp (ksw_global_warp).  MAPQ needs libm's log() and is finished on the
 // host from the fields written here (A.12).
 #include "pipeline.cuh"
+#include <algorithm>
 #include <cstdlib>
 #include "ksw_warp.cuh"
 #include "ksort_dev.cuh"
@@ -15,7 +16,7 @@ namespace {
 
 constexpr int FIN_THREADS = 128;
 constexpr int FIN_WARPS = FIN_THREADS / 32;
-// thread-per-region kernel limits: band columns (circular row buffer), target rows, query length
+// thread-per-region routing limits (narrow_class): band columns of a first try, target rows, query length
 constexpr int NARROW_NC = 64;
 constexpr int NARROW_TMAX = 192;
 constexpr int NARROW_QMAX = 160;
@@ -191,31 +192,8 @@ __device__ __forceinline__ int gen_cigar_band(const DevOpts& o, int l_query, int
     return w > min_w ? w : min_w;
 }
 
-__device__ __forceinline__ bool narrow_is_tight(const DevOpts& o, int lq, int rlen, bool simple_mat, int wt);
-// 0: align on the warp here; 1: thread-per-region narrow-band DP; 2: thread-per-region, no DP (equal lengths, zero band).
-// tight_ok: the tight passes are on and the matrix is the plain one -- then a region whose band is wider than any thread kernel's
-// still gets its first try there (the proof of the tight passes does not care how wide the band asked for is; a region they cannot
-// settle travels on to the exact-band lists, whose kernels hand a band they do not hold to the warp-cooperative one).
-__device__ __forceinline__ int narrow_class(const DevOpts& o, const RegRec& ar, uint32_t max_len, bool tight_ok) {
-    const int lq = ar.qe - ar.qb; const int64_t rl = ar.re - ar.rb;
-    if (max_len > NARROW_QMAX || lq <= 0 || rl <= 0 || rl > NARROW_TMAX) return 0;
-    int w2 = reg2aln_w2(o, ar);
-    w2 = w2 < o.w << 2 ? w2 : o.w << 2;
-    if (lq == rl) return 2;   // equal lengths: first a thread checks whether the gap-free diagonal is provably the unique optimum
-    if (2 * gen_cigar_band(o, lq, (int)rl, w2) + 1 <= NARROW_NC) return 1;
-    return tight_ok && narrow_is_tight(o, lq, (int)rl, true, 8) ? 1 : 0;
-}
-
-// the register-band kernel derives scores from the three values bwa_fill_scmat produces (match, mismatch, ambiguous)
-__device__ __forceinline__ bool mat_is_simple(const int* smat) {
-    bool ok = true;
-    for (int a = 0; a < 5; ++a)
-        for (int b = 0; b < 5; ++b) ok = ok && smat[a * 5 + b] == ((a == 4 || b == 4) ? smat[4] : (a == b ? smat[0] : smat[1]));
-    return ok;
-}
-
 // A job list holds both classes of thread-per-region work so that the lanes of a warp do similar work: regions whose band
-// fits the register window (w <= REG_WT) grow from the front, wider ones (shared-memory kernel) from the back.
+// fits the register window (w <= REG_WT) grow from the front, wider ones (the wide register kernel, w <= REG_WT2) from the back.
 constexpr int REG_WT = 16;
 // tight first tries: MODE 4 runs a 9-column window, MODE 3 a 17-column one; a result is accepted only when no path that leaves
 // the window can reach the score found inside it (lists T4 -> T8 -> A)
@@ -224,15 +202,27 @@ constexpr int REG_WT3 = 8;
 constexpr int REG_WT4 = 4;
 constexpr int NARROW_T4_CNT = 20, NARROW_T8_CNT = 21;   // counters of lists T4 / T8 behind narrow_cnt (ctl words 52, 53)
 constexpr int REG_WT2 = 32;   // second register kernel: bands of half-width 17..32 (65 columns of H and E in registers, 2 CTAs per SM)
-__device__ __forceinline__ bool narrow_is_big(const DevOpts& o, int lq, int rlen, int w2, bool simple_mat) {
+__device__ __forceinline__ bool narrow_is_big(const DevOpts& o, int lq, int rlen, int w2) {
     w2 = w2 < o.w << 2 ? w2 : o.w << 2;
-    return !simple_mat || gen_cigar_band(o, lq, rlen, w2) > REG_WT;
+    return gen_cigar_band(o, lq, rlen, w2) > REG_WT;
 }
 // the tight pass takes a region when the register kernels can score it and the end cell lies inside the tight window
-__device__ __forceinline__ bool narrow_is_tight(const DevOpts& o, int lq, int rlen, bool simple_mat, int wt = REG_WT3) {
-    static_assert(REG_WT3 == 8, "narrow_class passes the literal");
+__device__ __forceinline__ bool narrow_is_tight(const DevOpts& o, int lq, int rlen, int wt = REG_WT3) {
     const int dl = lq - rlen;
-    return simple_mat && (dl < 0 ? -dl : dl) <= wt && o.o_del >= 0 && o.e_del >= 0 && o.o_ins >= 0 && o.e_ins >= 0 && o.mat_max > 0;
+    return (dl < 0 ? -dl : dl) <= wt && o.o_del >= 0 && o.e_del >= 0 && o.o_ins >= 0 && o.e_ins >= 0 && o.mat_max > 0;
+}
+// 0: align on the warp here; 1: thread-per-region narrow-band DP; 2: thread-per-region, no DP (equal lengths, zero band).
+// A region whose band is wider than any thread kernel's still gets its first try there when the tight passes can take it (their
+// proof does not care how wide the band asked for is; a region they cannot settle travels on to the exact-band lists, whose
+// kernels hand a band they do not hold to the warp-cooperative one).
+__device__ __forceinline__ int narrow_class(const DevOpts& o, const RegRec& ar, uint32_t max_len) {
+    const int lq = ar.qe - ar.qb; const int64_t rl = ar.re - ar.rb;
+    if (max_len > NARROW_QMAX || lq <= 0 || rl <= 0 || rl > NARROW_TMAX) return 0;
+    int w2 = reg2aln_w2(o, ar);
+    w2 = w2 < o.w << 2 ? w2 : o.w << 2;
+    if (lq == rl) return 2;   // equal lengths: first a thread checks whether the gap-free diagonal is provably the unique optimum
+    if (2 * gen_cigar_band(o, lq, (int)rl, w2) + 1 <= NARROW_NC) return 1;
+    return narrow_is_tight(o, lq, (int)rl) ? 1 : 0;
 }
 __device__ __forceinline__ void push_narrow(NarrowJob* list, uint32_t cap, uint32_t* cnt_reg, uint32_t* cnt_big, const NarrowJob& jb, bool big) {
     if (big) list[cap - 1u - atomicAdd(cnt_big, 1u)] = jb;
@@ -304,16 +294,15 @@ __global__ void __launch_bounds__(128) regs_finalize_thread(FinalizeParams P, De
         if (n == 0) { P.row_cnt[r] = 0; done = true; }
         else if (n == 1) {
             RegRec ar = P.regs[blk.base];
-            const int ncls = narrow_class(o, ar, P.max_len, P.narrow_tight && mat_is_simple(o.mat));
+            const int ncls = narrow_class(o, ar, P.max_len);
             if (ncls != 0) {
                 ar.sub = 0; ar.secondary = -1; ar.hash = hash_64((uint64_t)P.ids[r]);      // mem_mark_primary_se, n == 1
                 P.regs[blk.base] = ar;
                 P.rows[blk.base] = row_from_reg(ar, P.ann_id);
                 jb.slot = blk.base; jb.w2 = reg2aln_w2(o, ar);
                 if (ncls == 1) {
-                    const bool sm = mat_is_simple(o.mat);
-                    if (P.narrow_tight && narrow_is_tight(o, ar.qe - ar.qb, (int)(ar.re - ar.rb), sm)) cat = narrow_is_tight(o, ar.qe - ar.qb, (int)(ar.re - ar.rb), sm, REG_WT4) ? 4 : 5;
-                    else cat = narrow_is_big(o, ar.qe - ar.qb, (int)(ar.re - ar.rb), jb.w2, sm) ? 2 : 1;
+                    if (narrow_is_tight(o, ar.qe - ar.qb, (int)(ar.re - ar.rb))) cat = narrow_is_tight(o, ar.qe - ar.qb, (int)(ar.re - ar.rb), REG_WT4) ? 4 : 5;
+                    else cat = narrow_is_big(o, ar.qe - ar.qb, (int)(ar.re - ar.rb), jb.w2) ? 2 : 1;
                 } else cat = 3;
                 P.row_cnt[r] = 1;
                 done = true;
@@ -346,7 +335,6 @@ __global__ void __launch_bounds__(FIN_THREADS, 6) regs_finalize(FinalizeParams P
     __shared__ int smat[25];
     if (threadIdx.x < 25) smat[threadIdx.x] = o.mat[threadIdx.x];
     __syncthreads();
-    const bool simple_mat = mat_is_simple(smat);
     const int lane = lane_id();
     const uint32_t gwarp = (blockIdx.x * FIN_THREADS + threadIdx.x) >> 5;
     FScratch S;
@@ -481,7 +469,7 @@ __global__ void __launch_bounds__(FIN_THREADS, 6) regs_finalize(FinalizeParams P
         for (int i = 0; i < n; ++i) {
             const RegRec ar = a[i];
             RowDev row = row_from_reg(ar, P.ann_id);
-            const int ncls = P.narrow_jobs != nullptr ? narrow_class(o, ar, P.max_len, P.narrow_tight && simple_mat) : 0;
+            const int ncls = P.narrow_jobs != nullptr ? narrow_class(o, ar, P.max_len) : 0;
             const bool narrow = ncls != 0;
             if (lane == 0) {
                 rows[i] = row;
@@ -489,11 +477,11 @@ __global__ void __launch_bounds__(FIN_THREADS, 6) regs_finalize(FinalizeParams P
                     // DP regions and no-DP regions go to separate lists so that the lanes of a warp do similar work
                     NarrowJob jb; jb.r = r; jb.slot = blk.base + i; jb.w2 = reg2aln_w2(o, ar); jb.last_sc = -(1 << 30); jb.it = 0; jb.score = 0;
                     NarrowJob* lists = reinterpret_cast<NarrowJob*>(P.narrow_jobs);
-                    if (ncls == 1 && P.narrow_tight && narrow_is_tight(o, ar.qe - ar.qb, (int)(ar.re - ar.rb), simple_mat)) {
-                        if (narrow_is_tight(o, ar.qe - ar.qb, (int)(ar.re - ar.rb), simple_mat, REG_WT4)) lists[3u * P.narrow_cap + atomicAdd(P.narrow_cnt + NARROW_T4_CNT, 1u)] = jb;
+                    if (ncls == 1 && narrow_is_tight(o, ar.qe - ar.qb, (int)(ar.re - ar.rb))) {
+                        if (narrow_is_tight(o, ar.qe - ar.qb, (int)(ar.re - ar.rb), REG_WT4)) lists[3u * P.narrow_cap + atomicAdd(P.narrow_cnt + NARROW_T4_CNT, 1u)] = jb;
                         else lists[4u * P.narrow_cap + atomicAdd(P.narrow_cnt + NARROW_T8_CNT, 1u)] = jb;
                     }
-                    else if (ncls == 1) push_narrow(lists, P.narrow_cap, P.narrow_cnt, P.narrow_cnt + 5, jb, narrow_is_big(o, ar.qe - ar.qb, (int)(ar.re - ar.rb), jb.w2, simple_mat));
+                    else if (ncls == 1) push_narrow(lists, P.narrow_cap, P.narrow_cnt, P.narrow_cnt + 5, jb, narrow_is_big(o, ar.qe - ar.qb, (int)(ar.re - ar.rb), jb.w2));
                     else lists[2u * P.narrow_cap + atomicAdd(P.narrow_cnt + 3, 1u)] = jb;
                 }
             }
@@ -671,43 +659,34 @@ __device__ __forceinline__ int diag_mismatches(const uint8_t* qg, int lq, bool r
 
 // ---------------------------------------------------------------------------------------------------
 // Thread-per-region mem_reg2aln for narrow bands (the common case for 150 bp reads: w = 6..31).
-// One thread runs the scalar ksw_global2 recurrence; the row buffer is a 64-entry circular window in
-// shared memory laid out [column][thread] (bank = thread, conflict-free for any column), the query is
-// staged in shared memory the same way, reference bases are decoded from pac once per row, traceback
-// bytes go to a per-warp global buffer laid out [cell][lane] (coalesced while lanes run in step).
-// A region whose retry needs a wider band is handed to regs_cigar_wide (warp-cooperative rows).
+// One thread runs the ksw_global2 recurrence with the band in registers (global_dp_reg), reference bases are
+// decoded from pac once per row, traceback bytes go to a per-warp global buffer laid out [cell][lane]
+// (coalesced while lanes run in step).  A region whose band the kernel does not hold is handed to
+// regs_cigar_wide (warp-cooperative rows).
 struct NarrowParams {
     const uint8_t* seqs; const uint64_t* offs; const RegRec* regs; RowDev* rows;
     const NarrowJob* jobs; int job_stride; const uint32_t* n_jobs;      // jobs[k * job_stride]: a list's front (+1) or back (-1) section
     NarrowJob* requeue; uint32_t requeue_cap; uint32_t* requeue_cnt; uint32_t* requeue_big_cnt; uint64_t* wide_jobs; uint32_t* wide_cnt;
     uint32_t* cigar_pool; uint32_t cigar_cap; uint32_t* cigar_top;
     uint8_t* zbuf; uint32_t* ticket; uint32_t* overflow; unsigned long long* counters;
-    int big_go_wide; // experiment (BSQ_FIN_BIG_TO_WIDE): bands wider than the register window go to the warp-cooperative kernel
-    NarrowJob* tight; uint32_t* tight_cnt;   // list T: first tries the tight pass (MODE 3) takes; nullptr = no tight pass
+    NarrowJob* tight; uint32_t* tight_cnt;   // the next tight list: T4 for the diagonal pass (MODE 5), T8 for MODE 4
     uint32_t short_list;   // lists of at most this many regions are handed to the warp-cooperative kernel (BSQ_FIN_SHORT_LIST)
-    int diag_pass;   // 1: equal-length regions -- finish the ones whose diagonal is provably optimal, hand the rest to the DP list
 };
 
 // MODE 5: the diagonal pass only (no DP code, few registers: the pass is a chain of dependent loads per region and lives on occupancy).
-// MODE 0: circular row window in shared memory (bands up to NARROW_NC columns); MODE 1: the band in registers
-// (global_dp_reg, w <= REG_WT), no shared memory, regions with a wider band are passed on to a MODE 0 launch.
+// MODE 1: the band in registers (global_dp_reg, w <= REG_WT); MODE 2: the same for w <= REG_WT2 (2 CTAs per SM); MODE 4 / 3: the
+// tight passes.  Scores come from the three values of bwa_fill_scmat, the only matrix DevOpts carries (fill_dev_opts).
 template <int MODE>
-__global__ void __launch_bounds__(NARROW_THREADS, MODE == 5 ? 10 : (MODE >= 3 ? 6 : (MODE == 1 ? 4 : (MODE == 2 ? 2 : 1)))) regs_cigar_narrow(NarrowParams P, DevIndex ix, DevOpts o) {
-    extern __shared__ __align__(16) uint8_t dyn_smem[];
+__global__ void __launch_bounds__(NARROW_THREADS, MODE == 5 ? 10 : (MODE >= 3 ? 6 : (MODE == 1 ? 4 : 2))) regs_cigar_narrow(NarrowParams P, DevIndex ix, DevOpts o) {
     __shared__ int smat[25];
     if (threadIdx.x < 25) smat[threadIdx.x] = o.mat[threadIdx.x];
     __syncthreads();
     const int tid = threadIdx.x, lane = tid & 31;
-    int* H = reinterpret_cast<int*>(dyn_smem) + tid;                                 // H[c * NARROW_THREADS]
-    int* E = reinterpret_cast<int*>(dyn_smem) + NARROW_NC * NARROW_THREADS + tid;
-    uint8_t* Q = dyn_smem + 2 * NARROW_NC * NARROW_THREADS * 4 + tid;               // Q[j * NARROW_THREADS]
     const uint32_t gwarp = (blockIdx.x * NARROW_THREADS + tid) >> 5;
     // traceback bytes, 4 cells per 32-bit store, laid out [row][4-cell group][lane]: a warp store is 128 contiguous bytes
-    constexpr int WTM = MODE == 2 ? REG_WT2 : (MODE == 3 ? REG_WT3 : (MODE == 4 ? REG_WT4 : REG_WT));                                // half-width of the register window (MODE 1 / 2)
-    constexpr size_t Z_PER_WARP = MODE != 0 ? (size_t)NARROW_TMAX * ((2 * WTM + 1 + 3) / 4) * 4 * 32 : (size_t)NARROW_TMAX * NARROW_NC * 32;
-    constexpr int ZROW = MODE != 0 ? (2 * WTM + 1 + 3) / 4 : NARROW_NC / 4;         // words per row and lane
-    uint32_t* Z = reinterpret_cast<uint32_t*>(P.zbuf + (size_t)gwarp * Z_PER_WARP) + lane;
-    const bool simple_mat = mat_is_simple(smat);
+    constexpr int WTM = MODE == 2 ? REG_WT2 : (MODE == 3 ? REG_WT3 : (MODE == 4 ? REG_WT4 : REG_WT));                                // half-width of the register window
+    constexpr int ZROW = (2 * WTM + 1 + 3) / 4;                                      // words per row and lane
+    uint32_t* Z = reinterpret_cast<uint32_t*>(P.zbuf + (size_t)gwarp * NARROW_TMAX * ZROW * 4 * 32) + lane;
     int oe_del = o.o_del + o.e_del, oe_ins = o.o_ins + o.e_ins, e_del = o.e_del, e_ins = o.e_ins;
     // keep the four gap constants in registers: left to itself the compiler re-reads them from the constant bank per cell
     asm volatile("" : "+r"(oe_del), "+r"(oe_ins), "+r"(e_del), "+r"(e_ins));
@@ -715,7 +694,9 @@ __global__ void __launch_bounds__(NARROW_THREADS, MODE == 5 ? 10 : (MODE >= 3 ? 
     const uint32_t n_jobs = *P.n_jobs;
     // A short list is a latency problem for one thread per region (a launch lasts as long as ONE region's DP, hundreds of
     // microseconds): its regions go to the warp-cooperative kernel, which runs a row's cells side by side.
-    const bool short_list = MODE != 0 && !P.diag_pass && n_jobs <= P.short_list;
+    // MODE 5 (the diagonal pass): equal-length regions -- finish the ones whose diagonal is provably optimal, hand the rest to the DP list
+    constexpr bool diag_pass = MODE == 5;
+    const bool short_list = !diag_pass && n_jobs <= P.short_list;
     unsigned long long cells = 0, calls = 0;
     for (;;) {
         uint32_t t = next_ticket(P.ticket);
@@ -739,8 +720,7 @@ __global__ void __launch_bounds__(NARROW_THREADS, MODE == 5 ? 10 : (MODE >= 3 ? 
             // libbwa reverses query and reference on the reverse strand; both then read pac ascending
             const int64_t tbase = rev ? (l_pac << 1) - re : rb;
             const uint8_t* qg = P.seqs + P.offs[r] + qb;
-            if (MODE == 0) for (int j = 0; j < lq; ++j) Q[j * NARROW_THREADS] = rev ? qg[lq - 1 - j] : qg[j];
-            auto qat = [&](int j) -> int { return MODE == 0 ? (int)Q[j * NARROW_THREADS] : (int)(rev ? qg[lq - 1 - j] : qg[j]); };
+            auto qat = [&](int j) -> int { return (int)(rev ? qg[lq - 1 - j] : qg[j]); };
             // ONE try of the band-doubling loop per pass; a region that needs another try is re-queued so that the
             // lanes of a warp stay balanced (the loop state travels in the job record)
             int n_cigar = 0, NM = -1, score = jb.score;
@@ -752,25 +732,23 @@ __global__ void __launch_bounds__(NARROW_THREADS, MODE == 5 ? 10 : (MODE >= 3 ? 
                 int nm_known = -1;       // mismatches of a gap-free row, when the packed comparison has counted them already
                 if (!reject) {
                     bool diagonal = lq == rlen && w2 == 0;   // bwa_gen_cigar2's own no-DP case
-                    if (P.diag_pass && lq == rlen) {
+                    if (diag_pass && lq == rlen) {
                         // Equal lengths: any alignment other than the gap-free diagonal has >= 1 insertion and >= 1 deletion and at
                         // most lq - 1 aligned pairs, so it scores <= (lq - 1) max(mat) - oe_ins - oe_del.  If the diagonal beats that
                         // bound it is the UNIQUE optimum of ksw_global2 for every band (the diagonal lies inside any band), so the
                         // traceback is lq M and the score is band-independent: the DP and the band-doubling retries are skipped.
                         int sc = 0;
                         bool fast = false;
-                        if (MODE != 0 && simple_mat) {
-                            const int mm = diag_mismatches(qg, lq, rev, ix.pac, tbase, &fast);
-                            if (fast) { sc = smat[0] * (lq - mm) + smat[1] * mm; nm_known = mm; }
-                        }
-                        if (!fast) for (int i = 0; i < lq; ++i) {
+                        const int mm = diag_mismatches(qg, lq, rev, ix.pac, tbase, &fast);
+                        if (fast) { sc = smat[0] * (lq - mm) + smat[1] * mm; nm_known = mm; }
+                        else for (int i = 0; i < lq; ++i) {
                             const int tb = rev ? 3 - (int)pac_get(ix.pac, tbase + i) : (int)pac_get(ix.pac, tbase + i);
                             sc += smat[tb * 5 + qat(i)];
                         }
                         if (diagonal || sc > (lq - 1) * o.mat_max - oe_ins - oe_del) { score = sc; cg[0] = (uint32_t)lq << 4; n_cigar = 1; diagonal = true; }
                         else {   // needs the DP: over to the tight pass or the DP list, same try
-                            if (P.tight && narrow_is_tight(o, lq, rlen, simple_mat)) P.tight[atomicAdd(P.tight_cnt, 1u)] = jb;
-                            else push_narrow(P.requeue, P.requeue_cap, P.requeue_cnt, P.requeue_big_cnt, jb, narrow_is_big(o, lq, rlen, jb.w2, simple_mat));
+                            if (narrow_is_tight(o, lq, rlen)) P.tight[atomicAdd(P.tight_cnt, 1u)] = jb;
+                            else push_narrow(P.requeue, P.requeue_cap, P.requeue_cnt, P.requeue_big_cnt, jb, narrow_is_big(o, lq, rlen, jb.w2));
                             again = true; break;
                         }
                     } else if (diagonal) {
@@ -789,79 +767,27 @@ __global__ void __launch_bounds__(NARROW_THREADS, MODE == 5 ? 10 : (MODE >= 3 ? 
                         // sees the same winner as under the band bwa_gen_cigar2 asks for (an alternative through outside cells, continued
                         // along the same suffix, would be a full path scoring >= the optimum): score and CIGAR are those of band w.
                         const int w = MODE >= 3 ? (wx < WTM ? wx : WTM) : wx;
-                        if (MODE >= 3 && (!narrow_is_tight(o, lq, rlen, simple_mat, WTM) || rlen > NARROW_TMAX)) {
-                            push_narrow(P.requeue, P.requeue_cap, P.requeue_cnt, P.requeue_big_cnt, jb, narrow_is_big(o, lq, rlen, jb.w2, simple_mat));
+                        if (MODE >= 3 && (!narrow_is_tight(o, lq, rlen, WTM) || rlen > NARROW_TMAX)) {
+                            push_narrow(P.requeue, P.requeue_cap, P.requeue_cnt, P.requeue_big_cnt, jb, narrow_is_big(o, lq, rlen, jb.w2));
                             again = true; break;
                         }
-                        const int n_col = lq < 2 * w + 1 ? lq : 2 * w + 1;
-                        if (MODE >= 3) {}
-                        else if ((MODE != 0 ? (w > WTM || !simple_mat) : (2 * w + 1 > NARROW_NC || P.big_go_wide)) || rlen > NARROW_TMAX) { go_wide = true; break; }
+                        if (MODE < 3 && (w > WTM || rlen > NARROW_TMAX)) { go_wide = true; break; }
                         ++calls;
-                        if (MODE != 0) {
-                            uint32_t amb = 0;
-                            score = global_dp_reg<WTM, (MODE >= 3)>(qg, lq, rev, ix.pac, tbase, rlen, w, smat[0], smat[1], smat[4], o.o_del, e_del, o.o_ins, e_ins, Z, cells, &amb);
-                            if (MODE >= 3 && (amb & ~3u)) {            // an ambiguous base in the query: the exact-band kernels score it
-                                push_narrow(P.requeue, P.requeue_cap, P.requeue_cnt, P.requeue_big_cnt, jb, narrow_is_big(o, lq, rlen, jb.w2, simple_mat));
+                        uint32_t amb = 0;
+                        score = global_dp_reg<WTM, (MODE >= 3)>(qg, lq, rev, ix.pac, tbase, rlen, w, smat[0], smat[1], smat[4], o.o_del, e_del, o.o_ins, e_ins, Z, cells, &amb);
+                        if (MODE >= 3 && (amb & ~3u)) {            // an ambiguous base in the query: the exact-band kernels score it
+                            push_narrow(P.requeue, P.requeue_cap, P.requeue_cnt, P.requeue_big_cnt, jb, narrow_is_big(o, lq, rlen, jb.w2));
+                            again = true; break;
+                        }
+                        if (MODE >= 3 && w < wx) {
+                            const int k = w + 1, dl = lq - rlen;
+                            const int ubp = o.mat_max * (lq - k) - (o.o_ins + e_ins * k) - (o.o_del + e_del * (k - dl));
+                            const int ubm = o.mat_max * (rlen - k) - (o.o_del + e_del * k) - (o.o_ins + e_ins * (k + dl));
+                            if (score <= (ubp > ubm ? ubp : ubm)) {    // not provable: the next wider window, or the band bwa asks for; same try
+                                if (MODE == 4) P.tight[atomicAdd(P.tight_cnt, 1u)] = jb;
+                                else push_narrow(P.requeue, P.requeue_cap, P.requeue_cnt, P.requeue_big_cnt, jb, narrow_is_big(o, lq, rlen, jb.w2));
                                 again = true; break;
                             }
-                            if (MODE >= 3 && w < wx) {
-                                const int k = w + 1, dl = lq - rlen;
-                                const int ubp = o.mat_max * (lq - k) - (o.o_ins + e_ins * k) - (o.o_del + e_del * (k - dl));
-                                const int ubm = o.mat_max * (rlen - k) - (o.o_del + e_del * k) - (o.o_ins + e_ins * (k + dl));
-                                if (score <= (ubp > ubm ? ubp : ubm)) {    // not provable: the next wider window, or the band bwa asks for; same try
-                                    if (MODE == 4 && P.tight) P.tight[atomicAdd(P.tight_cnt, 1u)] = jb;
-                                    else push_narrow(P.requeue, P.requeue_cap, P.requeue_cnt, P.requeue_big_cnt, jb, narrow_is_big(o, lq, rlen, jb.w2, simple_mat));
-                                    again = true; break;
-                                }
-                            }
-                        } else {
-                        // first row of the band
-                        H[0] = 0; E[0] = KSW_NEG_INF;
-                        for (int j = 1; j <= lq && j <= w; ++j) { H[(j & (NARROW_NC - 1)) * NARROW_THREADS] = -(o.o_ins + e_ins * j); E[(j & (NARROW_NC - 1)) * NARROW_THREADS] = KSW_NEG_INF; }
-                        if (w + 1 <= lq) { H[((w + 1) & (NARROW_NC - 1)) * NARROW_THREADS] = KSW_NEG_INF; E[((w + 1) & (NARROW_NC - 1)) * NARROW_THREADS] = KSW_NEG_INF; }
-                        for (int i = 0; i < rlen; ++i) {
-                            const int beg = i > w ? i - w : 0;
-                            const int end = i + w + 1 < lq ? i + w + 1 : lq;
-                            int h1 = beg == 0 ? -(o.o_del + e_del * (i + 1)) : KSW_NEG_INF;
-                            int f = KSW_NEG_INF;
-                            const int tb = rev ? 3 - (int)pac_get(ix.pac, tbase + i) : (int)pac_get(ix.pac, tbase + i);
-                            const int* mrow = smat + tb * 5;
-                            uint32_t* zi = Z + (size_t)i * ZROW * 32;
-                            cells += (unsigned long long)(end - beg);
-                            uint32_t zpack = 0; int zsh = 0;
-                            // walking pointers: circular row window (wraps after NARROW_NC columns), staged query column
-                            int* hp = H + (beg & (NARROW_NC - 1)) * NARROW_THREADS;
-                            int* const hwrap = H + NARROW_NC * NARROW_THREADS;
-                            const uint8_t* qp = Q + beg * NARROW_THREADS;
-                            for (int j = beg; j < end; ++j) {
-                                int m = hp[0], e = hp[NARROW_NC * NARROW_THREADS];
-                                hp[0] = h1;
-                                m += mrow[*qp];
-                                int d = m >= e ? 0 : 1;
-                                int h = m >= e ? m : e;
-                                d = h >= f ? d : 2;
-                                h = h >= f ? h : f;
-                                h1 = h;
-                                int tt = m - oe_del;
-                                e -= e_del;
-                                d |= e > tt ? 1 << 2 : 0;
-                                e = e > tt ? e : tt;
-                                hp[NARROW_NC * NARROW_THREADS] = e;
-                                tt = m - oe_ins;
-                                f -= e_ins;
-                                d |= f > tt ? 2 << 4 : 0;
-                                f = f > tt ? f : tt;
-                                zpack |= (uint32_t)d << zsh;
-                                zsh += 8;
-                                if (zsh == 32) { *zi = zpack; zi += 32; zpack = 0; zsh = 0; }
-                                hp += NARROW_THREADS; if (hp == hwrap) hp = H;
-                                qp += NARROW_THREADS;
-                            }
-                            if (zsh) *zi = zpack;
-                            const int ce = (end & (NARROW_NC - 1)) * NARROW_THREADS;
-                            H[ce] = h1; E[ce] = KSW_NEG_INF;
-                        }
-                        score = H[(lq & (NARROW_NC - 1)) * NARROW_THREADS];
                         }
                         // traceback
                         {
@@ -872,7 +798,7 @@ __global__ void __launch_bounds__(NARROW_THREADS, MODE == 5 ? 10 : (MODE >= 3 ? 
                                 else cg[n_cigar - 1] += len << 4;
                             };
                             while (i >= 0 && k >= 0) {
-                                const int jj = MODE != 0 ? k - i + WTM : k - (i > w ? i - w : 0);
+                                const int jj = k - i + WTM;
                                 which = (int)(Z[((size_t)i * ZROW + (jj >> 2)) * 32] >> ((jj & 3) << 3) & 0xff) >> (which << 1) & 3;
                                 if (which == 0) { push(0, 1); --i; --k; }
                                 else if (which == 1) { push(2, 1); --i; }
@@ -883,7 +809,6 @@ __global__ void __launch_bounds__(NARROW_THREADS, MODE == 5 ? 10 : (MODE >= 3 ? 
                             if (full) { go_wide = true; break; }
                             for (int a = 0; a < n_cigar >> 1; ++a) { uint32_t x = cg[a]; cg[a] = cg[n_cigar - 1 - a]; cg[n_cigar - 1 - a] = x; }
                         }
-                        (void)n_col;
                     }
                     // NM
                     int x = 0, y = 0, n_mm = 0, n_gap = 0;
@@ -894,7 +819,7 @@ __global__ void __launch_bounds__(NARROW_THREADS, MODE == 5 ? 10 : (MODE >= 3 ? 
                             bool fast = false;
                             int mm = 0;
                             // a run of M: q[x .. x+len) against the reference from y on -- the packed comparison of the diagonal pass
-                            if (MODE != 0 && len >= 16) mm = diag_mismatches(rev ? qg + (lq - x - len) : qg + x, len, rev, ix.pac, tbase + y, &fast);
+                            if (len >= 16) mm = diag_mismatches(rev ? qg + (lq - x - len) : qg + x, len, rev, ix.pac, tbase + y, &fast);
                             if (fast) n_mm += mm;
                             else for (int i = 0; i < len; ++i) {
                                 const int tb = rev ? 3 - (int)pac_get(ix.pac, tbase + y + i) : (int)pac_get(ix.pac, tbase + y + i);
@@ -907,11 +832,11 @@ __global__ void __launch_bounds__(NARROW_THREADS, MODE == 5 ? 10 : (MODE >= 3 ? 
                     NM = n_mm + n_gap;
                 }
                 if (score == jb.last_sc || w2 == o.w << 2) break;
-                if (P.diag_pass && !reject && lq == rlen && !(lq == rlen && w2 == 0)) break;   // band-independent result (see above)
+                if (diag_pass && !reject && lq == rlen && !(lq == rlen && w2 == 0)) break;   // band-independent result (see above)
                 if (jb.it + 1 < 3 && score < ar.truesc - o.a) {
                     again = true;
                     NarrowJob nx; nx.r = r; nx.slot = slot; nx.w2 = w2 << 1; nx.last_sc = score; nx.it = jb.it + 1; nx.score = score;
-                    push_narrow(P.requeue, P.requeue_cap, P.requeue_cnt, P.requeue_big_cnt, nx, narrow_is_big(o, lq, rlen, nx.w2, simple_mat));
+                    push_narrow(P.requeue, P.requeue_cap, P.requeue_cnt, P.requeue_big_cnt, nx, narrow_is_big(o, lq, rlen, nx.w2));
                 }
             } while (false);
             if (go_wide) {
@@ -1025,36 +950,17 @@ int finalize_resident_warps() {
     return cached_blocks_per_sm(regs_finalize<false>, FIN_THREADS, 0) * cached_sm_count() * FIN_WARPS;
 }
 
-// resident warps of the two thread-per-region kernels and their traceback buffers (the kernels of a DP pass run side by side, so
-// each has its own: the register kernel's first, the shared-memory kernel's behind it)
-static void narrow_geometry(int* warps_smem, int* warps_reg, int* warps_reg2, size_t* zbytes_reg, size_t* zbytes_smem, int* warps_reg3 = nullptr, int* warps_reg4 = nullptr) {
-    const size_t smem = (size_t)NARROW_THREADS * (2 * NARROW_NC * 4 + NARROW_QMAX);
-    const int nb = cached_blocks_per_sm(regs_cigar_narrow<0>, NARROW_THREADS, smem), nr = cached_blocks_per_sm(regs_cigar_narrow<1>, NARROW_THREADS, 0);
-    const int nr2 = cached_blocks_per_sm(regs_cigar_narrow<2>, NARROW_THREADS, 0);
-    const int sms = cached_sm_count();
-    const int ws = nb * sms * (NARROW_THREADS / 32), wr = nr * sms * (NARROW_THREADS / 32), wr2 = nr2 * sms * (NARROW_THREADS / 32);
-    if (warps_smem) *warps_smem = ws;
-    if (warps_reg) *warps_reg = wr;
-    if (warps_reg2) *warps_reg2 = wr2;
-    // the back-section kernel is either the shared-memory one or the wide register one: one buffer, sized for the larger
-    const size_t zs = (size_t)ws * NARROW_TMAX * NARROW_NC * 32, z2 = (size_t)wr2 * NARROW_TMAX * ((2 * REG_WT2 + 1 + 3) / 4) * 4 * 32;
-    if (zbytes_smem) *zbytes_smem = zs > z2 ? zs : z2;
-    const int wr3 = cached_blocks_per_sm(regs_cigar_narrow<3>, NARROW_THREADS, 0) * sms * (NARROW_THREADS / 32);
-    const int wr4 = cached_blocks_per_sm(regs_cigar_narrow<4>, NARROW_THREADS, 0) * sms * (NARROW_THREADS / 32);
-    if (warps_reg3) *warps_reg3 = wr3;
-    if (warps_reg4) *warps_reg4 = wr4;
-    const size_t z1 = (size_t)wr * NARROW_TMAX * ((2 * REG_WT + 1 + 3) / 4) * 4 * 32, z3 = (size_t)wr3 * NARROW_TMAX * ((2 * REG_WT3 + 1 + 3) / 4) * 4 * 32;
-    const size_t z4 = (size_t)wr4 * NARROW_TMAX * ((2 * REG_WT4 + 1 + 3) / 4) * 4 * 32;
-    const size_t zm = z1 > z3 ? z1 : z3;
-    if (zbytes_reg) *zbytes_reg = zm > z4 ? zm : z4;    // the tight passes run alone and share the first buffer
+// resident CTAs of a thread-per-region kernel on the whole chip (a launch fills it once; the kernel takes jobs by ticket)
+template <int MODE> static int narrow_blocks() { return cached_blocks_per_sm(regs_cigar_narrow<MODE>, NARROW_THREADS, 0) * cached_sm_count(); }
+// traceback buffer of a kernel whose register window has half-width wt
+static size_t narrow_z_bytes(int blocks, int wt) { return (size_t)blocks * (NARROW_THREADS / 32) * NARROW_TMAX * ((2 * wt + 1 + 3) / 4) * 4 * 32; }
+// The two kernels of a DP pass run side by side, so each has its own traceback buffer: MODE 1's first (the tight passes run alone
+// and share it), MODE 2's behind it.
+static size_t narrow_z_front() {
+    return std::max(narrow_z_bytes(narrow_blocks<1>(), REG_WT), std::max(narrow_z_bytes(narrow_blocks<3>(), REG_WT3), narrow_z_bytes(narrow_blocks<4>(), REG_WT4)));
 }
 
-size_t narrow_zbuf_bytes(int* n_warps_out) {
-    int ws = 0; size_t zr = 0, zs = 0;
-    narrow_geometry(&ws, nullptr, nullptr, &zr, &zs);
-    if (n_warps_out) *n_warps_out = ws;
-    return zr + zs;
-}
+size_t narrow_zbuf_bytes() { return narrow_z_front() + narrow_z_bytes(narrow_blocks<2>(), REG_WT2); }
 
 void launch_finalize(const FinalizeParams& p, const DevIndex& ix, const DevOpts& o, cudaStream_t st, uint32_t rseq_cap, int n_warps, uint64_t* launches, const ExtAux* aux) {
     const uint32_t cig_cap = fin_cig_cap(p.max_len, rseq_cap);
@@ -1073,26 +979,15 @@ void launch_finalize(const FinalizeParams& p, const DevIndex& ix, const DevOpts&
     if (!p.narrow_jobs) return;
     // phase 2: thread-per-region narrow-band mem_reg2aln, one try of the band-doubling loop per pass (<= 3 tries)
     {
-        int warps = 0, warps_reg = 0, warps_reg2 = 0, warps_reg3 = 0, warps_reg4 = 0; size_t z_reg = 0;
-        narrow_geometry(&warps, &warps_reg, &warps_reg2, &z_reg, nullptr, &warps_reg3, &warps_reg4);
-        // the scoring matrix of this path is mem_opt_init's and never changes (SURVEY B#5): match / mismatch / N, which is what the
-        // register kernels assume; any other matrix takes the shared-memory kernel
-        bool simple = true;
-        for (int a = 0; a < 5 && simple; ++a) for (int c = 0; c < 5; ++c) {
-            const int want = (a == 4 || c == 4) ? o.mat[4] : (a == c ? o.mat[0] : o.mat[1]);
-            if (o.mat[a * 5 + c] != want) { simple = false; break; }
-        }
-        static const bool no_reg2 = getenv("BSQ_FIN_NO_REG2") != nullptr;
         NarrowJob* listA = reinterpret_cast<NarrowJob*>(p.narrow_jobs);
         NarrowJob* listB = listA + p.narrow_cap;
         NarrowJob* listS = listA + 2 * (size_t)p.narrow_cap;
         NarrowJob* listT4 = listA + 3 * (size_t)p.narrow_cap;
         NarrowJob* listT8 = listA + 4 * (size_t)p.narrow_cap;
-        const size_t nsmem = (size_t)NARROW_THREADS * (2 * NARROW_NC * 4 + NARROW_QMAX);
         for (int pass = 0; pass < 4; ++pass) {
             // pass 0: equal-length regions (list S): diagonal proof, the rest joins list A; pass 1: DP regions (A -> re-queue B);
             // pass 2: second tries (B -> A); pass 3: third tries (A).  A DP pass is two launches: the register-band kernel on
-            // the front section of the list, the shared-memory kernel on the back section (bands wider than the register window).
+            // the front section of the list, the wide register-band kernel on the back section (bands wider than REG_WT).
             // counters: 0 A front, 1 B front, 2 A front (third tries), 3 S, 4 sink, 5 A back, 6 B back, 7 A back (third tries)
             NarrowParams q;
             q.seqs = p.seqs; q.offs = p.offs; q.regs = p.regs; q.rows = p.rows;
@@ -1101,37 +996,31 @@ void launch_finalize(const FinalizeParams& p, const DevIndex& ix, const DevOpts&
             q.requeue_cnt = p.narrow_cnt + (pass == 0 ? 0 : (pass == 1 ? 1 : (pass == 2 ? 2 : 4)));   // pass 3 never re-queues
             q.requeue_big_cnt = p.narrow_cnt + (pass == 0 ? 5 : (pass == 1 ? 6 : (pass == 2 ? 7 : 4)));
             q.wide_jobs = p.wide_jobs; q.wide_cnt = p.wide_cnt; q.cigar_pool = p.cigar_pool; q.cigar_cap = p.cigar_cap; q.cigar_top = p.cigar_top;
-            q.zbuf = p.narrow_z; q.overflow = p.overflow; q.counters = p.counters; q.diag_pass = pass == 0;
-            q.tight = p.narrow_tight && simple ? listT4 : nullptr; q.tight_cnt = p.narrow_cnt + NARROW_T4_CNT;
-            { static const bool btw = getenv("BSQ_FIN_BIG_TO_WIDE") != nullptr; q.big_go_wide = btw; }
+            q.zbuf = p.narrow_z; q.overflow = p.overflow; q.counters = p.counters;
+            q.tight = listT4; q.tight_cnt = p.narrow_cnt + NARROW_T4_CNT;
             { static const uint32_t sl = getenv("BSQ_FIN_SHORT_LIST") ? (uint32_t)atoi(getenv("BSQ_FIN_SHORT_LIST")) : NARROW_SHORT_LIST; q.short_list = sl; }
             q.jobs = in; q.job_stride = 1; q.ticket = p.ticket + 1 + pass;
             q.n_jobs = p.narrow_cnt + (pass == 0 ? 3 : (pass == 1 ? 0 : (pass == 2 ? 1 : 2)));
             if (pass == 0) {
                 // the diagonal proof needs no band state: a build of the kernel without the DP (12 CTAs per SM)
-                static const int warps_diag = cached_blocks_per_sm(regs_cigar_narrow<5>, NARROW_THREADS, 0) * cached_sm_count() * (NARROW_THREADS / 32);
-                regs_cigar_narrow<5><<<warps_diag / (NARROW_THREADS / 32), NARROW_THREADS, 0, st>>>(q, ix, o);
-                if (launches) ++*launches;
-                if (q.tight) {
-                    // passes T4, T8: every first try whose end cell fits the tight window; what T4 cannot prove goes to T8, what T8
-                    // cannot prove joins list A -- always the same try
-                    q.diag_pass = 0; q.jobs = listT4; q.n_jobs = p.narrow_cnt + NARROW_T4_CNT; q.ticket = p.ticket + 9;
-                    q.tight = listT8; q.tight_cnt = p.narrow_cnt + NARROW_T8_CNT;
-                    regs_cigar_narrow<4><<<warps_reg4 / (NARROW_THREADS / 32), NARROW_THREADS, 0, st>>>(q, ix, o);
-                    q.jobs = listT8; q.n_jobs = p.narrow_cnt + NARROW_T8_CNT; q.ticket = p.ticket + 10; q.tight = nullptr;
-                    regs_cigar_narrow<3><<<warps_reg3 / (NARROW_THREADS / 32), NARROW_THREADS, 0, st>>>(q, ix, o);
-                    if (launches) *launches += 2;
-                }
+                regs_cigar_narrow<5><<<narrow_blocks<5>(), NARROW_THREADS, 0, st>>>(q, ix, o);
+                // passes T4, T8: every first try whose end cell fits the tight window; what T4 cannot prove goes to T8, what T8
+                // cannot prove joins list A -- always the same try
+                q.jobs = listT4; q.n_jobs = p.narrow_cnt + NARROW_T4_CNT; q.ticket = p.ticket + 9;
+                q.tight = listT8; q.tight_cnt = p.narrow_cnt + NARROW_T8_CNT;
+                regs_cigar_narrow<4><<<narrow_blocks<4>(), NARROW_THREADS, 0, st>>>(q, ix, o);
+                q.jobs = listT8; q.n_jobs = p.narrow_cnt + NARROW_T8_CNT; q.ticket = p.ticket + 10;
+                regs_cigar_narrow<3><<<narrow_blocks<3>(), NARROW_THREADS, 0, st>>>(q, ix, o);
+                if (launches) *launches += 3;
             } else {
                 // the two kernels of a DP pass work on disjoint sections of the list: side by side when a side stream is there
                 cudaStream_t s2 = aux ? aux->st[0] : st;
                 if (aux) { cudaEventRecord(aux->ev[0], st); cudaStreamWaitEvent(s2, aux->ev[0], 0); }
-                regs_cigar_narrow<1><<<warps_reg / (NARROW_THREADS / 32), NARROW_THREADS, 0, st>>>(q, ix, o);
+                regs_cigar_narrow<1><<<narrow_blocks<1>(), NARROW_THREADS, 0, st>>>(q, ix, o);
                 q.jobs = in + p.narrow_cap - 1; q.job_stride = -1; q.ticket = p.ticket + 5 + pass;      // tickets 6..8
                 q.n_jobs = p.narrow_cnt + (pass == 1 ? 5 : (pass == 2 ? 6 : 7));
-                q.zbuf = p.narrow_z + z_reg;
-                if (simple && !no_reg2) regs_cigar_narrow<2><<<warps_reg2 / (NARROW_THREADS / 32), NARROW_THREADS, 0, s2>>>(q, ix, o);
-                else regs_cigar_narrow<0><<<warps / (NARROW_THREADS / 32), NARROW_THREADS, nsmem, s2>>>(q, ix, o);
+                q.zbuf = p.narrow_z + narrow_z_front();
+                regs_cigar_narrow<2><<<narrow_blocks<2>(), NARROW_THREADS, 0, s2>>>(q, ix, o);
                 if (aux) { cudaEventRecord(aux->ev[1], s2); cudaStreamWaitEvent(st, aux->ev[1], 0); }
                 if (launches) *launches += 2;
             }

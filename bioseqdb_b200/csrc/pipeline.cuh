@@ -64,7 +64,7 @@ struct ExtendParams {
 void launch_extend(const ExtendParams& p, const DevIndex& ix, const DevOpts& o, cudaStream_t st);
 void launch_extend_finish(const ExtendParams& p, const DevIndex& ix, const DevOpts& o, cudaStream_t st);
 struct ExtAux { cudaStream_t st[3]; cudaEvent_t ev[4]; };
-void launch_extend_memo(const ExtendParams& p, const DevIndex& ix, const DevOpts& o, cudaStream_t st, uint64_t* launches, const ExtAux* aux);
+void launch_extend_memo(const ExtendParams& p, const DevIndex& ix, const DevOpts& o, cudaStream_t st, uint64_t* launches, const ExtAux& aux);
 constexpr int EXT_MEMO_BINS = 160;
 size_t extend_scratch_per_warp(uint32_t max_len, uint32_t rseq_cap);
 int extend_resident_warps();
@@ -102,19 +102,18 @@ struct FinalizeParams {
     const int64_t* ann_id;
     // narrow-band regions are queued (read << 32 | row slot) for the thread-per-region kernel; regions that
     // need a wider band on a retry come back through wide_jobs.  narrow_jobs == nullptr disables the split.
-    bool narrow_tight = true;      // first tries go through the tight-band pass (lists T4, T8 of narrow_jobs)
     void* narrow_jobs; uint32_t narrow_cap;   // five lists of narrow_cap job records (24 B each): A, B (ping-pong between tries), S (equal-length regions), T4, T8 (tight first tries)
     uint32_t* narrow_cnt;                     // eight consecutive counters: list A, list B, list A (third tries), list S, sink, wide-band hand-over lists of passes 1..3
-    uint64_t* wide_jobs; uint32_t* wide_cnt; uint8_t* narrow_z; int narrow_warps;
-    uint32_t* ticket;              // eleven consecutive tickets: finalize, narrow pass 0..3, wide, shared-memory narrow kernel of passes 1..3, the two tight passes
+    uint64_t* wide_jobs; uint32_t* wide_cnt; uint8_t* narrow_z;
+    uint32_t* ticket;              // eleven consecutive tickets: finalize, narrow pass 0..3, wide, wide register-band narrow kernel of passes 1..3, the two tight passes
     uint32_t* overflow;
     uint32_t* need_rseq;           // see ExtendParams
     unsigned long long* counters;  // optional: [0] = ksw_global2 cells, [1] = calls
     uint32_t* todo; uint32_t* todo_cnt;   // reads the thread-per-read pass left for regs_finalize (nullptr = no thread pass)
 };
 struct ExtAux;
-// aux (optional): side streams + events; the two kernels of a DP pass (register band / shared-memory band) then run side by side
+// aux (optional): side streams + events; the two kernels of a DP pass (register band / wide register band) then run side by side
 void launch_finalize(const FinalizeParams& p, const DevIndex& ix, const DevOpts& o, cudaStream_t st, uint32_t rseq_cap, int n_warps, uint64_t* launches, const ExtAux* aux);
-size_t narrow_zbuf_bytes(int* n_warps_out);
+size_t narrow_zbuf_bytes();
 size_t finalize_scratch_per_warp(uint32_t max_len, uint32_t rseq_cap, uint32_t* z_cap_out);
 int finalize_resident_warps();

@@ -15,7 +15,6 @@
 #include "seed_thread.cuh"
 #include "launch_cache.cuh"
 #include <algorithm>
-#include <cstdlib>
 
 namespace {
 
@@ -23,7 +22,7 @@ constexpr int SEED_THREADS = 256;
 constexpr int SEED_WARPS = SEED_THREADS / 32;
 // prefix table: bi-intervals of every t-mer, t = 1..K, levels back to back.  K is chosen per index, about log4 of the text
 // length, so that a K-mer has a handful of occurrences at most: 12 -> 358 MB, 13 -> 1.4 GB, 14 -> 5.7 GB (of 180 GB HBM)
-constexpr int KMER_K_MAX = 14;      // automatic choice; BSQ_KMER_K may ask for 15 (23 GB)
+constexpr int KMER_K_MAX = 14;      // choice by text length; ensure_kmer_table goes to 15 (23 GB) where HBM allows
 __host__ __device__ constexpr uint32_t kmer_level_off(int t) { return (0x55555555u >> (32 - 2 * t)) - 1u; }   // first entry of level t = (4^t - 4) / 3, 1 <= t <= 16
 
 template <class IdxT> struct IvT { IdxT x0, x1; uint32_t x2, info; };   // info = end of the match on the query
@@ -530,7 +529,7 @@ __device__ __forceinline__ void collect_intv(const Ctx<IdxT>& C, const DevOpts& 
         // evaluates f(x + t L) on its own -- K-mer from the prefix table, then (unique K-mer) one text comparison of the
         // remaining L - K bases -- so the dependent loads of up to 32 starts are in flight together; the chain then consumes
         // the results in order for as long as each start is the predicted one and was decidable without Occ.
-        const bool spec_ok = C.kmer_tab != nullptr && C.isa != nullptr && pk != nullptr && !has_n &&
+        const bool spec_ok = C.kmer_tab != nullptr && pk != nullptr && !has_n &&
                              min_len >= C.kk && o.max_mem_intv > 1 && L <= 32;
         const int lane = C.lane;
         while (x < len) {
@@ -976,22 +975,18 @@ bool seed_lists_fit_smem(uint32_t list_cap, uint32_t read_cap, int sa_bytes) {
 void launch_seed(const SeedParams& p, const DevIndex& ix, const DevOpts& o, cudaStream_t st, int* n_warps_out) {
     const bool wide = ix.sa_bytes == 8;   // 64-bit row indices
     if (wide) {
-        static const int ctas = getenv("BSQ_SEED_WIDE_CTAS") ? atoi(getenv("BSQ_SEED_WIDE_CTAS")) : 3;
-        if (p.lists_in_smem) {
-            if (ctas >= 3) launch_mode<uint64_t, true, 3>(p, ix, o, st, lists_bytes<uint64_t>(p.list_cap, p.read_cap), n_warps_out);
-            else launch_mode<uint64_t, true, 2>(p, ix, o, st, lists_bytes<uint64_t>(p.list_cap, p.read_cap), n_warps_out);
-        } else launch_mode<uint64_t, false, 1>(p, ix, o, st, 0, n_warps_out);
+        if (p.lists_in_smem) launch_mode<uint64_t, true, 3>(p, ix, o, st, lists_bytes<uint64_t>(p.list_cap, p.read_cap), n_warps_out);
+        else launch_mode<uint64_t, false, 1>(p, ix, o, st, 0, n_warps_out);
     } else {
         if (p.lists_in_smem) launch_mode<uint32_t, true, 4>(p, ix, o, st, lists_bytes<uint32_t>(p.list_cap, p.read_cap), n_warps_out);
         else launch_mode<uint32_t, false, 1>(p, ix, o, st, 0, n_warps_out);
     }
 }
 
-// The thread-per-read pass takes a batch when the prefix table and the inverse SA exist, seeds are longer than the table is deep
-// (so that an emitted match always carries its rows) and the reads fit its packed shared-memory copy and 9-bit sort key.
+// The thread-per-read pass takes a batch when the prefix table (and with it the inverse SA) exists, seeds are longer than the table
+// is deep (so that an emitted match always carries its rows) and the reads fit its packed shared-memory copy and 9-bit sort key.
 bool seed_thread_usable(const SeedParams& p, const DevOpts& o, uint32_t max_len) {
-    static const bool off = getenv("BSQ_NO_SEED_THREAD") != nullptr;
-    return !off && p.kmer_tab && p.isa && p.todo && p.pk && o.min_seed_len > p.kmer_k && o.max_mem_intv > 1 && max_len <= 496 && p.cap / 2 >= 16 && p.cap / 2 <= 64;
+    return p.kmer_tab && p.todo && p.pk && o.min_seed_len > p.kmer_k && o.max_mem_intv > 1 && max_len <= 496 && p.cap / 2 >= 16 && p.cap / 2 <= 64;
 }
 
 int seed_thread_words(uint32_t max_len) { return (int)(max_len >> 4) + 3; }
@@ -1010,9 +1005,7 @@ int launch_seed_thread(const SeedParams& p, const DevIndex& ix, const DevOpts& o
         seed_calls<uint64_t><<<nb * sms, ST_THREADS, smem, st>>>(p, ix, o, ticket, words);
         seed_last<uint64_t><<<last_blocks, ST_THREADS, smem, st>>>(p, ix, o, words);
     } else {
-        int nb = cached_blocks_per_sm(seed_calls<uint32_t>, ST_THREADS, smem);
-        static const int cap = getenv("BSQ_SEED_CTAS") ? atoi(getenv("BSQ_SEED_CTAS")) : 0;
-        if (cap > 0 && cap < nb) nb = cap;
+        const int nb = cached_blocks_per_sm(seed_calls<uint32_t>, ST_THREADS, smem);
         seed_calls<uint32_t><<<nb * sms, ST_THREADS, smem, st>>>(p, ix, o, ticket, words);
         seed_last<uint32_t><<<last_blocks, ST_THREADS, smem, st>>>(p, ix, o, words);
     }

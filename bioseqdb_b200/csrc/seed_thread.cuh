@@ -60,7 +60,7 @@ template <class IdxT> struct Index {
     const uint32_t* occ; const U4* tab; int kk;
     const uint32_t* ztab;    // sizes only (the .z of every table entry, same indexing): what the walks compare; 4 bytes per entry, so the
                              // levels that stay in L2 reach two levels deeper than with the 16-byte entries (nullptr: read tab)
-    const IdxT* sa; const IdxT* isa; const uint8_t* pac;
+    const IdxT* sa; const IdxT* isa; const uint8_t* pac;    // the inverse SA is always there: the pass runs only beside the prefix table
     IdxT l_pac, n, primary; IdxT L2[5];
 };
 struct Opts { int min_seed_len, split_len, split_width, max_mem_intv; };
@@ -281,7 +281,7 @@ ST_HD void smem_forward(const Index<IdxT>& X, const Read& R, int x, uint32_t min
         const U4 e = ld_u4(X.tab + level_off(maxt) + (w0 >> (32 - 2 * maxt)));
         Iv<IdxT> ik; ik.x0 = tab_x0<IdxT>(e); ik.x1 = tab_x1<IdxT>(e); ik.x2 = cur_x2;
         for (; i < len; ++i) {
-            if (X.isa && ik.x2 == 1 && min_intv == 1) {
+            if (ik.x2 == 1 && min_intv == 1) {
                 // unique match q[x .. i): walk to the first base that does not match (or the end of the read) by text comparison
                 const IdxT pos = ld_idx(X.sa + ik.x0);
                 const int run = match_run_fwd(X, R, (IdxT)(pos + (IdxT)(i - x)), i, len - i);
@@ -333,7 +333,7 @@ template <class IdxT>
 ST_HD void smem_column(const Index<IdxT>& X, const Opts& o, const Read& R, int k, Work<IdxT>& W, bool live) {
     const int K = X.kk, x = W.x;
     const uint32_t min_intv = W.min_intv;
-    const bool can_uq = X.isa != nullptr && min_intv == 1;
+    const bool can_uq = min_intv == 1;
     int end = 0, b = 0, i = x - 1, nb = 0;
     uint32_t cur = 0; IdxT x0 = 0, x1 = 0; bool rows = false;
     if (live) {
@@ -443,7 +443,7 @@ ST_HD int seed_strategy1(const Index<IdxT>& X, const Opts& o, const Read& R, int
         return len;
     }
     for (; i < len; ++i) {
-        if (X.isa && ik.x2 == 1 && max_intv > 1 && i - x <= min_len) {
+        if (ik.x2 == 1 && max_intv > 1 && i - x <= min_len) {
             // unique match q[x .. i): the walk ends at j = x + min_len (emit iff still matching) or at the end of the read
             const int stop = x + min_len;
             const int lim = (stop < len ? stop + 1 : len) - i;       // bases q[i .. i + lim) are looked at
@@ -474,7 +474,7 @@ constexpr int MWL = 4;                       // K-mer occurrences the LAST-like 
 template <class IdxT> ST_HD void last_like_pass(const Index<IdxT>& X, const Opts& o, const Read& R, Work<IdxT>& W) {
     if (o.max_mem_intv <= 0) return;
     const int len = R.len, K = X.kk, min_len = o.min_seed_len, L = min_len + 1;
-    const bool spec_ok = X.isa != nullptr && o.max_mem_intv > 1 && min_len >= K;
+    const bool spec_ok = o.max_mem_intv > 1 && min_len >= K;
     int x = 0;
     while (x < len && !W.fail) {
         const int nb = spec_ok ? ((len - x) / L < LAST_BATCH ? (len - x) / L : LAST_BATCH) : 0;   // starts whose whole L-mer lies in the read

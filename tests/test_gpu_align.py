@@ -1,5 +1,7 @@
 """End-to-end parity through the C ABI (bsq_align_batch) vs the oracle: identical ordered rows --
 rid, rb, re, qb, qe, strand, score, truesc, secondary, sub, sub_n, CIGAR, NM, MAPQ, hash order."""
+import ctypes as C
+
 import numpy as np
 import pytest
 
@@ -166,23 +168,44 @@ def _flat_cigars(res):
     return res.cigar[idx]
 
 
-def test_align_batch_chunked_pipeline(gpu_lib):
+def _own_result(gpu, call):
+    """a result as the library hands it out (`call` fills the bsq_result pointer), so that bsq_result_tuples recognises it as its own"""
+    from bioseqdb_b200._lib import BsqResult, check
+    res = C.POINTER(BsqResult)()
+    check(call(C.byref(res)))
+    return res
+
+
+def test_align_batch_chunked_pipeline(gpu_lib, monkeypatch):
     """bsq_align_batch cuts a large batch into chunks on two lanes (copies overlapped with compute): rows, their order
-    and the rebased CIGAR offsets must equal the single-lane resident path's, and the oracle's on a sample."""
+    and the rebased CIGAR offsets must equal the single-lane resident path's, and the oracle's on a sample.  With three chunks
+    the lanes no longer hold the whole result: its tuples take the path that uploads rows and reads, and must equal the tuples
+    the resident batch of the same reads serves."""
     from helpers import PARITY_FIELDS
+    from bioseqdb_b200._lib import ptr
+    monkeypatch.setenv("BSQ_CHUNK_READS", str(1 << 17))
     rows = synth.reference_rows([600_001, 400_003], seed=71)
     rows = synth.plant_repeats(rows, n_families=6, copies=6, unit=(200, 800), divergence=0.02)
     orc, gpu = build_pair(rows, O.sql_default_opts(2))
     n = 2 * (1 << 17) + 12_345                      # two full chunks and a ragged third
     seqs, offs, _ = synth.simulate_reads(rows, n, 100, sub=0.015, ins=0.002, dele=0.002, seed=72, n_frac=0.001)
     ids = synth.lrand48_ids_fast(n)
-    g = gpu.align_batch(seqs, offs, ids)             # chunked
-    assert gpu.timing().launches > 40                # more launches than one pass of the pipeline: the chunks really ran
-    gpu.upload(seqs, offs, ids); gpu.align_resident(); r = gpu.download_result()
+    g_res = _own_result(gpu, lambda p: gpu.L.bsq_align_batch(gpu.h, ptr(seqs), ptr(offs), ptr(ids), n, p))   # chunked
+    chunked_launches = gpu.timing().launches
+    g_tup = gpu._fetch_tuples(g_res, ptr(seqs), ptr(offs), 0)
+    g = gpu._collect(g_res)
+    gpu.upload(seqs, offs, ids); gpu.align_resident()
+    # three pipeline passes; two would stay below three resident passes (the chunks add only a few copy kernels each)
+    assert chunked_launches >= 3 * gpu.timing().launches
+    r_res = _own_result(gpu, lambda p: gpu.L.bsq_result_download(gpu.h, p))
+    r_tup = gpu._fetch_tuples(r_res, None, None, 0)      # served from the resident batch: nothing uploaded
+    r = gpu._collect(r_res)
     assert np.array_equal(g.row_off, r.row_off)
     for f in PARITY_FIELDS:
         assert np.array_equal(g.rows[f], r.rows[f]), f
     assert np.array_equal(_flat_cigars(g), _flat_cigars(r))
+    assert np.array_equal(g_tup.off, r_tup.off) and np.array_equal(g_tup.ref_match, r_tup.ref_match)
+    assert np.array_equal(g_tup.data, r_tup.data)
     # the oracle on reads that straddle the chunk boundaries and the tail
     pick = np.concatenate([np.arange((1 << 17) - 600, (1 << 17) + 600), np.arange(2 * (1 << 17) - 600, 2 * (1 << 17) + 600), np.arange(n - 800, n)])
     s_offs = np.zeros(len(pick) + 1, dtype=np.uint64)

@@ -40,14 +40,17 @@ def test_datum_batch_equals_ascii_batch(gpu_lib):
 
 def test_datum_batch_chunked(gpu_lib, monkeypatch):
     """large batch => the two-lane chunk pipeline; chunks are cut out of the datum block by their offsets"""
-    monkeypatch.setenv("BSQ_CHUNK_READS", "20000")
+    monkeypatch.setenv("BSQ_CHUNK_READS", "65536")
     rows = synth.reference_rows([400_001], seed=111)
     _, gpu = build_pair(rows, O.sql_default_opts(1))
-    seqs, offs, _ = synth.simulate_reads(rows, 90_123, 100, seed=112)
+    seqs, offs, _ = synth.simulate_reads(rows, 2 * 65536 + 4321, 100, seed=112)     # 2 x 64 K reads at least: the batch is chunked
     ids = synth.lrand48_ids_fast(len(offs) - 1)
     data, off, _ = nuclseq_image_block(seqs, offs)
     d = gpu.align_batch_datums(data, off, ids)
-    gpu.upload(seqs, offs, ids); gpu.align_resident(); r = gpu.download_result()
+    chunked_launches = gpu.timing().launches
+    gpu.upload(seqs, offs, ids); gpu.align_resident()
+    assert chunked_launches >= 3 * gpu.timing().launches     # three chunks ran, each a pipeline pass
+    r = gpu.download_result()
     _same(d, r)
 
 
