@@ -5,6 +5,7 @@ Everything below the class runs on the GPU through the C ABI (include/bioseqdb_g
 from __future__ import annotations
 
 import ctypes as C
+import os
 from dataclasses import dataclass
 
 import numpy as np
@@ -190,6 +191,27 @@ class BwaIndex:
         m = BsqMeta()
         check(self.L.bsq_index_get_meta(self.h, C.byref(m)))
         return m
+
+    def save(self, path, key: bytes | None = None):
+        """Write the built index to one file (bsq_index_save): pac, Occ, annotations, host state and every 32nd suffix-array entry.
+        The file appears under `path` only when complete.  key: 16 opaque bytes kept in the header (BwaIndexCache stores its digest)."""
+        check(self.L.bsq_index_save(self.h, os.fsencode(path), _key_arg(key)))
+
+    def load(self, path, key: bytes | None = None) -> float:
+        """Fill this fresh index (nothing added, not built) from a file written by save(); the full suffix array is rebuilt on the GPU.
+        key: when given, the file's key must equal it.  Returns the wall milliseconds of the load."""
+        ms = C.c_float(0)
+        check(self.L.bsq_index_load(self.h, os.fsencode(path), _key_arg(key), C.byref(ms)))
+        self.n_rows = int(self.meta().n_anns)        # max_occ's default counts the rows, as replica_finish does
+        self._view = None
+        return float(ms.value)
+
+    def last_load(self) -> dict:
+        """Where the last load() spent its time (bsq_index_last_load)."""
+        from ._lib import BsqLoadInfo
+        i = BsqLoadInfo()
+        check(self.L.bsq_index_last_load(self.h, C.byref(i)))
+        return {k: getattr(i, k) for k, _ in BsqLoadInfo._fields_}
 
     def verify(self, n_samples: int = 1 << 22, seed: int = 20261018) -> dict:
         """Device-side check of the index against its text (bsq_index_verify): every `*_bad` must be 0 and every `*_ok` 1."""
@@ -518,6 +540,15 @@ class MultiBwaIndex:
         t = BsqTiming()
         check(self.L.bsq_multi_last_timing(self.m, C.byref(t)))
         return t
+
+
+def _key_arg(key):
+    if key is None:
+        return None
+    key = bytes(key)
+    if len(key) != 16:
+        raise ValueError("an index file key is 16 bytes")
+    return key
 
 
 def _i32(v: int) -> int:

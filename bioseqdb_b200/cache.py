@@ -8,11 +8,18 @@ mem_opt_t, which only the aligner reads) -- and are applied to the cached handle
 
 The reference's per-read id comes from glibc's process-wide lrand48 state, which survives across SQL calls of one
 session; the cache therefore owns that state and lends it to whichever index serves a call.
+
+With a `directory` the cache also has a disk tier, for what one process cannot keep: in PostgreSQL every backend is its own
+process, and a new one would build the same index again.  A built index is written to `<directory>/<digest hex>.bsqidx`
+(BwaIndex.save: atomic replace, the digest kept in the file's header) and a memory miss loads it from there when it exists.
+A file that does not load (damaged, or written for other content) is rebuilt and replaced; a file that cannot be written
+(disk full, read-only directory) costs the next process a build, never this call.
 """
 from __future__ import annotations
 
 import ctypes as C
 import hashlib
+import os
 from collections import OrderedDict
 
 import numpy as np
@@ -32,13 +39,16 @@ def rows_digest(rows) -> bytes:
 
 
 class BwaIndexCache:
-    def __init__(self, device: int = 0, max_bytes: int = 96 << 30, factory=None):
+    def __init__(self, device: int = 0, max_bytes: int = 96 << 30, factory=None, directory=None):
         """max_bytes: HBM budget for resident indexes (index arrays + derived arrays + batch pools, as reported by
-        bsq_index_device_bytes).  factory(device) -> a BwaIndex-like object; defaults to the CUDA-backed BwaIndex."""
+        bsq_index_device_bytes).  factory(device) -> a BwaIndex-like object; defaults to the CUDA-backed BwaIndex.
+        directory: where the disk tier keeps its index files (None: no disk tier)."""
         self.device, self.max_bytes = device, max_bytes
         self._factory = factory
+        self.directory = directory
         self._lru: OrderedDict[bytes, object] = OrderedDict()
         self.hits = self.misses = self.evictions = 0
+        self.disk_hits = self.disk_saves = self.disk_errors = 0
         self.lrand_state = 0
 
     def _new_index(self):
@@ -67,15 +77,45 @@ class BwaIndexCache:
             self.hits += 1
         else:
             self.misses += 1
-            ix = self._new_index()
-            for rid, seq in rows:
-                ix.add_ref_sequence(rid, seq)
-            ix.set_options_from_composite(opts)     # max_occ's default depends on the row count: set before build as the reference does
-            ix.build()
+            # an empty reference builds nothing (bwa.cpp:108-109): there is no index to keep on disk
+            path = self.file_path(key) if self.directory is not None and any(seq.len for _, seq in rows) else None
+            ix = self._load(path, key) if path is not None and os.path.exists(path) else None
+            if ix is None:
+                ix = self._new_index()
+                for rid, seq in rows:
+                    ix.add_ref_sequence(rid, seq)
+                ix.set_options_from_composite(opts)     # max_occ's default depends on the row count: set before build as the reference does
+                ix.build()
+                if path is not None:
+                    self._save(ix, path, key)
             self._lru[key] = ix
             self._evict(keep=key)
         ix.set_options_from_composite(opts)
         return _Lease(self, ix)
+
+    def file_path(self, key: bytes) -> str:
+        return os.path.join(self.directory, key.hex() + ".bsqidx")
+
+    def _load(self, path, key):
+        """The index saved under `path` for `key`, or None when the file does not load (the caller rebuilds and replaces it)."""
+        ix = self._new_index()
+        try:
+            ix.load(path, key=key)
+        except (RuntimeError, OSError, ValueError):
+            self.disk_errors += 1
+            if hasattr(ix, "close"):
+                ix.close()
+            return None
+        self.disk_hits += 1
+        return ix
+
+    def _save(self, ix, path, key):
+        try:
+            ix.save(path, key=key)
+        except (RuntimeError, OSError, ValueError):
+            self.disk_errors += 1            # the index is built and serves this call; only the next process pays
+            return
+        self.disk_saves += 1
 
     def _evict(self, keep):
         while len(self._lru) > 1 and self.total_bytes() > self.max_bytes:

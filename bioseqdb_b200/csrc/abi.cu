@@ -21,6 +21,7 @@
 #include "loader.cuh"
 #include "primitives.cuh"
 #include "debug_kernels.cuh"
+#include "index_file.cuh"
 
 static thread_local char g_err[1024] = "";
 void bsq_set_error(const char* fmt, ...) {
@@ -125,6 +126,7 @@ struct bsq_index {
     uint32_t flags = 0;              // BSQ_FLAG_*
     uint64_t lrand_state = 0;        // glibc lrand48 state of the session (one draw per aligned read when the caller passes no ids)
     bool replica_pending = false;    // device arrays allocated by bsq_index_alloc_replica, host mirrors not yet rebuilt (bsq_index_replica_finish)
+    bsq_index_load_info last_load{};  // the last successful bsq_index_load
     uint64_t counters[8] = {0, 0, 0, 0, 0, 0, 0, 0};
 };
 
@@ -353,9 +355,11 @@ int bsq_index_download(const bsq_index* h, int what, void* dst, uint64_t bytes) 
     return BSQ_OK;
 }
 
-int bsq_index_alloc_replica(bsq_index* h, const bsq_index_meta* m) {
-    BSQ_ENTRY();
-    if (!h || !m || !m->built) { bsq_set_error("bad argument"); return BSQ_ERR; }
+}  // extern "C"
+
+// The arrays of an index described by *m, to be filled from elsewhere (a peer copy, a file); the handle answers once
+// replica_finish has run.
+static int alloc_replica(bsq_index* h, const bsq_index_meta* m) {
     CUDA_CHECK(cudaSetDevice(h->device));
     free_index_arrays(h);
     h->meta = *m;
@@ -369,32 +373,10 @@ int bsq_index_alloc_replica(bsq_index* h, const bsq_index_meta* m) {
     return BSQ_OK;
 }
 
-// Host-side state that has no device copy: the ambiguity holes of the reference rows (copied un-rebased, bwa.cpp:98-104) and the
-// row each one came from.  Blob = u64 n_holes | n_holes x bsq_hole | n_holes x u32 row.
-int bsq_index_host_state_size(const bsq_index* h, uint64_t* bytes) {
-    BSQ_ENTRY();
-    if (!h || !bytes) { bsq_set_error("null argument"); return BSQ_ERR; }
-    *bytes = 8 + h->holes.size() * (sizeof(bsq_hole) + 4);
-    return BSQ_OK;
-}
-
-int bsq_index_host_state_get(const bsq_index* h, void* buf, uint64_t bytes) {
-    BSQ_ENTRY();
-    if (!h || !buf) { bsq_set_error("null argument"); return BSQ_ERR; }
-    const uint64_t nh = h->holes.size();
-    if (bytes < 8 + nh * (sizeof(bsq_hole) + 4)) { bsq_set_error("host-state buffer too small"); return BSQ_ERR; }
-    uint8_t* p = static_cast<uint8_t*>(buf);
-    memcpy(p, &nh, 8);
-    if (nh) { memcpy(p + 8, h->holes.data(), nh * sizeof(bsq_hole)); memcpy(p + 8 + nh * sizeof(bsq_hole), h->hole_ann.data(), nh * 4); }
-    return BSQ_OK;
-}
-
-// After the device arrays of a replica have been filled (broadcast / peer copy): rebuild the host mirrors the row
+// After the device arrays of a replica have been filled (broadcast / peer copy / file): rebuild the host mirrors the row
 // materialisation and the host adapters read -- pac and the annotation vectors from the device copy, the holes from the
 // source's host-state blob -- so that every replica answers exactly like the index it was copied from.
-int bsq_index_replica_finish(bsq_index* h, const void* host_state, uint64_t bytes) {
-    BSQ_ENTRY();
-    if (!h || !h->meta.built) { bsq_set_error("replica not allocated"); return BSQ_ERR; }
+static int replica_finish(bsq_index* h, const void* host_state, uint64_t bytes) {
     CUDA_CHECK(cudaSetDevice(h->device));
     CUDA_CHECK(cudaDeviceSynchronize());
     const bsq_index_meta& m = h->meta;
@@ -420,6 +402,45 @@ int bsq_index_replica_finish(bsq_index* h, const void* host_state, uint64_t byte
     return BSQ_OK;
 }
 
+static __global__ void k_sa_sample(const void* sa, int sa_bytes, uint64_t n_sa, uint64_t* out) {
+    for (uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n_sa; k += (uint64_t)gridDim.x * blockDim.x)
+        out[k] = sa_bytes == 4 ? (uint64_t)static_cast<const uint32_t*>(sa)[k * 32] : static_cast<const uint64_t*>(sa)[k * 32];
+}
+
+extern "C" {
+
+int bsq_index_alloc_replica(bsq_index* h, const bsq_index_meta* m) {
+    BSQ_ENTRY();
+    if (!h || !m || !m->built) { bsq_set_error("bad argument"); return BSQ_ERR; }
+    return alloc_replica(h, m);
+}
+
+// Host-side state that has no device copy: the ambiguity holes of the reference rows (copied un-rebased, bwa.cpp:98-104) and the
+// row each one came from.  Blob = u64 n_holes | n_holes x bsq_hole | n_holes x u32 row.
+int bsq_index_host_state_size(const bsq_index* h, uint64_t* bytes) {
+    BSQ_ENTRY();
+    if (!h || !bytes) { bsq_set_error("null argument"); return BSQ_ERR; }
+    *bytes = 8 + h->holes.size() * (sizeof(bsq_hole) + 4);
+    return BSQ_OK;
+}
+
+int bsq_index_host_state_get(const bsq_index* h, void* buf, uint64_t bytes) {
+    BSQ_ENTRY();
+    if (!h || !buf) { bsq_set_error("null argument"); return BSQ_ERR; }
+    const uint64_t nh = h->holes.size();
+    if (bytes < 8 + nh * (sizeof(bsq_hole) + 4)) { bsq_set_error("host-state buffer too small"); return BSQ_ERR; }
+    uint8_t* p = static_cast<uint8_t*>(buf);
+    memcpy(p, &nh, 8);
+    if (nh) { memcpy(p + 8, h->holes.data(), nh * sizeof(bsq_hole)); memcpy(p + 8 + nh * sizeof(bsq_hole), h->hole_ann.data(), nh * 4); }
+    return BSQ_OK;
+}
+
+int bsq_index_replica_finish(bsq_index* h, const void* host_state, uint64_t bytes) {
+    BSQ_ENTRY();
+    if (!h || !h->meta.built) { bsq_set_error("replica not allocated"); return BSQ_ERR; }
+    return replica_finish(h, host_state, bytes);
+}
+
 int bsq_index_bwt_plain(const bsq_index* h, uint32_t* out) {
     BSQ_ENTRY();
     if (!h || !h->meta.built) { bsq_set_error("index not built"); return BSQ_ERR; }
@@ -428,11 +449,6 @@ int bsq_index_bwt_plain(const bsq_index* h, uint32_t* out) {
     uint64_t nw = (h->meta.seq_len + 15) / 16;
     for (uint64_t i = 0; i < nw; ++i) out[i] = occ[(i >> 3 << 4) + 8 + (i & 7)];
     return BSQ_OK;
-}
-
-static __global__ void k_sa_sample(const void* sa, int sa_bytes, uint64_t n_sa, uint64_t* out) {
-    for (uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n_sa; k += (uint64_t)gridDim.x * blockDim.x)
-        out[k] = sa_bytes == 4 ? (uint64_t)static_cast<const uint32_t*>(sa)[k * 32] : static_cast<const uint64_t*>(sa)[k * 32];
 }
 
 int bsq_index_sa_sampled(const bsq_index* h, uint64_t* out, uint64_t n_sa) {
@@ -468,6 +484,71 @@ int bsq_index_prepare(bsq_index* h, float* ms) {
     if (ms) cudaEventElapsedTime(ms, e0, e1);
     cudaEventDestroy(e0); cudaEventDestroy(e1);
     return rc;
+}
+
+// Index files (layout and kernels: index_file.cu).  A loaded index is one more replica: allocated and finished by the same code as a
+// broadcast's, its arrays filled from the file instead of a peer.
+int bsq_index_save(bsq_index* h, const char* path, const uint8_t* key) {
+    BSQ_ENTRY();
+    if (!h || !path) { bsq_set_error("null argument"); return BSQ_ERR; }
+    if (!h->meta.built) { bsq_set_error("bsq_index_save: the index is not built (an empty reference builds nothing)"); return BSQ_ERR; }
+    if (h->replica_pending) { bsq_set_error("bsq_index_save: replica without host state"); return BSQ_ERR; }
+    CUDA_CHECK(cudaSetDevice(h->device));
+    std::vector<uint8_t> hs(8 + h->holes.size() * (sizeof(bsq_hole) + 4));
+    if (bsq_index_host_state_get(h, hs.data(), hs.size()) != BSQ_OK) return BSQ_ERR;
+    const uint64_t n_sa = (h->meta.seq_len + 32) / 32;
+    uint64_t* d_samples = nullptr;
+    CUDA_CHECK(cudaMalloc(&d_samples, n_sa * 8));
+    k_sa_sample<<<148 * 8, 256, 0, h->stream>>>(h->d_sa, (int)h->meta.sa_bytes, n_sa, d_samples);   // sample 0 = SA[0] = seq_len
+    const IndexFileArrays a{h->d_pac, h->d_occ, h->d_sa, h->d_ann_offset, h->d_ann_len, h->d_ann_id};
+    const int rc = index_file_save(path, h->meta, a, d_samples, h->pac.data(), h->ann_offset.data(), h->ann_len.data(), h->ann_id.data(), hs, key, h->stream);
+    cudaFree(d_samples);
+    return rc;
+}
+
+int bsq_index_load(bsq_index* h, const char* path, const uint8_t* key, float* ms) {
+    BSQ_ENTRY();
+    const auto t0 = std::chrono::steady_clock::now();
+    if (!h || !path) { bsq_set_error("null argument"); return BSQ_ERR; }
+    if (h->meta.built || !h->ann_offset.empty()) { bsq_set_error("bsq_index_load: the handle already has reference rows or an index (load needs a fresh handle)"); return BSQ_ERR; }
+    CUDA_CHECK(cudaSetDevice(h->device));
+    IndexFileReader r;
+    bsq_index_meta m;
+    bsq_index_load_info info;
+    memset(&info, 0, sizeof(info));
+    std::vector<uint8_t> hs;
+    int rc = index_file_open(r, path, key, &m);
+    if (rc == BSQ_OK) rc = alloc_replica(h, &m);
+    if (rc == BSQ_OK) {
+        const IndexFileArrays a{h->d_pac, h->d_occ, h->d_sa, h->d_ann_offset, h->d_ann_len, h->d_ann_id};
+        rc = index_file_fill(r, a, hs, h->device, h->stream, &info);
+    }
+    info.file_bytes = r.file_bytes;
+    index_file_close(r);
+    if (rc == BSQ_OK) {
+        const auto t1 = std::chrono::steady_clock::now();
+        rc = replica_finish(h, hs.data(), hs.size());
+        info.host_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t1).count();
+    }
+    if (rc != BSQ_OK) {   // leave the handle as fresh as it came
+        cudaStreamSynchronize(h->stream);
+        free_index_arrays(h);
+        memset(&h->meta, 0, sizeof(h->meta));
+        h->replica_pending = false;
+        h->pac.clear(); h->ann_offset.clear(); h->ann_len.clear(); h->ann_id.clear(); h->holes.clear(); h->hole_ann.clear();
+        return BSQ_ERR;
+    }
+    info.total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    h->last_load = info;
+    if (ms) *ms = info.total_ms;
+    return BSQ_OK;
+}
+
+int bsq_index_last_load(const bsq_index* h, bsq_index_load_info* out) {
+    BSQ_ENTRY();
+    if (!h || !out) { bsq_set_error("null argument"); return BSQ_ERR; }
+    *out = h->last_load;
+    return BSQ_OK;
 }
 
 }  // extern "C"

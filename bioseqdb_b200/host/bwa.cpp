@@ -3,6 +3,7 @@
 #include <algorithm>
 #include <cstring>
 #include <stdexcept>
+#include <unistd.h>
 
 namespace bioseqdb {
 
@@ -38,6 +39,28 @@ void BwaIndex::build() {
     if (bsq_index_build(index) != BSQ_OK) fail();
 }
 
+void BwaIndex::save(const std::string& path, const uint8_t* key) const {
+    if (bsq_index_save(index, path.c_str(), key) != BSQ_OK) fail();
+}
+
+void BwaIndex::load(const std::string& path, const uint8_t* key) {
+    if (bsq_index_load(index, path.c_str(), key, nullptr) != BSQ_OK) fail();
+    bsq_index_meta m;
+    if (bsq_index_get_meta(index, &m) != BSQ_OK) fail();
+    pac_forward.resize(m.arr_bytes[BSQ_ARR_PAC]);
+    offsets.resize(m.n_anns);
+    if (bsq_index_download(index, BSQ_ARR_PAC, pac_forward.data(), pac_forward.size()) != BSQ_OK) fail();
+    if (bsq_index_download(index, BSQ_ARR_ANN_OFFSET, offsets.data(), offsets.size() * 8) != BSQ_OK) fail();
+    uint64_t nb = 0;
+    if (bsq_index_host_state_size(index, &nb) != BSQ_OK) fail();
+    std::vector<uint8_t> st(nb);
+    if (bsq_index_host_state_get(index, st.data(), nb) != BSQ_OK) fail();
+    uint64_t nh = 0;
+    memcpy(&nh, st.data(), 8);
+    holes.resize(nh);
+    if (nh) memcpy(holes.data(), st.data() + 8, nh * sizeof(bsq_hole));
+}
+
 uint64_t BwaIndex::device_bytes() const {
     uint64_t b = 0;
     if (bsq_index_device_bytes(index, &b) != BSQ_OK) fail();
@@ -69,7 +92,14 @@ std::pair<uint64_t, uint64_t> BwaIndexCache::digest(const Rows& rows) {
     return {a, b};
 }
 
-BwaIndexCache::BwaIndexCache(int device_, uint64_t max_bytes_) : device(device_), max_bytes(max_bytes_) {}
+BwaIndexCache::BwaIndexCache(int device_, uint64_t max_bytes_, std::string directory_)
+    : device(device_), max_bytes(max_bytes_), directory(std::move(directory_)) {}
+
+std::string BwaIndexCache::file_path(const std::pair<uint64_t, uint64_t>& key) const {
+    char hex[33];
+    snprintf(hex, sizeof(hex), "%016llx%016llx", (unsigned long long)key.first, (unsigned long long)key.second);
+    return directory + "/" + hex + ".bsqidx";
+}
 
 BwaIndex& BwaIndexCache::get(const Rows& rows, const bsq_opts& opts) {
     const auto key = digest(rows);
@@ -83,10 +113,30 @@ BwaIndex& BwaIndexCache::get(const Rows& rows, const bsq_opts& opts) {
             return ix;
         }
     ++misses;
-    std::unique_ptr<BwaIndex> ix(new BwaIndex(device));
-    for (const auto& r : rows) ix->add_ref_sequence(r.first, *r.second);
-    ix->options = opts;
-    ix->build();
+    uint8_t fkey[16];
+    memcpy(fkey, &key.first, 8); memcpy(fkey + 8, &key.second, 8);
+    bool empty = true;                     // an empty reference builds nothing (bwa.cpp:108-109): nothing to keep on disk
+    for (const auto& r : rows) empty = empty && r.second->len == 0;
+    const std::string path = directory.empty() || empty ? std::string() : file_path(key);
+    std::unique_ptr<BwaIndex> ix;
+    if (!path.empty() && access(path.c_str(), F_OK) == 0) {
+        ix.reset(new BwaIndex(device));
+        try { ix->load(path, fkey); ++disk_hits; }
+        catch (const std::runtime_error&) { ++disk_errors; ix.reset(); }   // damaged or foreign: rebuilt and replaced below
+    }
+    if (ix) {
+        ix->options = opts;
+        if (bsq_index_set_opts(ix->index, &ix->options) != BSQ_OK) fail();
+    } else {
+        ix.reset(new BwaIndex(device));
+        for (const auto& r : rows) ix->add_ref_sequence(r.first, *r.second);
+        ix->options = opts;
+        ix->build();
+        if (!path.empty()) {
+            try { ix->save(path, fkey); ++disk_saves; }
+            catch (const std::runtime_error&) { ++disk_errors; }          // this call is served; the next process builds
+        }
+    }
     lru.push_front(Entry{key, std::move(ix)});
     uint64_t total = 0;
     for (const Entry& e : lru) total += e.index->device_bytes();

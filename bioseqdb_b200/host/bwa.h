@@ -72,6 +72,10 @@ public:
     BwaTupleBatch align_sequences_tuples(const std::vector<const NucleotideSequence*>& seqs, uint32_t flags = 0);
     void build();
     void add_ref_sequence(int64_t id, const NucleotideSequence& seq);
+    // Index files (bsq_index_save / bsq_index_load): build once, load in any process.  key: 16 bytes kept in the file's header, or
+    // nullptr.  load() fills a fresh index and refills the host copies extract_reference_subseq reads (pac, row offsets, holes).
+    void save(const std::string& path, const uint8_t* key = nullptr) const;
+    void load(const std::string& path, const uint8_t* key = nullptr);
 
     bsq_opts options;            // written by bwa_index_from_query before build()
     size_t ref_count() const { return offsets.size(); }
@@ -93,19 +97,24 @@ private:
 // resident in HBM, finds them again by a 128-bit digest of (id, length, payload, holes) of every row in cursor order,
 // applies the call's options to the cached handle, and evicts least-recently-used indexes beyond `max_bytes`.  It also
 // owns the session's lrand48 state (process-wide in the reference), lending it to the index that serves a call.
+// With a `directory` a memory miss first looks for `<directory>/<digest hex>.bsqidx` (another backend may have built it) and
+// loads it; otherwise it builds and writes the file.  A file that does not load is rebuilt and replaced; a failed write only
+// counts in disk_errors.  Empty references are never written.
 class BwaIndexCache {
 public:
     using Rows = std::vector<std::pair<int64_t, const NucleotideSequence*>>;
-    explicit BwaIndexCache(int device = 0, uint64_t max_bytes = 96ull << 30);
+    explicit BwaIndexCache(int device = 0, uint64_t max_bytes = 96ull << 30, std::string directory = "");
     BwaIndex& get(const Rows& rows, const bsq_opts& opts);     // built, options applied; owned by the cache
     // align through a cached index with the session's id stream
     std::vector<std::vector<BwaMatch>> align_sequences(BwaIndex& ix, const std::vector<const NucleotideSequence*>& seqs);
     uint64_t hits = 0, misses = 0, evictions = 0;
+    uint64_t disk_hits = 0, disk_saves = 0, disk_errors = 0;
     static std::pair<uint64_t, uint64_t> digest(const Rows& rows);
+    std::string file_path(const std::pair<uint64_t, uint64_t>& key) const;
 private:
     struct Entry { std::pair<uint64_t, uint64_t> key; std::unique_ptr<BwaIndex> index; };
     std::list<Entry> lru;                  // front = most recently used
-    int device; uint64_t max_bytes; uint64_t lrand_state = 0;
+    int device; uint64_t max_bytes; std::string directory; uint64_t lrand_state = 0;
 };
 
 std::string cigar_compressed_to_string(const uint32_t* raw, int len);   // htslib letters on bwa op codes (bwa.cpp:70-77)

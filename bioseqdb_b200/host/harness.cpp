@@ -7,11 +7,14 @@
 // GPU-built column -- the two NUCLSEQ datums, the CIGAR string, ref_match_* -- is compared with what build_tuple_bwa
 // (extension.cpp:282-305) would form from the BwaMatch; with check_bulk=1 the reference rows' texts go through the bulk
 // text -> NUCLSEQ conversion and are compared with nuclseq_from_text.  A difference is an error (exit code 1).
+// With index_cache=DIR the index comes from a BwaIndexCache with that directory, as a backend's would: the first process builds
+// it and writes DIR/<digest>.bsqidx, every later one loads that file.  The counters go to stderr ("index_cache: ...").
 #include <cstdio>
 #include <cstring>
 #include <fstream>
 #include <iostream>
 #include <map>
+#include <memory>
 #include <stdexcept>
 #include "bwa.h"
 
@@ -38,7 +41,9 @@ int main(int argc, char** argv) {
     if (argc < 3) { fprintf(stderr, "usage: %s reference.tsv queries.tsv [bwa_options name=value ...]\n", argv[0]); return 2; }
     try {
         std::map<std::string, int32_t> opts;
+        std::string index_cache;               // a string option: taken out before the int options are parsed
         for (int i = 3; i < argc; ++i) {
+            if (strncmp(argv[i], "index_cache=", 12) == 0) { index_cache = argv[i] + 12; continue; }
             const char* eq = strchr(argv[i], '=');
             if (!eq) throw std::runtime_error("options are name=value");
             opts[std::string(argv[i], (size_t)(eq - argv[i]))] = (int32_t)atoi(eq + 1);
@@ -51,23 +56,42 @@ int main(int argc, char** argv) {
         };
         const bool check_tuples = opts.count("check_tuples") && opts["check_tuples"]; opts.erase("check_tuples");
         const bool check_bulk = opts.count("check_bulk") && opts["check_bulk"]; opts.erase("check_bulk");
-        BwaIndex bwa;
-        std::vector<NucleotideSequence> ref_rows;
-        size_t count = iterate_nuclseq_table(argv[1], [&](int64_t id, const NucleotideSequence& s) { bwa.add_ref_sequence(id, s); if (check_bulk) ref_rows.push_back(s); });
-        bwa.options.max_occ = get_opt_or("max_occ", (int32_t)std::max<size_t>(500, count * 2));
-        bwa.options.min_seed_len = get_opt_or("min_seed_len", 19);
-        bwa.options.a = get_opt_or("match_score", 1);
-        bwa.options.b = get_opt_or("mismatch_penalty", 4);
-        bwa.options.pen_clip3 = get_opt_or("pen_clip3", 5);
-        bwa.options.pen_clip5 = get_opt_or("pen_clip5", 5);
-        bwa.options.zdrop = get_opt_or("zdrop", 100);
-        bwa.options.w = get_opt_or("bandwidth", 100);
+        std::unique_ptr<BwaIndex> own;
+        std::unique_ptr<BwaIndexCache> cache;
+        if (index_cache.empty()) own.reset(new BwaIndex());
+        else cache.reset(new BwaIndexCache(0, 96ull << 30, index_cache));
+        std::vector<NucleotideSequence> ref_rows; std::vector<int64_t> ref_ids;
+        size_t count = iterate_nuclseq_table(argv[1], [&](int64_t id, const NucleotideSequence& s) {
+            if (own) own->add_ref_sequence(id, s);
+            if (check_bulk || cache) { ref_rows.push_back(s); ref_ids.push_back(id); }
+        });
+        bsq_opts o;
+        bsq_opts_init(&o);
+        o.max_occ = get_opt_or("max_occ", (int32_t)std::max<size_t>(500, count * 2));
+        o.min_seed_len = get_opt_or("min_seed_len", 19);
+        o.a = get_opt_or("match_score", 1);
+        o.b = get_opt_or("mismatch_penalty", 4);
+        o.pen_clip3 = get_opt_or("pen_clip3", 5);
+        o.pen_clip5 = get_opt_or("pen_clip5", 5);
+        o.zdrop = get_opt_or("zdrop", 100);
+        o.w = get_opt_or("bandwidth", 100);
         // defaults as delivered by the SQL function bwa_opts() (positional mix-up, SURVEY.md B#1)
-        bwa.options.o_del = get_opt_or("o_del", 6);
-        bwa.options.o_ins = get_opt_or("o_ins", 1);
-        bwa.options.e_del = get_opt_or("e_del", 6);
-        bwa.options.e_ins = get_opt_or("e_ins", 1);
-        bwa.build();
+        o.o_del = get_opt_or("o_del", 6);
+        o.o_ins = get_opt_or("o_ins", 1);
+        o.e_del = get_opt_or("e_del", 6);
+        o.e_ins = get_opt_or("e_ins", 1);
+        BwaIndex* ix = own.get();
+        if (own) {
+            own->options = o;
+            own->build();
+        } else {
+            BwaIndexCache::Rows rows;
+            for (size_t i = 0; i < ref_rows.size(); ++i) rows.emplace_back(ref_ids[i], &ref_rows[i]);
+            ix = &cache->get(rows, o);
+            fprintf(stderr, "index_cache: disk_hits=%llu disk_saves=%llu disk_errors=%llu\n", (unsigned long long)cache->disk_hits,
+                    (unsigned long long)cache->disk_saves, (unsigned long long)cache->disk_errors);
+        }
+        BwaIndex& bwa = *ix;
         std::vector<int64_t> qids; std::vector<NucleotideSequence> queries;
         iterate_nuclseq_table(argv[2], [&](int64_t id, NucleotideSequence s) { qids.push_back(id); queries.push_back(std::move(s)); });
         std::vector<const NucleotideSequence*> ptrs;

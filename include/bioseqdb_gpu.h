@@ -13,6 +13,7 @@
  *   bsq_align_batch      the loop over BwaIndex::align_sequence (mem_align1 + mem_reg2aln per region)
  *                                                              bioseqdb/bwa.cpp:141-181, extension.cpp:362-370
  *   bsq_result_free / bsq_index_free   BwaIndex::~BwaIndex     bioseqdb/bwa.cpp:131-139
+ *   bsq_index_save / bsq_index_load    (no reference counterpart: bwa index writes files, bwa mem loads them; the adapter rebuilds)
  * There is no CPU fallback: without a CUDA device every compute entry point fails.
  */
 #ifndef BIOSEQDB_GPU_H
@@ -185,6 +186,29 @@ int bsq_index_host_state_size(const bsq_index* h, uint64_t* bytes);
 int bsq_index_host_state_get(const bsq_index* h, void* buf, uint64_t bytes);
 int bsq_index_replica_finish(bsq_index* h, const void* host_state, uint64_t bytes);
 int bsq_index_prepare(bsq_index* h, float* ms);   /* build the per-device derived arrays (inverse SA, prefix table) now; *ms = time spent */
+/* Index files: build once, load in every process that aligns against the same reference (bwa index / bwa mem).  One file holds pac, Occ,
+ * the annotations, the host state and 1/32 of the suffix array; the load rebuilds the full suffix array on the device by LF walks from
+ * the samples.  The per-device derived arrays are not stored (bsq_index_prepare builds them).  Layout: bioseqdb_b200/csrc/index_file.cuh.
+ * Writes the built index to `path` (written to a temporary name in the same directory, fsync'd, then renamed, so a reader never sees a
+ * partial file).  key: 16 opaque bytes stored in the header (the index cache passes its digest), or NULL. */
+int bsq_index_save(bsq_index* h, const char* path, const uint8_t* key);
+/* Fills a FRESH handle (bsq_index_new, nothing added, not built) from a file written by bsq_index_save: header and sizes checked on the
+ * host, sections uploaded and checksummed on the device, full SA rebuilt from its samples, host mirrors restored.  key != NULL: the
+ * file's key must match.  *ms = wall time of the call.  Options and flags are the handle's, as for any index.  On failure the handle is
+ * left fresh. */
+int bsq_index_load(bsq_index* h, const char* path, const uint8_t* key, float* ms);
+/* Where the last successful bsq_index_load of the handle spent its time (file in the page cache or not: whatever the OS gave it). */
+typedef struct bsq_index_load_info {
+    uint64_t file_bytes;
+    float read_ms;       /* wall: file read + upload of every section through the pinned staging buffers */
+    float checksum_ms;   /* device: k_section_checksum over the uploaded sections */
+    float sa_ms;         /* device: k_sa_from_samples */
+    float host_ms;       /* wall: host mirrors (pac, annotations, holes) restored */
+    float total_ms;      /* wall: the whole call */
+    uint64_t lf_steps;   /* LF steps of the suffix-array rebuild (seq_len + 1 for a sound file) */
+    uint64_t lane_slots; /* warp iterations x 32 of the rebuild: lf_steps / lane_slots = its lane efficiency */
+} bsq_index_load_info;
+int bsq_index_last_load(const bsq_index* h, bsq_index_load_info* out);
 /* One process, one host thread, several GPUs (SURVEY.md 8b / 8e; reference extension.cpp:346-377 is one backend, one thread): the
  * index of `built` is copied to devices[1..] (peer copies over NVLink + the host-side state), every device derives its own inverse SA /
  * prefix table, and a batch is cut into contiguous blocks of reads, one per device (read i keeps lrand48 id i).  The rows of all
