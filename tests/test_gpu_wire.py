@@ -120,6 +120,32 @@ def test_tuples_from_resident_batch(gpu_lib):
             assert np.array_equal(tup2.off, ref2.off) and np.array_equal(tup2.data, ref2.data) and np.array_equal(tup2.ref_match, ref2.ref_match)
 
 
+def test_tuples_of_another_result_leave_the_resident_batch(gpu_lib):
+    """bsq_result_tuples on a result that is not resident works in buffers of its own: a tuples call on another, host-assembled result
+    between the alignment of a batch and the tuples of that batch's result must leave the batch servable (no reads passed) and its
+    tuples unchanged."""
+    import ctypes as C
+    from bioseqdb_b200._lib import BsqResult, check, ptr
+    rows = synth.reference_rows([250_001, 150_003], seed=161)
+    _, gpu = build_pair(rows, O.sql_default_opts(2))
+    s_other, o_other, _ = synth.simulate_reads(rows, 6000, 150, seed=162)
+    other = gpu.align_batch(s_other, o_other, synth.lrand48_ids_fast(6000))     # copied to the host: no longer the library's own result
+    seqs, offs, _ = synth.simulate_reads(rows, 4000, 100, seed=163, n_frac=0.003)
+    ids = synth.lrand48_ids_fast(4000)
+    res = C.POINTER(BsqResult)()
+    check(gpu.L.bsq_align_batch(gpu.h, ptr(seqs), ptr(offs), ptr(ids), 4000, C.byref(res)))
+    try:
+        before = gpu._fetch_tuples(res, None, None, 0)
+        staged = gpu.tuples(other, s_other, o_other)
+        after = gpu._fetch_tuples(res, None, None, 0)
+    finally:
+        gpu.L.bsq_result_free(res)
+    assert len(other.rows) > 5000 and len(staged.off) == 3 * len(other.rows) + 1
+    assert len(before.off) > 3 * 3600
+    assert np.array_equal(before.off, after.off) and np.array_equal(before.ref_match, after.ref_match)
+    assert np.array_equal(before.data, after.data)
+
+
 def test_pool_oom_drops_a_table_level(gpu_lib, monkeypatch):
     """Device memory short while sizing the batch pools (simulated: BSQ_TEST_POOL_OOM makes one pool allocation fail): the library gives back
     the deepest level of the seeding prefix table, rebuilds the shallower one and finishes the call; the rows do not change (the table
