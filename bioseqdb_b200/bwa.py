@@ -372,19 +372,9 @@ class BwaIndex:
     def tuples(self, res: AlignResult, seqs: np.ndarray, offs: np.ndarray, flags: int = 0) -> "Tuples":
         """Row materialisation on the GPU (SURVEY.md 8f-2): for every row of `res` the NUCLSEQ datum images of ref_subseq and
         query_subseq, the CIGAR string and ref_match_* -- what build_tuple_bwa (extension.cpp:282-305) assembles from a BwaMatch."""
+        r, keep = _host_result(res)
         seqs = np.ascontiguousarray(seqs, dtype=np.uint8)
         offs = np.ascontiguousarray(offs, dtype=np.uint64)
-        row_off = np.ascontiguousarray(res.row_off, dtype=np.uint64)
-        rows = np.zeros(len(res.rows), dtype=PUB_ROW_DTYPE)
-        for f in PUB_ROW_DTYPE.names:
-            rows[f] = res.rows[f]
-        cigar = np.ascontiguousarray(res.cigar, dtype=np.uint32)
-        r = BsqResult()
-        r.n_reads = len(row_off) - 1
-        r.row_off = row_off.ctypes.data_as(C.POINTER(C.c_uint64))
-        r.rows = rows.ctypes.data
-        r.cigar = cigar.ctypes.data_as(C.POINTER(C.c_uint32))
-        r.n_cigar_words = len(cigar)
         return self._fetch_tuples(C.byref(r), ptr(seqs), ptr(offs), flags)
 
     def _fetch_tuples(self, res, seqs, offs, flags: int) -> "Tuples":
@@ -393,15 +383,7 @@ class BwaIndex:
         from ._lib import BsqTuples
         tp = C.POINTER(BsqTuples)()
         check(self.L.bsq_result_tuples(self.h, res, seqs, offs, int(flags), C.byref(tp)))
-        t = tp.contents
-        n = int(t.n_rows)
-        off = np.ctypeslib.as_array(t.off, shape=(3 * n + 1,)).copy()
-        ref_match = np.ctypeslib.as_array(t.ref_match, shape=(max(3 * n, 1),))[:3 * n].copy().reshape(n, 3)
-        nb = int(t.n_bytes)
-        data = np.ctypeslib.as_array(t.bytes, shape=(max(nb, 1),))[:nb].copy()
-        ms = float(t.device_ms)
-        self.L.bsq_tuples_free(tp)
-        return Tuples(off, ref_match, data, ms)
+        return _take_tuples(self.L, tp)
 
     def timing(self) -> BsqTiming:
         t = BsqTiming()
@@ -540,6 +522,83 @@ class MultiBwaIndex:
         t = BsqTiming()
         check(self.L.bsq_multi_last_timing(self.m, C.byref(t)))
         return t
+
+    def tuples(self, res: AlignResult, seqs: np.ndarray, offs: np.ndarray, flags: int = 0) -> Tuples:
+        """BwaIndex.tuples on every device (bsq_multi_result_tuples): each device materialises the rows of its block of reads.  A host
+        result is staged: every device uploads its block's rows, CIGAR words and reads."""
+        r, keep = _host_result(res)
+        seqs = np.ascontiguousarray(seqs, dtype=np.uint8)
+        offs = np.ascontiguousarray(offs, dtype=np.uint64)
+        return self._fetch_tuples(C.byref(r), ptr(seqs), ptr(offs), flags)
+
+    def _fetch_tuples(self, res, seqs, offs, flags: int) -> Tuples:
+        from ._lib import BsqTuples
+        tp = C.POINTER(BsqTuples)()
+        check(self.L.bsq_multi_result_tuples(self.m, res, seqs, offs, int(flags), C.byref(tp)))
+        return _take_tuples(self.L, tp)
+
+    def align_tuples_datums(self, data, off, ids=None, flags: int = 0):
+        """bsq_multi_align_batch_datums, then the tuples of its result, which every device serves from its resident block (no
+        re-upload, no reads passed).  Returns (AlignResult, Tuples)."""
+        data = np.ascontiguousarray(data, dtype=np.uint8)
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        if ids is not None:
+            ids = np.ascontiguousarray(ids, dtype=np.int64)
+        res = C.POINTER(BsqResult)()
+        check(self.L.bsq_multi_align_batch_datums(self.m, ptr(data), ptr(off), ptr(ids) if ids is not None else None, len(off) - 1, C.byref(res)))
+        try:
+            tup = self._fetch_tuples(res, None, None, flags)
+        except Exception:
+            self.L.bsq_result_free(res)
+            raise
+        return self.ix._collect(res), tup
+
+    def align_tuples_raw(self, data_ptr: int, off_ptr: int, ids_ptr: int | None, n: int, flags: int = 0):
+        """bench helper, as BwaIndex.align_tuples_raw: one bsq_multi_align_batch_datums call on raw (pinned) host pointers, then
+        bsq_multi_result_tuples on its result.  Returns (device ms of both calls, bytes that came back, tuple bytes)."""
+        from ._lib import BsqTuples
+        res = C.POINTER(BsqResult)()
+        check(self.L.bsq_multi_align_batch_datums(self.m, C.c_void_p(data_ptr), C.c_void_p(off_ptr), C.c_void_p(ids_ptr) if ids_ptr else None, n, C.byref(res)))
+        t = self.timing()
+        tp = C.POINTER(BsqTuples)()
+        try:
+            check(self.L.bsq_multi_result_tuples(self.m, res, None, None, int(flags), C.byref(tp)))
+            ms = float(t.total) + float(tp.contents.device_ms)
+            tb = int(tp.contents.n_bytes)
+            nbytes = int(t.d2h_bytes) + tb + int(tp.contents.n_rows) * 36 + 8
+            self.L.bsq_tuples_free(tp)
+        finally:
+            self.L.bsq_result_free(res)
+        return ms, nbytes, tb
+
+
+def _host_result(res: AlignResult):
+    """A bsq_result over the arrays of a host AlignResult; the second value keeps those arrays alive."""
+    row_off = np.ascontiguousarray(res.row_off, dtype=np.uint64)
+    rows = np.zeros(len(res.rows), dtype=PUB_ROW_DTYPE)
+    for f in PUB_ROW_DTYPE.names:
+        rows[f] = res.rows[f]
+    cigar = np.ascontiguousarray(res.cigar, dtype=np.uint32)
+    r = BsqResult()
+    r.n_reads = len(row_off) - 1
+    r.row_off = row_off.ctypes.data_as(C.POINTER(C.c_uint64))
+    r.rows = rows.ctypes.data
+    r.cigar = cigar.ctypes.data_as(C.POINTER(C.c_uint32))
+    r.n_cigar_words = len(cigar)
+    return r, (row_off, rows, cigar)
+
+
+def _take_tuples(L, tp) -> Tuples:
+    """Copies a bsq_tuples out of the library's pinned block and frees it."""
+    t = tp.contents
+    n = int(t.n_rows)
+    off = np.ctypeslib.as_array(t.off, shape=(3 * n + 1,)).copy()
+    ref_match = np.ctypeslib.as_array(t.ref_match, shape=(max(3 * n, 1),))[:3 * n].copy().reshape(n, 3)
+    nb = int(t.n_bytes)
+    data = np.ctypeslib.as_array(t.bytes, shape=(max(nb, 1),))[:nb].copy()
+    ms = float(t.device_ms)
+    L.bsq_tuples_free(tp)
+    return Tuples(off, ref_match, data, ms)
 
 
 def _key_arg(key):

@@ -150,6 +150,7 @@ struct bsq_index {
     bool replica_pending = false;    // device arrays allocated by bsq_index_alloc_replica, host mirrors not yet rebuilt (bsq_index_replica_finish)
     bsq_index_load_info last_load{};  // the last successful bsq_index_load
     uint64_t counters[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    uint64_t* tup_host = nullptr;    // pinned, 4 words: byte total [0] and CIGAR span [1..2] of a staged row materialisation piece
 };
 
 static void fill_dev_opts(bsq_index* h) {
@@ -324,6 +325,7 @@ void bsq_index_free(bsq_index* h) {
     if (h->d_logtab) cudaFree(h->d_logtab);
     if (h->stream) cudaStreamDestroy(h->stream);
     if (h->stream2) cudaStreamDestroy(h->stream2);
+    if (h->tup_host) cudaFreeHost(h->tup_host);
     delete h;
 }
 
@@ -1455,30 +1457,89 @@ static void index_holes_sorted(const bsq_index* h, uint32_t flags, std::vector<T
 // the tuples handed out: one pinned block from the library's cache, off | ref_match | bytes
 struct TuplesImpl { bsq_tuples pub; void* host = nullptr; size_t host_bytes = 0; ~TuplesImpl() { if (host) pinned_put(host, host_bytes); } };
 
-// A piece of a result to materialise: device views of the TupleParams inputs, the stream it runs on, its scratch and the host word
-// its byte total comes back to
+struct StagedResult;
+
+// A piece of a result to materialise on the handle h (its device, pac, annotations and launch counter): device views of the TupleParams
+// inputs, the stream it runs on, its scratch, the host word its byte total comes back to and, for a piece that is not resident, the
+// uploads that fill those views
 struct TuplePiece {
+    bsq_index* h;
     const RowPub* rows; uint64_t n_rows; const uint32_t* cigar; const uint8_t* seqs; const uint64_t* offs;
     const uint64_t* row_off; uint64_t n_reads, row_base;    // row offsets of the piece's reads, counted from row_base
     cudaStream_t st; TupleScratch* s; uint64_t* n_bytes;
+    StagedResult* stage;
 };
 
-// A result that is not resident (assembled by the caller, three or more chunks, a bsq_multi result): rows, CIGAR words, row offsets,
-// reads and read offsets go to call-local buffers as they are
+// Reads [r0, r0 + n) of a result that is not resident (assembled by the caller, three or more chunks, another call's result, a device
+// that has aligned something else since): their rows, row offsets, reads and read offsets go to call-local buffers as they are.  The
+// whole result takes every CIGAR word; a part of it takes the span of words its rows use, which the device finds first (k_cigar_span).
 struct StagedResult {
     const bsq_result* res = nullptr; const char* seqs = nullptr; const uint64_t* offs = nullptr;
-    DevBuf<RowPub> rows; DevBuf<uint32_t> cigar; DevBuf<uint8_t> text; DevBuf<uint64_t> row_off, read_off;
-    TupleScratch s; uint64_t n_bytes = 0;
+    uint64_t r0 = 0, n = 0, row0 = 0; bool whole = true;
+    DevBuf<RowPub> rows; DevBuf<uint32_t> cigar; DevBuf<uint8_t> text; DevBuf<uint64_t> row_off, read_off; DevBuf<unsigned long long> span;
+    TupleScratch s;
 };
 
-static int stage_upload(const StagedResult& S, cudaStream_t st, uint64_t* launches) {
-    const bsq_result* r = S.res; const uint64_t n = r->n_reads, total = S.offs[n] - S.offs[0];
-    CUDA_CHECK_AS("bsq_result_tuples", cudaMemcpyAsync(S.rows.p, r->rows, r->row_off[n] * sizeof(RowPub), cudaMemcpyHostToDevice, st));
-    CUDA_CHECK_AS("bsq_result_tuples", cudaMemcpyAsync(S.row_off.p, r->row_off, n * 8, cudaMemcpyHostToDevice, st));
-    if (r->n_cigar_words) CUDA_CHECK_AS("bsq_result_tuples", cudaMemcpyAsync(S.cigar.p, r->cigar, r->n_cigar_words * 4, cudaMemcpyHostToDevice, st));
-    if (total) CUDA_CHECK_AS("bsq_result_tuples", cudaMemcpyAsync(S.text.p, S.seqs + S.offs[0], total, cudaMemcpyHostToDevice, st));
-    CUDA_CHECK_AS("bsq_result_tuples", cudaMemcpyAsync(S.read_off.p, S.offs, (n + 1) * 8, cudaMemcpyHostToDevice, st));
-    if (S.offs[0]) { k_rebase_offs<<<(unsigned)std::min<uint64_t>((n + 256) / 256, 148 * 8), 256, 0, st>>>(S.read_off.p, n + 1, S.offs[0]); ++*launches; }
+// [first, end) of the CIGAR words that rows with a CIGAR use; span[0] starts at ~0 and span[1] at 0
+static __global__ void k_cigar_span(const RowPub* rows, uint64_t n_rows, unsigned long long* span) {
+    unsigned long long lo = ~0ull, hi = 0;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_rows; i += (uint64_t)gridDim.x * blockDim.x)
+        if (rows[i].n_cigar) { lo = min(lo, (unsigned long long)rows[i].cigar_off); hi = max(hi, (unsigned long long)rows[i].cigar_off + rows[i].n_cigar); }
+    for (int o = 16; o; o >>= 1) { lo = min(lo, __shfl_xor_sync(~0u, lo, o)); hi = max(hi, __shfl_xor_sync(~0u, hi, o)); }
+    if ((threadIdx.x & 31) == 0) { atomicMin(span, lo); atomicMax(span + 1, hi); }
+}
+
+// The piece of reads [r0, r0 + n) of `res` on handle h, with its call-local buffers in S.  A block without rows uploads nothing.
+static int stage_block(bsq_index* h, StagedResult& S, const bsq_result* res, const char* seqs, const uint64_t* offs, uint64_t r0, uint64_t n,
+                       const char* what, TuplePiece& pc) {
+    const uint64_t row0 = r0 ? res->row_off[r0] : 0;
+    if (n && res->row_off[r0 + n] < row0) { bsq_set_error("%s: row offsets must be non-decreasing", what); return BSQ_ERR; }
+    const uint64_t n_rows = n ? res->row_off[r0 + n] - row0 : 0;
+    pc = TuplePiece{h, nullptr, n_rows, nullptr, nullptr, nullptr, nullptr, n, row0, h->stream, &S.s, nullptr, nullptr};
+    if (!n_rows) return BSQ_OK;
+    CUDA_CHECK_AS(what, cudaSetDevice(h->device));
+    if (!h->tup_host && cudaHostAlloc(&h->tup_host, 4 * 8, cudaHostAllocDefault) != cudaSuccess) {
+        cudaGetLastError(); h->tup_host = nullptr; bsq_set_error("cannot allocate pinned host memory for the tuples"); return BSQ_ERR;
+    }
+    S.res = res; S.seqs = seqs; S.offs = offs; S.r0 = r0; S.n = n; S.row0 = row0; S.whole = r0 == 0 && n == res->n_reads;
+    CUDA_CHECK_AS(what, S.rows.alloc(n_rows));
+    if (S.whole) CUDA_CHECK_AS(what, S.cigar.alloc(res->n_cigar_words + 1)); else CUDA_CHECK_AS(what, S.span.alloc(2));
+    CUDA_CHECK_AS(what, S.text.alloc(offs[r0 + n] - offs[r0] + 64));
+    CUDA_CHECK_AS(what, S.row_off.alloc(n)); CUDA_CHECK_AS(what, S.read_off.alloc(n + 1));
+    pc.rows = S.rows.p; pc.cigar = S.cigar.p; pc.seqs = S.text.p; pc.offs = S.read_off.p; pc.row_off = S.row_off.p;
+    pc.n_bytes = h->tup_host; pc.stage = &S;
+    return BSQ_OK;
+}
+
+// first half of a staged piece's uploads: its rows and, for a part of a result, the span of CIGAR words they use
+static int stage_rows(const TuplePiece& pc, const char* what) {
+    const StagedResult& S = *pc.stage;
+    CUDA_CHECK_AS(what, cudaMemcpyAsync(S.rows.p, S.res->rows + S.row0, pc.n_rows * sizeof(RowPub), cudaMemcpyHostToDevice, pc.st));
+    if (!S.whole) {
+        CUDA_CHECK_AS(what, cudaMemsetAsync(S.span.p, 0xff, 8, pc.st)); CUDA_CHECK_AS(what, cudaMemsetAsync(S.span.p + 1, 0, 8, pc.st));
+        k_cigar_span<<<(unsigned)std::min<uint64_t>((pc.n_rows + 255) / 256, 148 * 8), 256, 0, pc.st>>>(S.rows.p, pc.n_rows, S.span.p); ++pc.h->timing.launches;
+        CUDA_CHECK_AS(what, cudaMemcpyAsync(pc.n_bytes + 1, S.span.p, 16, cudaMemcpyDeviceToHost, pc.st));
+    }
+    return BSQ_OK;
+}
+
+// second half, once a part's span has landed: CIGAR words, row offsets, reads and read offsets (rebased to the piece's first read)
+static int stage_rest(TuplePiece& pc, const char* what) {
+    StagedResult& S = *pc.stage;
+    const bsq_result* r = S.res; const uint64_t n = S.n, *offs = S.offs + S.r0, total = offs[n] - offs[0];
+    uint64_t lo = 0, hi = r->n_cigar_words;
+    if (!S.whole) {
+        lo = pc.n_bytes[1]; hi = pc.n_bytes[2];
+        if (hi <= lo) lo = hi = 0;   // no row of the piece has a CIGAR
+        else if (hi > r->n_cigar_words) { bsq_set_error("%s: a row's CIGAR words lie beyond the result's %llu words", what, (unsigned long long)r->n_cigar_words); return BSQ_ERR; }
+        CUDA_CHECK_AS(what, S.cigar.alloc(hi - lo + 1));
+        pc.cigar = S.cigar.p - lo;
+    }
+    if (hi > lo) CUDA_CHECK_AS(what, cudaMemcpyAsync(S.cigar.p, r->cigar + lo, (hi - lo) * 4, cudaMemcpyHostToDevice, pc.st));
+    CUDA_CHECK_AS(what, cudaMemcpyAsync(S.row_off.p, r->row_off + S.r0, n * 8, cudaMemcpyHostToDevice, pc.st));
+    if (total) CUDA_CHECK_AS(what, cudaMemcpyAsync(S.text.p, S.seqs + offs[0], total, cudaMemcpyHostToDevice, pc.st));
+    CUDA_CHECK_AS(what, cudaMemcpyAsync(S.read_off.p, offs, (n + 1) * 8, cudaMemcpyHostToDevice, pc.st));
+    if (offs[0]) { k_rebase_offs<<<(unsigned)std::min<uint64_t>((n + 256) / 256, 148 * 8), 256, 0, pc.st>>>(S.read_off.p, n + 1, offs[0]); ++pc.h->timing.launches; }
     return BSQ_OK;
 }
 
@@ -1494,53 +1555,89 @@ static int resident_pieces(bsq_index* h, const ResultImpl* R, TuplePiece* pc) {
         Batch& b = *piece[k];
         if (b.res_read_base != covered) return 0;
         covered += b.n;
-        pc[k] = TuplePiece{b.rows_compact.p, b.out_rows, b.cigar.p - b.cig_rebased, b.ascii.p, b.offs.p, b.row_off64.p, b.n, b.res_row_base,
-                           b.st, &b.tup, reinterpret_cast<uint64_t*>(b.ctl_host + 14)};
+        pc[k] = TuplePiece{h, b.rows_compact.p, b.out_rows, b.cigar.p - b.cig_rebased, b.ascii.p, b.offs.p, b.row_off64.p, b.n, b.res_row_base,
+                           b.st, &b.tup, reinterpret_cast<uint64_t*>(b.ctl_host + 14), nullptr};
     }
     return covered == R->pub.n_reads ? np : 0;
 }
 
-// Row materialisation of the np (1 or 2) pieces of a result, each on its own stream; S: the staged piece's uploads, which run inside
-// the timed window.  Sizes first, then one pinned block for the whole result, then the fill.
-static int tuples_materialise(bsq_index* h, TuplePiece* pc, int np, uint32_t flags, const StagedResult* S, bsq_tuples** out) {
-    std::unique_ptr<TuplesImpl> T(new TuplesImpl());   // declared first, so freed last: the cudaFree of the buffers below waits for the device
+// Row materialisation of the np pieces of a result, in read order, each on its own stream and its handle's device.  Sizes on every
+// device, one synchronise, one pinned block for the whole result, then the fill: each piece's byte offsets are moved behind the earlier
+// pieces' bytes on its device, and each device copies its rows into the block.  The hole table is sorted once and uploaded once per
+// device.  Staged uploads run inside the timed window; device_ms is the slowest device's window.  what: the prefix of the messages.
+static int tuples_materialise(TuplePiece* pc, int np, uint32_t flags, const char* what, bsq_tuples** out) {
+    std::unique_ptr<TuplesImpl> T(new TuplesImpl());
     std::vector<TupleHole> holes; std::vector<int64_t> maxend;
-    index_holes_sorted(h, flags, holes, maxend);
-    DevBuf<TupleHole> d_holes; DevBuf<int64_t> d_maxend;
-    Event e0, e1;
-    CUDA_CHECK_AS("bsq_result_tuples", cudaEventCreate(&e0.h)); CUDA_CHECK_AS("bsq_result_tuples", cudaEventCreate(&e1.h));
-    CUDA_CHECK_AS("bsq_result_tuples", d_holes.alloc(holes.size() + 1)); CUDA_CHECK_AS("bsq_result_tuples", d_maxend.alloc(holes.size() + 1));
+    index_holes_sorted(pc[0].h, flags, holes, maxend);
+    // per device: its hole table, the stream its window starts on, and the event its other streams wait for before they read the holes
+    struct DeviceSide { int device = -1; cudaStream_t home = nullptr; DevBuf<TupleHole> holes; DevBuf<int64_t> maxend; Event e0, ready; };
+    std::vector<DeviceSide> dv(np); std::vector<int> dev_of(np); std::vector<Event> e1(np); std::vector<uint64_t> nb(np, 0);
+    std::vector<TupleParams> P(np);
+    int nd = 0;
+    for (int k = 0; k < np; ++k) {
+        int d = 0;
+        while (d < nd && dv[d].device != pc[k].h->device) ++d;
+        if (d == nd) { dv[d].device = pc[k].h->device; dv[d].home = pc[k].st; ++nd; }
+        dev_of[k] = d;
+    }
+    // whatever a failed step left queued ends before the buffers above, the pieces' staging and the output block are freed
+    struct Drain { const TuplePiece* pc; int np; ~Drain() { for (int k = 0; k < np; ++k) { cudaSetDevice(pc[k].h->device); cudaStreamSynchronize(pc[k].st); } } } drain{pc, np};
     uint64_t n_rows = 0;
     for (int k = 0; k < np; ++k) {
         TupleScratch& s = *pc[k].s; const uint64_t nr = pc[k].n_rows;
+        CUDA_CHECK_AS(what, cudaSetDevice(pc[k].h->device));
+        CUDA_CHECK_AS(what, cudaEventCreate(&e1[k].h));
         if (cudaSuccess != s.off.ensure(3 * nr + 2) || cudaSuccess != s.tmp.ensure(tuple_scan_tmp_elems(nr)) || cudaSuccess != s.row_read.ensure(nr + 1) ||
-            cudaSuccess != s.nholes.ensure(2 * nr + 2) || cudaSuccess != s.rm.ensure(3 * nr + 3)) { bsq_set_error("bsq_result_tuples: out of device memory"); return BSQ_ERR; }
+            cudaSuccess != s.nholes.ensure(2 * nr + 2) || cudaSuccess != s.rm.ensure(3 * nr + 3)) { bsq_set_error("%s: out of device memory", what); return BSQ_ERR; }
         n_rows += nr;
     }
-    const cudaStream_t s0 = pc[0].st;
-    cudaEventRecord(e0, s0);
-    if (!holes.empty()) {
-        CUDA_CHECK_AS("bsq_result_tuples", cudaMemcpyAsync(d_holes.p, holes.data(), holes.size() * sizeof(TupleHole), cudaMemcpyHostToDevice, s0));
-        CUDA_CHECK_AS("bsq_result_tuples", cudaMemcpyAsync(d_maxend.p, maxend.data(), holes.size() * 8, cudaMemcpyHostToDevice, s0));
+    for (int d = 0; d < nd; ++d) {
+        DeviceSide& v = dv[d];
+        CUDA_CHECK_AS(what, cudaSetDevice(v.device));
+        CUDA_CHECK_AS(what, cudaEventCreate(&v.e0.h)); CUDA_CHECK_AS(what, cudaEventCreateWithFlags(&v.ready.h, cudaEventDisableTiming));
+        CUDA_CHECK_AS(what, v.holes.alloc(holes.size() + 1)); CUDA_CHECK_AS(what, v.maxend.alloc(holes.size() + 1));
+        CUDA_CHECK_AS(what, cudaEventRecord(v.e0, v.home));
+        if (!holes.empty()) {
+            CUDA_CHECK_AS(what, cudaMemcpyAsync(v.holes.p, holes.data(), holes.size() * sizeof(TupleHole), cudaMemcpyHostToDevice, v.home));
+            CUDA_CHECK_AS(what, cudaMemcpyAsync(v.maxend.p, maxend.data(), holes.size() * 8, cudaMemcpyHostToDevice, v.home));
+        }
+        CUDA_CHECK_AS(what, cudaEventRecord(v.ready, v.home));
     }
-    if (S && stage_upload(*S, s0, &h->timing.launches) != BSQ_OK) return BSQ_ERR;
-    if (np > 1) CUDA_CHECK_AS("bsq_result_tuples", cudaStreamSynchronize(s0));   // the other lane reads the holes
-    TupleParams P[2]; uint64_t nb[2] = {0, 0};
+    bool spans = false;
+    for (int k = 0; k < np; ++k) {   // staged uploads; a part of a result stops after its rows until its CIGAR span is known
+        TuplePiece& c = pc[k];
+        CUDA_CHECK_AS(what, cudaSetDevice(c.h->device));
+        if (c.st != dv[dev_of[k]].home) CUDA_CHECK_AS(what, cudaStreamWaitEvent(c.st, dv[dev_of[k]].ready, 0));
+        if (!c.stage) continue;
+        if (stage_rows(c, what) != BSQ_OK) return BSQ_ERR;
+        if (c.stage->whole) { if (stage_rest(c, what) != BSQ_OK) return BSQ_ERR; } else spans = true;
+    }
+    for (int k = 0; k < np && spans; ++k) {
+        TuplePiece& c = pc[k];
+        if (!c.stage || c.stage->whole) continue;
+        CUDA_CHECK_AS(what, cudaSetDevice(c.h->device)); CUDA_CHECK_AS(what, cudaStreamSynchronize(c.st));
+        if (stage_rest(c, what) != BSQ_OK) return BSQ_ERR;
+    }
     for (int k = 0; k < np; ++k) {       // sizes of every piece
-        const TuplePiece& c = pc[k]; TupleScratch& s = *c.s; const uint64_t nr = c.n_rows;
+        const TuplePiece& c = pc[k]; TupleScratch& s = *c.s; const uint64_t nr = c.n_rows; const DeviceSide& v = dv[dev_of[k]];
         TupleParams& q = P[k];
         q.rows = c.rows; q.n_rows = nr; q.row_read = s.row_read.p; q.cigar = c.cigar; q.seqs = c.seqs; q.offs = c.offs;
-        q.pac = h->d_pac; q.l_pac = h->meta.l_pac; q.ann_offset = h->d_ann_offset;
-        q.holes = d_holes.p; q.hole_maxend = d_maxend.p; q.n_holes = (uint32_t)holes.size();
+        q.pac = c.h->d_pac; q.l_pac = c.h->meta.l_pac; q.ann_offset = c.h->d_ann_offset;
+        q.holes = v.holes.p; q.hole_maxend = v.maxend.p; q.n_holes = (uint32_t)holes.size();
         q.nholes = s.nholes.p; q.off = s.off.p; q.ref_match = s.rm.p; q.bytes = nullptr; q.fix_reverse = (flags & BSQ_TUPLES_FIX_REVERSE) != 0;
         if (!nr) continue;
-        k_row_read<<<(unsigned)std::min<uint64_t>((c.n_reads + 255) / 256, 148 * 8), 256, 0, c.st>>>(c.row_off, c.n_reads, c.row_base, nr, s.row_read.p); ++h->timing.launches;
-        CUDA_CHECK_AS("bsq_result_tuples", cudaMemsetAsync(s.off.p, 0, (3 * nr + 1) * 8, c.st));
-        launch_tuple_sizes(q, s.tmp.p, c.st, &h->timing.launches);
-        CUDA_CHECK_AS("bsq_result_tuples", cudaMemcpyAsync(c.n_bytes, s.off.p + 3 * nr, 8, cudaMemcpyDeviceToHost, c.st));
+        CUDA_CHECK_AS(what, cudaSetDevice(c.h->device));
+        k_row_read<<<(unsigned)std::min<uint64_t>((c.n_reads + 255) / 256, 148 * 8), 256, 0, c.st>>>(c.row_off, c.n_reads, c.row_base, nr, s.row_read.p); ++c.h->timing.launches;
+        CUDA_CHECK_AS(what, cudaMemsetAsync(s.off.p, 0, (3 * nr + 1) * 8, c.st));
+        launch_tuple_sizes(q, s.tmp.p, c.st, &c.h->timing.launches);
+        CUDA_CHECK_AS(what, cudaMemcpyAsync(c.n_bytes, s.off.p + 3 * nr, 8, cudaMemcpyDeviceToHost, c.st));
     }
-    for (int k = 0; k < np; ++k) { CUDA_CHECK_AS("bsq_result_tuples", cudaStreamSynchronize(pc[k].st)); if (pc[k].n_rows) nb[k] = *pc[k].n_bytes; }
-    const uint64_t n_bytes = nb[0] + nb[1];
+    uint64_t n_bytes = 0;
+    for (int k = 0; k < np; ++k) {
+        CUDA_CHECK_AS(what, cudaSetDevice(pc[k].h->device)); CUDA_CHECK_AS(what, cudaStreamSynchronize(pc[k].st));
+        if (pc[k].n_rows) nb[k] = *pc[k].n_bytes;
+        n_bytes += nb[k];
+    }
     const size_t off_b = (3 * n_rows + 1) * 8, rm_b = (n_rows * 12 + 7) & ~(size_t)7;
     T->host = pinned_get(off_b + rm_b + n_bytes + 64, &T->host_bytes);
     if (!T->host) { bsq_set_error("cannot allocate pinned host memory for the tuples"); return BSQ_ERR; }
@@ -1551,23 +1648,30 @@ static int tuples_materialise(bsq_index* h, TuplePiece* pc, int np, uint32_t fla
     uint64_t row_base = 0, byte_base = 0;
     for (int k = 0; k < np; ++k) {
         const TuplePiece& c = pc[k]; TupleScratch& s = *c.s; const uint64_t nr = c.n_rows;
+        CUDA_CHECK_AS(what, cudaSetDevice(c.h->device));
         if (nr) {
-            if (cudaSuccess != s.bytes.ensure(nb[k] + 64)) { bsq_set_error("bsq_result_tuples: out of device memory"); return BSQ_ERR; }
-            CUDA_CHECK_AS("bsq_result_tuples", cudaMemsetAsync(s.bytes.p, 0, nb[k] + 64, c.st));
+            if (cudaSuccess != s.bytes.ensure(nb[k] + 64)) { bsq_set_error("%s: out of device memory", what); return BSQ_ERR; }
+            CUDA_CHECK_AS(what, cudaMemsetAsync(s.bytes.p, 0, nb[k] + 64, c.st));
             P[k].bytes = s.bytes.p;
-            launch_tuple_fill(P[k], c.st, &h->timing.launches);
-            if (byte_base) { k_add_u64<<<(unsigned)std::min<uint64_t>((3 * nr + 256) / 256, 148 * 8), 256, 0, c.st>>>(s.off.p, 3 * nr + 1, byte_base); ++h->timing.launches; }
-            CUDA_CHECK_AS("bsq_result_tuples", cudaMemcpyAsync(T->pub.off + 3 * row_base, s.off.p, (3 * nr + 1) * 8, cudaMemcpyDeviceToHost, c.st));
-            CUDA_CHECK_AS("bsq_result_tuples", cudaMemcpyAsync(T->pub.ref_match + 3 * row_base, s.rm.p, nr * 12, cudaMemcpyDeviceToHost, c.st));
-            CUDA_CHECK_AS("bsq_result_tuples", cudaMemcpyAsync(T->pub.bytes + byte_base, s.bytes.p, nb[k], cudaMemcpyDeviceToHost, c.st));
+            launch_tuple_fill(P[k], c.st, &c.h->timing.launches);
+            if (byte_base) { k_add_u64<<<(unsigned)std::min<uint64_t>((3 * nr + 256) / 256, 148 * 8), 256, 0, c.st>>>(s.off.p, 3 * nr + 1, byte_base); ++c.h->timing.launches; }
+            CUDA_CHECK_AS(what, cudaMemcpyAsync(T->pub.off + 3 * row_base, s.off.p, (3 * nr + 1) * 8, cudaMemcpyDeviceToHost, c.st));
+            CUDA_CHECK_AS(what, cudaMemcpyAsync(T->pub.ref_match + 3 * row_base, s.rm.p, nr * 12, cudaMemcpyDeviceToHost, c.st));
+            CUDA_CHECK_AS(what, cudaMemcpyAsync(T->pub.bytes + byte_base, s.bytes.p, nb[k], cudaMemcpyDeviceToHost, c.st));
         }
+        CUDA_CHECK_AS(what, cudaEventRecord(e1[k], c.st));
         row_base += nr; byte_base += nb[k];
     }
-    for (int k = 1; k < np; ++k) CUDA_CHECK_AS("bsq_result_tuples", cudaStreamSynchronize(pc[k].st));
-    cudaEventRecord(e1, s0);
-    CUDA_CHECK_AS("bsq_result_tuples", cudaStreamSynchronize(s0)); CUDA_CHECK_AS("bsq_result_tuples", cudaGetLastError());
+    float ms = 0.f;
+    for (int k = 0; k < np; ++k) {
+        CUDA_CHECK_AS(what, cudaSetDevice(pc[k].h->device)); CUDA_CHECK_AS(what, cudaStreamSynchronize(pc[k].st));
+        float t = 0.f;
+        CUDA_CHECK_AS(what, cudaEventElapsedTime(&t, dv[dev_of[k]].e0, e1[k]));
+        ms = std::max(ms, t);
+    }
+    CUDA_CHECK_AS(what, cudaGetLastError());
     T->pub.off[3 * n_rows] = n_bytes;
-    cudaEventElapsedTime(&T->pub.device_ms, e0, e1);
+    T->pub.device_ms = ms;
     *out = &T.release()->pub;
     return BSQ_OK;
 }
@@ -1582,7 +1686,7 @@ int bsq_result_tuples(bsq_index* h, const bsq_result* res, const char* seqs, con
         if (mine && h->meta.built) {
             if (cudaSetDevice(h->device) != cudaSuccess) { bsq_set_error("cudaSetDevice failed"); return BSQ_ERR; }
             TuplePiece pc[2];
-            if (const int np = resident_pieces(h, mine, pc)) return tuples_materialise(h, pc, np, flags, nullptr, out);
+            if (const int np = resident_pieces(h, mine, pc)) return tuples_materialise(pc, np, flags, "bsq_result_tuples", out);
         }
     }
     if (!offs) { bsq_set_error("null argument"); return BSQ_ERR; }
@@ -1590,15 +1694,9 @@ int bsq_result_tuples(bsq_index* h, const bsq_result* res, const char* seqs, con
     CUDA_CHECK(cudaSetDevice(h->device));
     const uint64_t n_reads = res->n_reads, n_rows = n_reads ? res->row_off[n_reads] : 0;
     if (n_rows && !seqs) { bsq_set_error("null argument"); return BSQ_ERR; }
-    StagedResult S;
-    if (n_rows) {
-        S.res = res; S.seqs = seqs; S.offs = offs;
-        CUDA_CHECK_AS("bsq_result_tuples", S.rows.alloc(n_rows)); CUDA_CHECK_AS("bsq_result_tuples", S.cigar.alloc(res->n_cigar_words + 1));
-        CUDA_CHECK_AS("bsq_result_tuples", S.text.alloc(offs[n_reads] - offs[0] + 64));
-        CUDA_CHECK_AS("bsq_result_tuples", S.row_off.alloc(n_reads)); CUDA_CHECK_AS("bsq_result_tuples", S.read_off.alloc(n_reads + 1));
-    }
-    TuplePiece pc{S.rows.p, n_rows, S.cigar.p, S.text.p, S.read_off.p, S.row_off.p, n_reads, 0, h->stream, &S.s, &S.n_bytes};
-    return tuples_materialise(h, &pc, 1, flags, n_rows ? &S : nullptr, out);
+    StagedResult S; TuplePiece pc;
+    if (stage_block(h, S, res, seqs, offs, 0, n_reads, "bsq_result_tuples", pc) != BSQ_OK) return BSQ_ERR;
+    return tuples_materialise(&pc, 1, flags, "bsq_result_tuples", out);
 }
 
 void bsq_tuples_free(bsq_tuples* t) { delete reinterpret_cast<TuplesImpl*>(t); }
@@ -1923,8 +2021,8 @@ bsq_multi* bsq_multi_new(bsq_index* built, const int* devices, int n_devices) {
         m->ix.push_back(r);
         r->flags = built->flags;
         if (bsq_index_alloc_replica(r, &built->meta) != BSQ_OK) { ok = false; break; }
-        int can = 0;
-        cudaDeviceCanAccessPeer(&can, devices[k], built->device);
+        int can = 0;   // a repeated device: the peer copies below are device-to-device copies, no peer access to enable
+        if (devices[k] != built->device) cudaDeviceCanAccessPeer(&can, devices[k], built->device);
         if (can) { cudaSetDevice(devices[k]); cudaDeviceEnablePeerAccess(built->device, 0); cudaGetLastError(); }
         for (int what = 0; what < BSQ_ARR_COUNT && ok; ++what) {
             const uint64_t nb = built->meta.arr_bytes[what];
@@ -2045,6 +2143,38 @@ int bsq_multi_last_timing(const bsq_multi* m, bsq_timing* t) {
     if (!m || !t) { bsq_set_error("null argument"); return BSQ_ERR; }
     *t = m->timing;
     return BSQ_OK;
+}
+
+int bsq_multi_result_tuples(bsq_multi* m, const bsq_result* res, const char* seqs, const uint64_t* offs, uint32_t flags, bsq_tuples** out) {
+    BSQ_ENTRY();
+    if (!m || !res || !out) { bsq_set_error("null argument"); return BSQ_ERR; }
+    for (const bsq_index* h : m->ix)
+        if (h->replica_pending) { bsq_set_error("replica without host state: call bsq_index_replica_finish after filling its arrays (the hole overlay of ref_subseq lives on the host)"); return BSQ_ERR; }
+    const ResultImpl* mine = nullptr;
+    { std::lock_guard<std::mutex> lk(g_live_mu); for (const ResultImpl* r : g_live) if (&r->pub == res) { mine = r; break; } }
+    // block d of the reads, as multi_align cut them: served from device d's batch while that batch still holds exactly it
+    const size_t D = m->ix.size(); const uint64_t n = res->n_reads;
+    std::vector<uint64_t> lo(D + 1);
+    for (size_t d = 0; d <= D; ++d) lo[d] = n * d / D;
+    std::vector<char> resident(D);
+    bool staged = false, staged_rows = false;
+    for (size_t d = 0; d < D; ++d) {
+        const Batch& b = m->ix[d]->batch; const uint64_t cnt = lo[d + 1] - lo[d];
+        resident[d] = cnt && mine && b.aligned && b.res_serial == mine->serial && b.res_read_base == lo[d] && b.n == cnt;
+        if (!resident[d] && cnt) { staged = true; staged_rows |= res->row_off[lo[d + 1]] > (lo[d] ? res->row_off[lo[d]] : 0); }
+    }
+    if ((staged && !offs) || (staged_rows && !seqs)) { bsq_set_error("null argument"); return BSQ_ERR; }
+    std::vector<TuplePiece> pc(D); std::vector<StagedResult> S(D);
+    int rc = BSQ_OK;
+    for (size_t d = 0; d < D && rc == BSQ_OK; ++d) {
+        bsq_index* h = m->ix[d]; Batch& b = h->batch;
+        if (resident[d]) pc[d] = TuplePiece{h, b.rows_compact.p, b.out_rows, b.cigar.p - b.cig_rebased, b.ascii.p, b.offs.p, b.row_off64.p, b.n,
+                                            b.res_row_base, b.st, &b.tup, reinterpret_cast<uint64_t*>(b.ctl_host + 14), nullptr};
+        else rc = stage_block(h, S[d], res, seqs, offs, lo[d], lo[d + 1] - lo[d], "bsq_multi_result_tuples", pc[d]);
+    }
+    if (rc == BSQ_OK) rc = tuples_materialise(pc.data(), (int)D, flags, "bsq_multi_result_tuples", out);
+    cudaSetDevice(m->ix[0]->device);
+    return rc;
 }
 
 }  // extern "C"

@@ -172,23 +172,20 @@ std::string BwaIndex::extract_reference_subseq(int64_t rb, int64_t re) const {
     return subseq;
 }
 
-std::vector<std::vector<BwaMatch>> BwaIndex::align_sequences(const std::vector<const NucleotideSequence*>& seqs) {
-    std::vector<std::vector<BwaMatch>> out(seqs.size());
-    if (pac_forward.empty() || seqs.empty()) return out;
-    std::string cat;
-    std::vector<uint64_t> offs(seqs.size() + 1, 0);
-    std::vector<int64_t> ids(seqs.size());
-    std::vector<std::string> texts(seqs.size());
+void BwaIndex::batch_of(const std::vector<const NucleotideSequence*>& seqs, std::string& cat, std::vector<uint64_t>& offs, std::vector<int64_t>& ids) {
+    offs.assign(seqs.size() + 1, 0);
+    ids.resize(seqs.size());
     for (size_t i = 0; i < seqs.size(); ++i) {
-        texts[i] = seqs[i]->to_text();
-        cat += texts[i];
+        cat += seqs[i]->to_text();
         offs[i + 1] = cat.size();
         lrand_state = (lrand_state * 0x5DEECE66DULL + 0xBULL) & 0xFFFFFFFFFFFFULL;   // id = lrand48()
         ids[i] = (int64_t)(lrand_state >> 17);
     }
-    bsq_result* res = nullptr;
-    if (bsq_align_batch(index, cat.data(), offs.data(), ids.data(), seqs.size(), &res) != BSQ_OK) fail();
-    for (size_t i = 0; i < seqs.size(); ++i) {
+}
+
+std::vector<std::vector<BwaMatch>> BwaIndex::matches_of(const bsq_result* res, const std::string& cat, const std::vector<uint64_t>& offs) const {
+    std::vector<std::vector<BwaMatch>> out(offs.size() - 1);
+    for (size_t i = 0; i < out.size(); ++i) {
         for (uint64_t k = res->row_off[i]; k < res->row_off[i + 1]; ++k) {
             const bsq_row& a = res->rows[k];
             const int64_t ref_offset = offsets[(size_t)a.rid];
@@ -198,7 +195,7 @@ std::vector<std::vector<BwaMatch>> BwaIndex::align_sequences(const std::vector<c
             m.ref_match_begin = (int32_t)(a.rb - ref_offset);
             m.ref_match_end = (int32_t)(a.re - ref_offset);
             m.ref_match_len = (int32_t)(a.re - a.rb);
-            m.query_subseq = texts[i].substr((size_t)a.qb, (size_t)(a.qe - a.qb));
+            m.query_subseq = cat.substr((size_t)(offs[i] + a.qb), (size_t)(a.qe - a.qb));
             m.query_match_begin = a.qb; m.query_match_end = a.qe; m.query_match_len = a.qe - a.qb;
             m.is_primary = (a.flag & 0x100) == 0; m.is_secondary = (a.flag & 0x100) != 0; m.is_reverse = a.is_rev != 0;
             m.cigar = cigar_compressed_to_string(res->cigar + a.cigar_off, (int)a.n_cigar);
@@ -206,25 +203,59 @@ std::vector<std::vector<BwaMatch>> BwaIndex::align_sequences(const std::vector<c
             out[i].push_back(std::move(m));
         }
     }
+    return out;
+}
+
+std::vector<std::vector<BwaMatch>> BwaIndex::align_sequences(const std::vector<const NucleotideSequence*>& seqs) {
+    if (pac_forward.empty() || seqs.empty()) return std::vector<std::vector<BwaMatch>>(seqs.size());
+    std::string cat; std::vector<uint64_t> offs; std::vector<int64_t> ids;
+    batch_of(seqs, cat, offs, ids);
+    bsq_result* res = nullptr;
+    if (bsq_align_batch(index, cat.data(), offs.data(), ids.data(), seqs.size(), &res) != BSQ_OK) fail();
+    auto out = matches_of(res, cat, offs);
     bsq_result_free(res);
     return out;
 }
 
 BwaTupleBatch BwaIndex::align_sequences_tuples(const std::vector<const NucleotideSequence*>& seqs, uint32_t flags) {
     if (pac_forward.empty() || seqs.empty()) return BwaTupleBatch();
-    std::string cat;
-    std::vector<uint64_t> offs(seqs.size() + 1, 0);
-    std::vector<int64_t> ids(seqs.size());
-    for (size_t i = 0; i < seqs.size(); ++i) {
-        cat += seqs[i]->to_text();
-        offs[i + 1] = cat.size();
-        lrand_state = (lrand_state * 0x5DEECE66DULL + 0xBULL) & 0xFFFFFFFFFFFFULL;   // id = lrand48()
-        ids[i] = (int64_t)(lrand_state >> 17);
-    }
+    std::string cat; std::vector<uint64_t> offs; std::vector<int64_t> ids;
+    batch_of(seqs, cat, offs, ids);
     bsq_result* res = nullptr;
     if (bsq_align_batch(index, cat.data(), offs.data(), ids.data(), seqs.size(), &res) != BSQ_OK) fail();
     bsq_tuples* tup = nullptr;
     if (bsq_result_tuples(index, res, cat.data(), offs.data(), flags, &tup) != BSQ_OK) { bsq_result_free(res); fail(); }
+    return BwaTupleBatch(res, tup);
+}
+
+// ---- BwaMultiIndex
+BwaMultiIndex::BwaMultiIndex(BwaIndex& ix_, const std::vector<int>& devices) : ix(ix_) {
+    if (ix.pac_forward.empty()) return;
+    multi = bsq_multi_new(ix.index, devices.data(), (int)devices.size());
+    if (!multi) fail();
+}
+
+BwaMultiIndex::~BwaMultiIndex() { bsq_multi_free(multi); }
+
+std::vector<std::vector<BwaMatch>> BwaMultiIndex::align_sequences(const std::vector<const NucleotideSequence*>& seqs) {
+    if (!multi || seqs.empty()) return std::vector<std::vector<BwaMatch>>(seqs.size());
+    std::string cat; std::vector<uint64_t> offs; std::vector<int64_t> ids;
+    ix.batch_of(seqs, cat, offs, ids);
+    bsq_result* res = nullptr;
+    if (bsq_multi_align_batch(multi, cat.data(), offs.data(), ids.data(), seqs.size(), &res) != BSQ_OK) fail();
+    auto out = ix.matches_of(res, cat, offs);
+    bsq_result_free(res);
+    return out;
+}
+
+BwaTupleBatch BwaMultiIndex::align_sequences_tuples(const std::vector<const NucleotideSequence*>& seqs, uint32_t flags) {
+    if (!multi || seqs.empty()) return BwaTupleBatch();
+    std::string cat; std::vector<uint64_t> offs; std::vector<int64_t> ids;
+    ix.batch_of(seqs, cat, offs, ids);
+    bsq_result* res = nullptr;
+    if (bsq_multi_align_batch(multi, cat.data(), offs.data(), ids.data(), seqs.size(), &res) != BSQ_OK) fail();
+    bsq_tuples* tup = nullptr;
+    if (bsq_multi_result_tuples(multi, res, cat.data(), offs.data(), flags, &tup) != BSQ_OK) { bsq_result_free(res); fail(); }
     return BwaTupleBatch(res, tup);
 }
 

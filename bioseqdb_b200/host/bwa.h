@@ -84,12 +84,36 @@ public:
 
 private:
     friend class BwaIndexCache;
+    friend class BwaMultiIndex;
     std::vector<uint8_t> pac_forward;      // kept on the host for extract_reference_subseq (bwa.cpp:55-68)
     std::vector<bsq_hole> holes;           // not rebased, as in the reference (bwa.cpp:100-104)
     std::vector<int64_t> offsets;
     bsq_index* index;
     uint64_t lrand_state;                  // glibc lrand48 state: one draw per aligned read (SURVEY.md A.10)
     std::string extract_reference_subseq(int64_t ref_begin, int64_t ref_end) const;
+    // the reads as one text with offsets, and their ids: one lrand48 draw per read from the session state
+    void batch_of(const std::vector<const NucleotideSequence*>& seqs, std::string& cat, std::vector<uint64_t>& offs, std::vector<int64_t>& ids);
+    // the BwaMatch rows of every read of `res`, computed from the reads in cat / offs
+    std::vector<std::vector<BwaMatch>> matches_of(const bsq_result* res, const std::string& cat, const std::vector<uint64_t>& offs) const;
+};
+
+// Several GPUs behind one backend (bsq_multi_*): the built `ix` replicated to `devices` (devices[0] is the device `ix` lives on; a
+// device may repeat).  A batch is cut into one contiguous block of reads per device and its rows come back in read order, with ids
+// drawn from ix's session lrand48 state exactly as BwaIndex draws them.  Options and flags are those of `ix`; it must outlive this.
+class BwaMultiIndex {
+public:
+    BwaMultiIndex(BwaIndex& ix, const std::vector<int>& devices);
+    ~BwaMultiIndex();
+    BwaMultiIndex(const BwaMultiIndex&) = delete;
+    BwaMultiIndex& operator=(const BwaMultiIndex&) = delete;
+
+    std::vector<std::vector<BwaMatch>> align_sequences(const std::vector<const NucleotideSequence*>& seqs);
+    // each device materialises the tuples of its own block from HBM (bsq_multi_result_tuples)
+    BwaTupleBatch align_sequences_tuples(const std::vector<const NucleotideSequence*>& seqs, uint32_t flags = 0);
+
+private:
+    BwaIndex& ix;
+    bsq_multi* multi = nullptr;            // none while `ix` holds no reference rows: every call then returns no rows, as BwaIndex's
 };
 
 // Index cache keyed by the content of the reference rows (SURVEY.md 8f-1).  The reference rebuilds a BwaIndex inside

@@ -9,6 +9,8 @@
 // text -> NUCLSEQ conversion and are compared with nuclseq_from_text.  A difference is an error (exit code 1).
 // With index_cache=DIR the index comes from a BwaIndexCache with that directory, as a backend's would: the first process builds
 // it and writes DIR/<digest>.bsqidx, every later one loads that file.  The counters go to stderr ("index_cache: ...").
+// With devices=0,1 the batch is aligned (and, with check_tuples=1, materialised) on those GPUs through BwaMultiIndex, one contiguous
+// block of reads per device, as a backend that drives several GPUs would; the output is the same.
 #include <cstdio>
 #include <cstring>
 #include <fstream>
@@ -41,9 +43,19 @@ int main(int argc, char** argv) {
     if (argc < 3) { fprintf(stderr, "usage: %s reference.tsv queries.tsv [bwa_options name=value ...]\n", argv[0]); return 2; }
     try {
         std::map<std::string, int32_t> opts;
-        std::string index_cache;               // a string option: taken out before the int options are parsed
+        std::string index_cache;               // string options: taken out before the int options are parsed
+        std::vector<int> devices;
         for (int i = 3; i < argc; ++i) {
             if (strncmp(argv[i], "index_cache=", 12) == 0) { index_cache = argv[i] + 12; continue; }
+            if (strncmp(argv[i], "devices=", 8) == 0) {
+                for (const char* p = argv[i] + 8; *p;) {
+                    char* end = nullptr;
+                    devices.push_back((int)strtol(p, &end, 10));
+                    if (end == p || (*end && *end != ',')) throw std::runtime_error("devices is a comma-separated list of device numbers");
+                    p = *end ? end + 1 : end;
+                }
+                continue;
+            }
             const char* eq = strchr(argv[i], '=');
             if (!eq) throw std::runtime_error("options are name=value");
             opts[std::string(argv[i], (size_t)(eq - argv[i]))] = (int32_t)atoi(eq + 1);
@@ -92,12 +104,14 @@ int main(int argc, char** argv) {
                     (unsigned long long)cache->disk_saves, (unsigned long long)cache->disk_errors);
         }
         BwaIndex& bwa = *ix;
+        std::unique_ptr<BwaMultiIndex> multi;
+        if (!devices.empty()) multi.reset(new BwaMultiIndex(bwa, devices));
         std::vector<int64_t> qids; std::vector<NucleotideSequence> queries;
         iterate_nuclseq_table(argv[2], [&](int64_t id, NucleotideSequence s) { qids.push_back(id); queries.push_back(std::move(s)); });
         std::vector<const NucleotideSequence*> ptrs;
         for (auto& q : queries) ptrs.push_back(&q);
         const uint64_t ids_at = bwa.session_lrand_state();
-        auto all = bwa.align_sequences(ptrs);
+        auto all = multi ? multi->align_sequences(ptrs) : bwa.align_sequences(ptrs);
         auto datum_of = [](const NucleotideSequence& s) {   // the datum as PostgreSQL stores it: length word + varlena payload
             std::vector<uint8_t> pl = s.varlena_payload();
             std::vector<uint8_t> d(4 + pl.size());
@@ -107,7 +121,7 @@ int main(int argc, char** argv) {
         };
         if (check_tuples) {
             bwa.session_lrand_state() = ids_at;
-            BwaTupleBatch tb = bwa.align_sequences_tuples(ptrs);
+            BwaTupleBatch tb = multi ? multi->align_sequences_tuples(ptrs) : bwa.align_sequences_tuples(ptrs);
             size_t n_rows = 0;
             for (size_t i = 0; i < all.size(); ++i) {
                 if (tb.row_begin(i + 1) - tb.row_begin(i) != all[i].size()) throw std::runtime_error("tuples: row count differs");

@@ -221,6 +221,14 @@ int bsq_multi_devices(const bsq_multi* m);
 int bsq_multi_align_batch(bsq_multi* m, const char* seqs, const uint64_t* offs, const int64_t* ids, uint64_t n, bsq_result** out);
 int bsq_multi_align_batch_datums(bsq_multi* m, const uint8_t* bytes, const uint64_t* off, const int64_t* ids, uint64_t n, bsq_result** out);
 int bsq_multi_last_timing(const bsq_multi* m, bsq_timing* t);   /* total = the slowest device's time from its first copy to the end of its download */
+/* Row materialisation of a result on every device of `m`: the same tuples, byte for byte, as bsq_result_tuples(built, res, seqs, offs,
+ * flags, ...), in one pinned block with the rows in read order, freed by bsq_tuples_free.  The reads are cut into the blocks of
+ * bsq_multi_align_batch* (block d = reads [n d / D, n (d + 1) / D)) and device d builds the rows of block d.  A device whose batch still
+ * holds that block of `res` (the latest bsq_multi_align_batch* call) takes rows, CIGARs and reads from HBM and uploads nothing; any other
+ * device uploads only its block's rows, CIGAR words and reads.  seqs / offs may be NULL only when every device serves its block from HBM.
+ * Any result is accepted: a caller-assembled, older or single-device result is staged across all devices.  device_ms = the slowest
+ * device's kernels + copies.  An error on any device fails the call. */
+int bsq_multi_result_tuples(bsq_multi* m, const bsq_result* res, const char* seqs, const uint64_t* offs, uint32_t flags, bsq_tuples** out);
 /* Check of the device index against the text it was built from, by kernels that share no code with the builder or the seeding
  * kernels: SA is a permutation of 0..n (sum / sum of squares over all rows), adjacent suffixes are in order (text comparison), the BWT
  * string is T[SA[k]-1], bwt_invPsi(k) = L2[c] + occ(k, c) lands on the row of SA[k]-1 (what bwt_sa / bwt_extend rely on, libbwa bwt.c
