@@ -70,7 +70,7 @@ class BsqTiming(C.Structure):
 class BsqMeta(C.Structure):
     _fields_ = [("l_pac", C.c_int64), ("seq_len", C.c_uint64), ("primary", C.c_uint64), ("L2", C.c_uint64 * 5), ("n_anns", C.c_uint64),
                 ("sa_bytes", C.c_uint32), ("built", C.c_uint32), ("arr_bytes", C.c_uint64 * ARR_COUNT), ("build_ms", C.c_double),
-                ("build_launches", C.c_uint64), ("sort_pass_bytes", C.c_uint64)]
+                ("build_launches", C.c_uint64), ("sort_pass_bytes", C.c_uint64), ("sa_interval", C.c_uint32), ("reserved", C.c_uint32)]
 
 
 class BsqIndexCheck(C.Structure):
@@ -151,6 +151,7 @@ def lib():
     L.bsq_index_bwt_plain.argtypes = [vp, vp]
     L.bsq_index_sa_sampled.argtypes = [vp, vp, u64]
     L.bsq_debug_seed.argtypes = [vp, vp, vp, u64, vp, u32, vp]
+    L.bsq_debug_sa_lookup.argtypes = [vp, vp, u64, vp]
     L.bsq_debug_ksw_extend.argtypes = [C.POINTER(BsqOpts), C.c_int, u64, vp, vp, vp, vp, vp, vp, vp, vp]
     L.bsq_debug_ksw_extend_thread.argtypes = [C.POINTER(BsqOpts), C.c_int, u64, vp, vp, vp, vp, vp, vp, vp, vp, C.c_int]
     L.bsq_debug_ksw_global.argtypes = [C.POINTER(BsqOpts), C.c_int, u64, vp, vp, vp, vp, vp, vp, vp, u32, vp]
@@ -168,7 +169,7 @@ ABI_SYMBOLS = [
     "bsq_last_error", "bsq_device_count", "bsq_opts_init", "bsq_index_new", "bsq_index_set_opts", "bsq_index_set_flags", "bsq_index_add_ref", "bsq_index_add_ref_datums", "bsq_index_build",
     "bsq_index_free", "bsq_align_batch", "bsq_align_batch_datums", "bsq_session_lrand48", "bsq_result_free", "bsq_last_timing", "bsq_result_tuples", "bsq_tuples_free", "bsq_nuclseq_from_text_batch", "bsq_nuclseqs_free", "bsq_reads_upload", "bsq_align_resident", "bsq_result_download",
     "bsq_index_get_meta", "bsq_index_device_bytes", "bsq_index_device_ptr", "bsq_index_download", "bsq_index_alloc_replica", "bsq_index_host_state_size", "bsq_index_host_state_get", "bsq_index_replica_finish", "bsq_index_prepare", "bsq_index_save", "bsq_index_load", "bsq_index_last_load", "bsq_multi_new", "bsq_multi_free", "bsq_multi_devices", "bsq_multi_align_batch", "bsq_multi_align_batch_datums", "bsq_multi_last_timing", "bsq_multi_result_tuples", "bsq_index_bwt_plain", "bsq_index_sa_sampled",
-    "bsq_debug_seed", "bsq_debug_ksw_extend", "bsq_debug_ksw_extend_thread", "bsq_debug_ksw_global", "bsq_bench_gather", "bsq_bench_dpx", "bsq_set_counters", "bsq_get_counters", "bsq_debug_ctl", "bsq_index_verify",
+    "bsq_debug_seed", "bsq_debug_sa_lookup", "bsq_debug_ksw_extend", "bsq_debug_ksw_extend_thread", "bsq_debug_ksw_global", "bsq_bench_gather", "bsq_bench_dpx", "bsq_set_counters", "bsq_get_counters", "bsq_debug_ctl", "bsq_index_verify",
 ]
 
 

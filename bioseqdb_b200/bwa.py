@@ -240,6 +240,14 @@ class BwaIndex:
         check(self.L.bsq_index_bwt_plain(self.h, ptr(out)))
         return out
 
+    def sa_lookup(self, rows) -> np.ndarray:
+        """bwt_sa of each row in [0, seq_len] (bsq_debug_sa_lookup): SA[row] on a full index, the LF walk of the alignment pipeline's
+        position resolve pass on a compact one (meta().sa_interval == 32).  Row 0 gives seq_len."""
+        r = np.ascontiguousarray(rows, dtype=np.uint64)
+        out = np.empty(len(r), dtype=np.uint64)
+        check(self.L.bsq_debug_sa_lookup(self.h, ptr(r), len(r), ptr(out)))
+        return out
+
     def sa_sampled(self) -> np.ndarray:
         m = self.meta()
         n_sa = (int(m.seq_len) + 32) // 32

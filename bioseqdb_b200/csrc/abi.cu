@@ -90,7 +90,8 @@ struct Batch {
     DevBuf<double> read_logtab; uint32_t read_logtab_n = 0; uint32_t rseq_cap = 0;
     DevBuf<uint8_t> ext_scratch, fin_scratch, narrow_z, narrow_jobs; DevBuf<uint64_t> wide_jobs;
     DevBuf<ExtMemo> ext_memo; DevBuf<uint8_t> ext_memo_key; DevBuf<uint32_t> ext_memo_perm, ext_memo_hist, ext_todo, chain_todo, fin_todo, seed_todo, seed_pk, seed_u32;   // thread-per-extension pre-pass (extend_plan.cu)
-    DevBuf<uint32_t> ctl;  // [0..3] tickets, [4] overflow, [5] pool_top, [6] cigar_top, [8..23] counters (u64 x 8), [24] narrow_cnt, [25] wide_cnt, [26..27] tickets, [56] reads left for sw_extend, [57] reads left for the warp chain kernel, [58] for regs_finalize
+    DevBuf<uint64_t> sa_pos, sa_pos_off;   // compact index: the position resolve pass (sa_resolve.cu), pool_cap slots / n + 1 offsets
+    DevBuf<uint32_t> ctl;  // [0..3] tickets, [4] overflow, [5] pool_top, [6] cigar_top, [8..23] counters (u64 x 8), [24] narrow_cnt, [25] wide_cnt, [26..27] tickets, [28..29] LF steps of the resolve pass (u64), [31] its ticket, [51] its error, [54..55] its warp iterations (u64), [56] reads left for sw_extend, [57] reads left for the warp chain kernel, [58] for regs_finalize
     // f(buf) for every DevBuf above: the one list release() frees and device_bytes() counts (BwaIndexCache's eviction budget)
     template <class B, class F> static void each(B& b, F f) {
         f(b.seqs); f(b.offs); f(b.ids); f(b.datums); f(b.datum_off); f(b.scan_tmp64); f(b.ascii); f(b.row_off64);
@@ -99,7 +100,7 @@ struct Batch {
         f(b.regs); f(b.rows); f(b.rows_compact); f(b.rows_ext); f(b.reg_cnt); f(b.row_cnt); f(b.row_off); f(b.scan_tmp); f(b.blocks); f(b.cigar);
         f(b.read_logtab); f(b.ext_scratch); f(b.fin_scratch); f(b.narrow_z); f(b.narrow_jobs); f(b.wide_jobs);
         f(b.ext_memo); f(b.ext_memo_key); f(b.ext_memo_perm); f(b.ext_memo_hist); f(b.ext_todo); f(b.chain_todo); f(b.fin_todo); f(b.seed_todo); f(b.seed_pk); f(b.seed_u32);
-        f(b.ctl);
+        f(b.sa_pos); f(b.sa_pos_off); f(b.ctl);
     }
     size_t device_bytes() const { size_t n = 0; each(*this, [&](const auto& d) { n += d.bytes(); }); return n; }
     bool resident = false, aligned = false;
@@ -107,11 +108,11 @@ struct Batch {
     // and the state of the attempt in flight (pipeline_enqueue -> pipeline_check)
     cudaStream_t st = nullptr;
     std::vector<bsq_row_ext> ext_tmp;   // extension records fetched only to finish a MAPQ on the host
-    uint32_t* ctl_host = nullptr;       // pinned, 16 words: ctl[0..7], total rows (2 words), host-MAPQ flag
+    uint32_t* ctl_host = nullptr;       // pinned, 16 words: ctl[0..7], total rows (2 words), host-MAPQ flag, error of the resolve pass
     cudaEvent_t ev[5]; bool ev_ok = false;
     cudaEvent_t ev_x[4]; bool evx_ok = false;   // chunked mode: upload begin/end, download begin/end
     ExtAux ext_aux; bool ext_aux_ok = false;    // side streams of the extension pre-pass
-    uint32_t att_rseq_cap = 0; bool idle = true;
+    uint32_t att_rseq_cap = 0; bool idle = true; bool att_compact = false;   // att_compact: the attempt in flight resolved positions (sa_resolve.cu)
     uint64_t out_rows = 0; uint32_t out_cig = 0;
     uint64_t rows_cap = 0;              // capacity of rows_compact (rows of the batch in read order)
     void release() {
@@ -137,7 +138,7 @@ struct bsq_index {
     cudaStream_t stream2 = nullptr;
     bsq_timing timing;
     double* d_logtab = nullptr;
-    void* d_isa = nullptr;           // inverse SA for the unique-match shortcut of the seeding kernel (built lazily, rows as wide as the SA's)
+    void* d_isa = nullptr;           // inverse SA for the unique-match shortcut of the seeding kernel (built lazily, rows as wide as the SA's; never on a compact index)
     uint32_t* d_kmer_z = nullptr;    // sizes-only copy of the prefix table
     void* d_kmer = nullptr; int kmer_k = 0;          // k-mer table of the LAST-like seeding pass (built lazily per device index)
     bool collect_counters = false;
@@ -179,7 +180,13 @@ static int check_opts(const bsq_opts* o) {
     return BSQ_OK;
 }
 
-namespace { DevIndex make_dev_index(const bsq_index* h); int ensure_kmer_table(bsq_index* h, const DevIndex& ix); }
+namespace { DevIndex make_dev_index(const bsq_index* h); int ensure_kmer_table(bsq_index* h); }
+
+// Test hook BSQ_TEST_COMPACT=1, read each time it could take effect: the allocation of the inverse SA and the allocation of the full SA
+// by bsq_index_load "fail" as if device memory were short, so that tests reach the compact layout on references of any size.
+static bool test_compact() { const char* v = getenv("BSQ_TEST_COMPACT"); return v && v[0] == '1' && v[1] == 0; }
+// the meta of the compact layout of an index: every 32nd SA entry, as wide as the full SA's
+static void compact_meta(bsq_index_meta& m) { m.sa_interval = 32; m.arr_bytes[BSQ_ARR_SA] = (m.seq_len + 32) / 32 * m.sa_bytes; }
 
 extern "C" {
 
@@ -310,7 +317,7 @@ int bsq_index_build(bsq_index* h) {
     h->d_occ = B.d_occ; h->d_sa = B.d_sa;
     bsq_index_meta& m = h->meta;
     m.l_pac = B.l_pac; m.seq_len = B.seq_len; m.primary = B.primary; memcpy(m.L2, B.L2, sizeof(m.L2));
-    m.n_anns = h->ann_offset.size(); m.sa_bytes = (uint32_t)B.sa_bytes; m.built = 1;
+    m.n_anns = h->ann_offset.size(); m.sa_bytes = (uint32_t)B.sa_bytes; m.built = 1; m.sa_interval = 1;
     m.arr_bytes[BSQ_ARR_PAC] = h->pac.size(); m.arr_bytes[BSQ_ARR_OCC] = B.occ_bytes; m.arr_bytes[BSQ_ARR_SA] = (B.seq_len + 1) * B.sa_bytes;
     m.arr_bytes[BSQ_ARR_ANN_OFFSET] = m.n_anns * 8; m.arr_bytes[BSQ_ARR_ANN_LEN] = m.n_anns * 4; m.arr_bytes[BSQ_ARR_ANN_ID] = m.n_anns * 8;
     m.build_ms = B.build_ms; m.build_launches = B.launches; m.sort_pass_bytes = B.sort_pass_bytes;
@@ -342,7 +349,7 @@ int bsq_index_device_bytes(const bsq_index* h, uint64_t* bytes) {
     uint64_t b = h->batch.device_bytes() + h->batch2.device_bytes();
     if (h->meta.built) {
         const uint64_t n = h->meta.seq_len;
-        b += (h->meta.l_pac + 3) / 4 + ((n + 127) / 128 + 1) * 64 + (n + 1) * h->meta.sa_bytes + h->meta.n_anns * 20;
+        b += (h->meta.l_pac + 3) / 4 + ((n + 127) / 128 + 1) * 64 + h->meta.arr_bytes[BSQ_ARR_SA] + h->meta.n_anns * 20;
         if (h->d_isa) b += (n + 1) * (uint64_t)h->meta.sa_bytes + 64;
         if (h->d_kmer) b += kmer_table_bytes(h->kmer_k);
         if (h->d_kmer_z) b += kmer_table_bytes(h->kmer_k) / 4;
@@ -378,15 +385,21 @@ int bsq_index_download(const bsq_index* h, int what, void* dst, uint64_t bytes) 
 }  // extern "C"
 
 // The arrays of an index described by *m, to be filled from elsewhere (a peer copy, a file); the handle answers once
-// replica_finish has run.
-static int alloc_replica(bsq_index* h, const bsq_index_meta* m) {
+// replica_finish has run.  may_compact: when the full SA does not fit, allocate the compact layout instead (h->meta says which).
+static int alloc_replica(bsq_index* h, const bsq_index_meta* m, bool may_compact = false) {
     CUDA_CHECK(cudaSetDevice(h->device));
     free_index_arrays(h);
     h->meta = *m;
     h->replica_pending = true;
     CUDA_CHECK(cudaMalloc(&h->d_pac, m->arr_bytes[BSQ_ARR_PAC] + 64));
     CUDA_CHECK(cudaMalloc(&h->d_occ, m->arr_bytes[BSQ_ARR_OCC] + 64));
-    CUDA_CHECK(cudaMalloc(&h->d_sa, m->arr_bytes[BSQ_ARR_SA] + 64));
+    cudaError_t e = may_compact && m->sa_interval == 1 && test_compact() ? cudaErrorMemoryAllocation : cudaMalloc(&h->d_sa, m->arr_bytes[BSQ_ARR_SA] + 64);
+    if (e == cudaErrorMemoryAllocation && may_compact && m->sa_interval == 1) {
+        cudaGetLastError(); h->d_sa = nullptr;
+        compact_meta(h->meta);
+        e = cudaMalloc(&h->d_sa, h->meta.arr_bytes[BSQ_ARR_SA] + 64);
+    }
+    CUDA_CHECK(e);
     CUDA_CHECK(cudaMalloc(&h->d_ann_offset, m->arr_bytes[BSQ_ARR_ANN_OFFSET] + 8));
     CUDA_CHECK(cudaMalloc(&h->d_ann_len, m->arr_bytes[BSQ_ARR_ANN_LEN] + 8));
     CUDA_CHECK(cudaMalloc(&h->d_ann_id, m->arr_bytes[BSQ_ARR_ANN_ID] + 8));
@@ -433,9 +446,36 @@ static int replica_finish(bsq_index* h, const void* host_state, uint64_t bytes) 
     return host_state ? host_state_decode(h, static_cast<const uint8_t*>(host_state), bytes) : BSQ_OK;
 }
 
-static __global__ void k_sa_sample(const void* sa, int sa_bytes, uint64_t n_sa, uint64_t* out) {
-    for (uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n_sa; k += (uint64_t)gridDim.x * blockDim.x)
-        out[k] = sa_bytes == 4 ? (uint64_t)static_cast<const uint32_t*>(sa)[k * 32] : static_cast<const uint64_t*>(sa)[k * 32];
+// out[k] = sa[k * stride] for k < n_sa, out_bytes wide: the samples of a full SA (stride 32) or of a compact one (stride 1)
+static __global__ void k_sa_sample(const void* sa, int sa_bytes, uint64_t stride, uint64_t n_sa, void* out, int out_bytes) {
+    for (uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n_sa; k += (uint64_t)gridDim.x * blockDim.x) {
+        const uint64_t v = sa_bytes == 4 ? (uint64_t)static_cast<const uint32_t*>(sa)[k * stride] : static_cast<const uint64_t*>(sa)[k * stride];
+        if (out_bytes == 4) static_cast<uint32_t*>(out)[k] = (uint32_t)v; else static_cast<uint64_t*>(out)[k] = v;
+    }
+}
+// SA[0], SA[32], SA[64], ... of the index, whatever its layout, into out (out_bytes per entry), on h->stream
+static void sa_samples_to(const bsq_index* h, void* out, int out_bytes) {
+    const uint64_t n_sa = (h->meta.seq_len + 32) / 32;
+    k_sa_sample<<<148 * 8, 256, 0, h->stream>>>(h->d_sa, (int)h->meta.sa_bytes, h->meta.sa_interval == 1 ? 32 : 1, n_sa, out, out_bytes);
+}
+
+// The compact layout (bsq_index_meta.sa_interval): the index keeps SA[0], SA[32], ... in an array of its SA width and frees the full SA
+// and the inverse SA -- 16 bytes per base at 64 bits become a quarter of a byte.  Positions are then resolved by LF walks
+// (sa_resolve.cu).  Taken only where the full layout cannot be allocated, and never undone.
+static int compact_index(bsq_index* h) {
+    bsq_index_meta m = h->meta;
+    if (m.sa_interval != 1) return BSQ_OK;
+    compact_meta(m);
+    void* d = nullptr;
+    CUDA_CHECK(cudaMalloc(&d, m.arr_bytes[BSQ_ARR_SA] + 64));
+    sa_samples_to(h, d, (int)m.sa_bytes);
+    const cudaError_t e = cudaStreamSynchronize(h->stream);
+    if (e != cudaSuccess) { cudaFree(d); bsq_set_error("compacting the index: %s", cudaGetErrorString(e)); return BSQ_ERR; }
+    cudaFree(h->d_sa); h->d_sa = d;   // cudaFree waits for every kernel already queued on the device, so none loses the SA under it
+    if (h->d_isa) { cudaFree(h->d_isa); h->d_isa = nullptr; }
+    h->meta = m;
+    h->timing.notes |= BSQ_NOTE_SA_COMPACTED;
+    return BSQ_OK;
 }
 
 extern "C" {
@@ -482,11 +522,11 @@ int bsq_index_sa_sampled(const bsq_index* h, uint64_t* out, uint64_t n_sa) {
     if (!h || !h->meta.built) { bsq_set_error("index not built"); return BSQ_ERR; }
     uint64_t n = h->meta.seq_len;
     if (n_sa != (n + 32) / 32) { bsq_set_error("n_sa must be (seq_len + 32) / 32"); return BSQ_ERR; }
-    // rows 0, 32, 64, ... of the full SA, gathered on the device (the full array is 50 GB at 3.1 Gbp)
+    // rows 0, 32, 64, ... of the SA, gathered on the device (the full array is 50 GB at 3.1 Gbp)
     CUDA_CHECK(cudaSetDevice(h->device));
     DevBuf<uint64_t> d;
     CUDA_CHECK(d.alloc(n_sa));
-    k_sa_sample<<<148 * 8, 256, 0, h->stream>>>(h->d_sa, (int)h->meta.sa_bytes, n_sa, d.p);
+    sa_samples_to(h, d.p, 8);
     CUDA_CHECK_AS("bsq_index_sa_sampled", cudaMemcpyAsync(out, d.p, n_sa * 8, cudaMemcpyDeviceToHost, h->stream));
     CUDA_CHECK_AS("bsq_index_sa_sampled", cudaStreamSynchronize(h->stream));
     out[0] = (uint64_t)-1;   // bwt_cal_sa: sa[0] = -1 (SURVEY A.3)
@@ -495,14 +535,14 @@ int bsq_index_sa_sampled(const bsq_index* h, uint64_t* out, uint64_t n_sa) {
 
 // Builds the arrays the seeding kernel derives from the index on this device (inverse SA, prefix table) now rather than inside
 // the first alignment call; *ms = wall time spent (0 when they were already there).  Every replica calls it after the broadcast.
+// When the inverse SA does not fit, the index compacts itself first (BSQ_NOTE_SA_COMPACTED in bsq_last_timing's notes).
 int bsq_index_prepare(bsq_index* h, float* ms) {
     BSQ_ENTRY();
     if (!h || !h->meta.built) { bsq_set_error("index not built"); return BSQ_ERR; }
     CUDA_CHECK(cudaSetDevice(h->device));
     Event e0, e1; cudaEventCreate(&e0.h); cudaEventCreate(&e1.h);
     cudaEventRecord(e0, h->stream);
-    const DevIndex ix = make_dev_index(h);
-    const int rc = ensure_kmer_table(h, ix);
+    const int rc = ensure_kmer_table(h);
     cudaEventRecord(e1, h->stream);
     cudaEventSynchronize(e1);
     if (ms) cudaEventElapsedTime(ms, e0, e1);
@@ -522,7 +562,7 @@ int bsq_index_save(bsq_index* h, const char* path, const uint8_t* key) {
     const uint64_t n_sa = (h->meta.seq_len + 32) / 32;
     DevBuf<uint64_t> d_samples;
     CUDA_CHECK(d_samples.alloc(n_sa));
-    k_sa_sample<<<148 * 8, 256, 0, h->stream>>>(h->d_sa, (int)h->meta.sa_bytes, n_sa, d_samples.p);   // sample 0 = SA[0] = seq_len
+    sa_samples_to(h, d_samples.p, 8);   // sample 0 = SA[0] = seq_len
     const IndexFileArrays a{h->d_pac, h->d_occ, h->d_sa, h->d_ann_offset, h->d_ann_len, h->d_ann_id};
     return index_file_save(path, h->meta, a, d_samples.p, h->pac.data(), h->ann_offset.data(), h->ann_len.data(), h->ann_id.data(), hs, key, h->stream);
 }
@@ -539,10 +579,10 @@ int bsq_index_load(bsq_index* h, const char* path, const uint8_t* key, float* ms
     memset(&info, 0, sizeof(info));
     std::vector<uint8_t> hs;
     int rc = index_file_open(r, path, key, &m);
-    if (rc == BSQ_OK) rc = alloc_replica(h, &m);
+    if (rc == BSQ_OK) rc = alloc_replica(h, &m, true);   // the compact layout when the full SA does not fit
     if (rc == BSQ_OK) {
         const IndexFileArrays a{h->d_pac, h->d_occ, h->d_sa, h->d_ann_offset, h->d_ann_len, h->d_ann_id};
-        rc = index_file_fill(r, a, hs, h->device, h->stream, &info);
+        rc = index_file_fill(r, a, h->meta.sa_interval != 1, hs, h->device, h->stream, &info);
     }
     info.file_bytes = r.file_bytes;
     index_file_close(r);
@@ -811,13 +851,22 @@ int upload_datums(bsq_index* h, Batch& b, const uint8_t* bytes, const uint64_t* 
     return upload_datums_end(h, b, n ? doff[0] : 0);
 }
 
-// k-mer table of the LAST-like seeding pass: built once per device index (also after a broadcast replica)
-int ensure_kmer_table(bsq_index* h, const DevIndex& ix) {
+// k-mer table of the LAST-like seeding pass: built once per device index (also after a broadcast replica).  The inverse SA beside it
+// is built only in the full layout; when it cannot be allocated, the index compacts itself and seeds without it.
+int ensure_kmer_table(bsq_index* h) {
+    DevIndex ix = make_dev_index(h);
     if (ix.seq_len >= (1ull << 40)) return BSQ_OK;   // the table packs rows in 40 bits
-    if (!h->d_isa) {
-        CUDA_CHECK(cudaMalloc(&h->d_isa, (ix.seq_len + 1) * (uint64_t)ix.sa_bytes + 64));
-        build_isa(ix, h->d_isa, h->stream, &h->timing.launches);
-        CUDA_CHECK(cudaStreamSynchronize(h->stream));
+    if (!h->d_isa && h->meta.sa_interval == 1) {
+        const cudaError_t e = test_compact() ? cudaErrorMemoryAllocation : cudaMalloc(&h->d_isa, (ix.seq_len + 1) * (uint64_t)ix.sa_bytes + 64);
+        if (e == cudaErrorMemoryAllocation) {
+            cudaGetLastError(); h->d_isa = nullptr;
+            if (compact_index(h) != BSQ_OK) return BSQ_ERR;
+            ix = make_dev_index(h);
+        } else {
+            CUDA_CHECK(e);
+            build_isa(ix, h->d_isa, h->stream, &h->timing.launches);
+            CUDA_CHECK(cudaStreamSynchronize(h->stream));
+        }
     }
     if (h->d_kmer || ix.seq_len < (1u << 16)) return BSQ_OK;
     h->kmer_k = kmer_table_depth(ix.seq_len);
@@ -879,6 +928,13 @@ int pipeline_enqueue(bsq_index* h, Batch& b) {
         rc = pipeline_enqueue_once(h, b);
         if (rc == BSQ_OK) bsq_set_error("");
     }
+    // the last rung: the full SA and the inverse SA give way to the compact layout (at 64 bits, 16 bytes per base)
+    if (rc != BSQ_OK && h->alloc_failed && h->meta.sa_interval == 1) {
+        if (compact_index(h) != BSQ_OK) return BSQ_ERR;
+        h->alloc_failed = false;
+        rc = pipeline_enqueue_once(h, b);
+        if (rc == BSQ_OK) bsq_set_error("");
+    }
     return rc;
 }
 static int pipeline_enqueue_once(bsq_index* h, Batch& b) {
@@ -887,10 +943,11 @@ static int pipeline_enqueue_once(bsq_index* h, Batch& b) {
     bsq_timing& T = h->timing;
     b.idle = true; b.out_rows = 0; b.out_cig = 0;
     if (n == 0 || !h->meta.built) { b.aligned = true; return BSQ_OK; }
+    if (ensure_kmer_table(h) != BSQ_OK) return BSQ_ERR;
     const DevIndex ix = make_dev_index(h);
     const DevOpts& o = h->dopts;
     cudaStream_t st = b.st;
-    if (ensure_kmer_table(h, ix) != BSQ_OK) return BSQ_ERR;
+    const bool compact = b.att_compact = h->meta.sa_interval != 1;
     const uint32_t max_len = std::max<uint32_t>(b.max_len, 1);
     const uint32_t rseq_cap = b.att_rseq_cap = std::max(rseq_cap_for(h, max_len), b.rseq_cap);
     if (b.intv_cap == 0) b.intv_cap = 48 + max_len / 4;
@@ -925,6 +982,7 @@ static int pipeline_enqueue_once(bsq_index* h, Batch& b) {
     ENS(b.narrow_z.ensure(narrow_zbuf_bytes())); ENS(b.narrow_jobs.ensure((size_t)b.pool_cap * 5 * 24)); ENS(b.wide_jobs.ensure(b.pool_cap));
     ENS(b.ctl.ensure(64)); ENS(b.chain_todo.ensure(n)); ENS(b.fin_todo.ensure(n)); ENS(b.seed_todo.ensure(n + 1));
     if (max_len <= 496) { ENS(b.seed_pk.ensure((size_t)n * seed_thread_words(max_len))); ENS(b.seed_u32.ensure(3 * (size_t)n)); }
+    if (compact) { ENS(b.sa_pos.ensure(b.pool_cap)); ENS(b.sa_pos_off.ensure((size_t)n + 1)); ENS(b.scan_tmp64.ensure(prim::scan_tmp_elems((size_t)n + 1) + 16)); }
     // the thread-per-extension pre-pass packs column scores in 16 bits: every value it stores is <= l_query * (a + 1)
     // Small batches take the warp-cooperative kernels for the DP stages: the thread-per-extension / thread-per-region kernels are built for
     // throughput (one thread runs a whole DP, ~0.5 ms of latency whatever the batch size), which is what a one-read call of
@@ -953,6 +1011,13 @@ static int pipeline_enqueue_once(bsq_index* h, Batch& b) {
         launch_seed(P, ix, o, st, nullptr); ++T.launches;
     }
     cudaEventRecord(ev[1], st);
+    if (compact) {   // the text positions of every SA lookup the chain kernels will make, by LF walks from the samples
+        SaResolveParams R;
+        R.intv = b.intv.p; R.intv_cnt = b.intv_cnt.p; R.intv_cap = b.intv_cap; R.n_reads = n; R.off = b.sa_pos_off.p; R.scan_tmp = b.scan_tmp64.p;
+        R.pos = b.sa_pos.p; R.pos_cap = b.pool_cap; R.ticket = b.ctl.p + 31; R.err = b.ctl.p + 51;
+        R.lf_steps = reinterpret_cast<unsigned long long*>(b.ctl.p + 28); R.iters = reinterpret_cast<unsigned long long*>(b.ctl.p + 54);
+        launch_sa_resolve_batch(R, ix, o, st, &T.launches);
+    }
     {
         ChainParams P;
         P.seqs = b.seqs.p; P.offs = b.offs.p; P.n_reads = n; P.intv = b.intv.p; P.intv_cnt = b.intv_cnt.p; P.intv_cap = b.intv_cap;
@@ -962,6 +1027,7 @@ static int pipeline_enqueue_once(bsq_index* h, Batch& b) {
         // short reads: a thread-per-read pass takes every read with a handful of seed occurrences, the warp kernel the rest
         const bool thread_chain = !P.logtab;
         P.todo = thread_chain ? b.chain_todo.p : nullptr; P.todo_cnt = b.ctl.p + 57;
+        P.sa_pos = compact ? b.sa_pos.p : nullptr; P.sa_pos_off = compact ? b.sa_pos_off.p : nullptr;
         if (thread_chain) { launch_chain_thread(P, ix, o, st); ++T.launches; }
         launch_chain(P, ix, o, st); ++T.launches;
     }
@@ -1014,6 +1080,7 @@ static int pipeline_enqueue_once(bsq_index* h, Batch& b) {
     ENS(cudaMemcpyAsync(b.ctl_host + 8, b.row_off.p + (n - 1), 4, cudaMemcpyDeviceToHost, st));
     ENS(cudaMemcpyAsync(b.ctl_host + 9, b.row_cnt.p + (n - 1), 4, cudaMemcpyDeviceToHost, st));
     ENS(cudaMemcpyAsync(b.ctl_host + 10, b.ctl.p + 30, 4, cudaMemcpyDeviceToHost, st));
+    if (compact) ENS(cudaMemcpyAsync(b.ctl_host + 11, b.ctl.p + 51, 4, cudaMemcpyDeviceToHost, st));
     b.idle = false;
     return BSQ_OK;
 #undef ENS
@@ -1029,6 +1096,10 @@ int pipeline_check(bsq_index* h, Batch& b, bool* again) {
     b.idle = true;
     { cudaError_t e_ = cudaGetLastError(); if (e_ != cudaSuccess) { bsq_set_error("kernel failure: %s", cudaGetErrorString(e_)); return BSQ_ERR; } }
     const uint32_t* ctl = b.ctl_host;
+    if (b.att_compact && ctl[11]) {
+        bsq_set_error("compact index: %s (the index is damaged)", ctl[11] == 1 ? "an SA lookup names a row outside [0, seq_len]" : "an LF walk is longer than seq_len");
+        return BSQ_ERR;
+    }
     cudaEvent_t* ev = b.ev;
     float ms;
     cudaEventElapsedTime(&ms, ev[0], ev[1]); T.seed += ms;
@@ -1794,7 +1865,8 @@ int bsq_index_verify(bsq_index* h, uint64_t n_samples, uint64_t seed, bsq_index_
     CUDA_CHECK(d.alloc(IV_WORDS));
     Event e0, e1; cudaEventCreate(&e0.h); cudaEventCreate(&e1.h);
     cudaEventRecord(e0, h->stream);
-    launch_index_verify(ix, n_samples, seed, 65536, d.p, h->stream);
+    const uint32_t iv = h->meta.sa_interval;
+    launch_index_verify(ix, iv, n_samples, seed, 65536, d.p, h->stream);
     cudaEventRecord(e1, h->stream);
     CUDA_CHECK_AS("bsq_index_verify", cudaMemcpyAsync(v, d.p, sizeof(v), cudaMemcpyDeviceToHost, h->stream));
     CUDA_CHECK_AS("bsq_index_verify", cudaStreamSynchronize(h->stream));
@@ -1805,8 +1877,8 @@ int bsq_index_verify(bsq_index* h, uint64_t n_samples, uint64_t seed, bsq_index_
     // sum and sum of squares of 0..n, exact in 128 bits (n < 2^41), compared mod 2^64
     const uint64_t want_sum = (uint64_t)(N * (N + 1) / 2), want_sq = (uint64_t)(N * (N + 1) * (2 * N + 1) / 6);
     out->rows = n + 1;
-    out->exhaustive = n_samples >= n + 1;
-    out->sa_permutation_ok = v[IV_SA_SUM] == want_sum && v[IV_SA_SUMSQ] == want_sq && v[IV_SA_RANGE_BAD] == 0;
+    out->exhaustive = iv == 1 && n_samples >= n + 1;
+    out->sa_permutation_ok = iv == 1 && v[IV_SA_SUM] == want_sum && v[IV_SA_SUMSQ] == want_sq && v[IV_SA_RANGE_BAD] == 0;
     out->sa_out_of_range = v[IV_SA_RANGE_BAD];
     out->order_checked = v[IV_ORDER_CHECKED]; out->order_bad = v[IV_ORDER_BAD]; out->order_undecided = v[IV_ORDER_UNDECIDED];
     out->rows_checked = v[IV_ROWS_CHECKED]; out->bwt_bad = v[IV_BWT_BAD]; out->lf_bad = v[IV_LF_BAD];
@@ -1827,6 +1899,39 @@ int bsq_debug_ctl(bsq_index* h, uint32_t* out64) {
     return BSQ_OK;
 }
 
+}  // extern "C"
+static __global__ void k_sa_gather(DevIndex ix, uint64_t* rows, uint64_t n) {
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) rows[i] = sa_at(ix, rows[i]);
+}
+extern "C" {
+
+// bwt_sa of explicit rows: on a compact index through the resolve kernel of the alignment pipeline, so that a test can check it on
+// every row against a suffix array computed elsewhere
+int bsq_debug_sa_lookup(bsq_index* h, const uint64_t* rows, uint64_t n, uint64_t* out) {
+    BSQ_ENTRY();
+    if (!h || !h->meta.built) { bsq_set_error("index not built"); return BSQ_ERR; }
+    if (n && (!rows || !out)) { bsq_set_error("null argument"); return BSQ_ERR; }
+    if (n >= (1ull << 31)) { bsq_set_error("bsq_debug_sa_lookup: %llu rows, fewer than 2^31 per call", (unsigned long long)n); return BSQ_ERR; }
+    for (uint64_t i = 0; i < n; ++i)
+        if (rows[i] > h->meta.seq_len) { bsq_set_error("bsq_debug_sa_lookup: row %llu outside [0, %llu]", (unsigned long long)rows[i], (unsigned long long)h->meta.seq_len); return BSQ_ERR; }
+    if (n == 0) return BSQ_OK;
+    CUDA_CHECK(cudaSetDevice(h->device));
+    const DevIndex ix = make_dev_index(h);
+    DevBuf<uint64_t> pos; DevBuf<uint32_t> w;
+    CUDA_CHECK(pos.alloc(n + 1)); CUDA_CHECK(w.alloc(2));
+    CUDA_CHECK(cudaMemcpyAsync(pos.p, rows, n * 8, cudaMemcpyHostToDevice, h->stream));
+    CUDA_CHECK(cudaMemcpyAsync(pos.p + n, &n, 8, cudaMemcpyHostToDevice, h->stream));
+    CUDA_CHECK(cudaMemsetAsync(w.p, 0, 8, h->stream));
+    if (h->meta.sa_interval == 1) k_sa_gather<<<(unsigned)std::min<uint64_t>((n + 255) / 256, 148 * 8), 256, 0, h->stream>>>(ix, pos.p, n);
+    else launch_sa_resolve(ix, pos.p, pos.p + n, n, w.p, w.p + 1, nullptr, nullptr, h->stream);
+    uint32_t err = 0;
+    CUDA_CHECK_AS("bsq_debug_sa_lookup", cudaMemcpyAsync(out, pos.p, n * 8, cudaMemcpyDeviceToHost, h->stream));
+    CUDA_CHECK_AS("bsq_debug_sa_lookup", cudaMemcpyAsync(&err, w.p + 1, 4, cudaMemcpyDeviceToHost, h->stream));
+    CUDA_CHECK_AS("bsq_debug_sa_lookup", cudaStreamSynchronize(h->stream));
+    if (err) { bsq_set_error("bsq_debug_sa_lookup: an LF walk is longer than seq_len (the index is damaged)"); return BSQ_ERR; }
+    return BSQ_OK;
+}
+
 int bsq_debug_seed(bsq_index* h, const char* seqs, const uint64_t* offs, uint64_t n, uint64_t* out, uint32_t cap, uint32_t* cnt) {
     BSQ_ENTRY();
     if (!h || !h->meta.built) { bsq_set_error("index not built"); return BSQ_ERR; }
@@ -1834,8 +1939,8 @@ int bsq_debug_seed(bsq_index* h, const char* seqs, const uint64_t* offs, uint64_
     std::vector<int64_t> ids(n, 0);
     if (upload_reads(h, h->batch, seqs, offs, ids.data(), n) != BSQ_OK) return BSQ_ERR;
     Batch& b = h->batch;
+    if (ensure_kmer_table(h) != BSQ_OK) return BSQ_ERR;
     const DevIndex ix = make_dev_index(h);
-    if (ensure_kmer_table(h, ix) != BSQ_OK) return BSQ_ERR;
     b.intv_cap = cap;
     b.list_cap = std::max<uint32_t>(b.max_len + 1, cap);
     const int seed_warps = seed_resident_warps();
@@ -2116,6 +2221,7 @@ static int multi_align(bsq_multi* m, const ReadSrc& S, uint64_t n, bsq_result** 
         MT.seed = std::max(MT.seed, h->timing.seed); MT.chain = std::max(MT.chain, h->timing.chain); MT.extend = std::max(MT.extend, h->timing.extend);
         MT.finalize = std::max(MT.finalize, h->timing.finalize);
         MT.launches += h->timing.launches; MT.h2d_bytes += h->timing.h2d_bytes; MT.d2h_bytes += h->timing.d2h_bytes;
+        MT.notes |= h->timing.notes;   // what any device had to do differently (a table downgrade, a compaction)
     }
     cudaSetDevice(h0->device);
     if (rc != BSQ_OK) { result_delete(R); return BSQ_ERR; }

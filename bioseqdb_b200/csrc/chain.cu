@@ -1,11 +1,13 @@
 // chain.cu -- kernel `chain_build`: SA lookup of every seed occurrence, seed chaining and chain filtering
 // (SURVEY.md A.5, A.6; replaces libbwa mem_chain / test_and_merge / mem_chain_weight / mem_chain_flt
 // reached from reference bioseqdb/bwa.cpp:149).  One warp per read.  The SA lookups (the only HBM
-// random reads here: one 4- or 8-byte load per occurrence because the full SA is resident) are issued by
+// random reads here: one 4- or 8-byte load per occurrence when the full SA is resident; on a compact index
+// the resolve pass of sa_resolve.cu has put every position in ChainParams::sa_pos) are issued by
 // all lanes in parallel; the ordered-insert chaining itself is sequential bookkeeping on a few records.
 #include "pipeline.cuh"
 #include "ksort_dev.cuh"
 #include "launch_cache.cuh"
+#include "sa_lookup.cuh"
 
 namespace {
 
@@ -123,18 +125,6 @@ __device__ int mem_seed_sw(const DevIndex& ix, const DevOpts& o, const int* smat
     __syncwarp();
     cells += (unsigned long long)qlen * (unsigned long long)tlen;
     return ksw_local_warp(o, smat, qlen, query + qb, tlen, tw, bH, bF);
-}
-
-// occurrences an interval contributes (the k/step loop of mem_chain, SURVEY A.5) and the stride between them
-__device__ __forceinline__ uint32_t occ_count(const DevOpts& o, uint64_t x2, uint64_t* step_out) {
-    uint64_t step = 1, cnt = x2;
-    if (x2 > (uint64_t)o.max_occ) {
-        step = x2 / (uint64_t)o.max_occ;
-        cnt = (x2 + step - 1) / step;
-        if (cnt > (uint64_t)o.max_occ) cnt = (uint64_t)o.max_occ;
-    }
-    if (step_out) *step_out = step;
-    return (uint32_t)cnt;
 }
 
 // ordered-insert chaining of a read's `total` seeds (raw[t].score holds the seed's rid on entry, its length on exit): returns the
@@ -268,25 +258,21 @@ __global__ void __launch_bounds__(CHAIN_THREADS) chain_build_thread(ChainParams 
     if (fast) {
         const uint32_t base = wbase + incl - need;
         ReadBlock blk; blk.base = base; blk.n_alloc = total; blk.n_chains = 0; blk.n_seeds = 0;
-        if (total == 0 || (uint64_t)base + total > (uint64_t)P.pool_cap) {
+        // a compact index whose batch has more lookups than position slots resolved none of them: no read chains on that attempt
+        if (total == 0 || (uint64_t)base + total > (uint64_t)P.pool_cap || (P.sa_pos && P.sa_pos_off[P.n_reads] > (uint64_t)P.pool_cap)) {
             if (total) atomicExch(P.overflow, 1u);
             blk.n_alloc = 0;
             P.blocks[r] = blk;
         } else {
             SeedRec* raw = P.raw + base; ChainTmp* ct = P.ctmp + base; uint32_t* ord = P.ord + base;
-            uint32_t t = 0;
-            for (int i = 0; i < n_iv; ++i) {
-                const Intv p = iv[i];
-                uint64_t step;
-                const uint32_t cnt = occ_count(o, p.x2, &step);
+            const uint64_t* pos = P.sa_pos ? P.sa_pos + P.sa_pos_off[r] : nullptr;
+            for_each_lookup(iv, n_iv, o, 0u, 1u, [&](uint32_t t, const Intv& p, uint64_t row) {
                 const int qb = (int)(p.info >> 32), ql = (int)((uint32_t)p.info - (uint32_t)(p.info >> 32));
-                for (uint32_t c = 0; c < cnt; ++c, ++t) {
-                    const int64_t rbeg = (int64_t)sa_at(ix, p.x0 + (uint64_t)c * step);
-                    SeedRec sd; sd.rbeg = rbeg; sd.qbeg = qb; sd.len = ql; sd.next = -1;
-                    sd.score = bns_intv2rid(ix, rbeg, rbeg + ql);
-                    raw[t] = sd;
-                }
-            }
+                const int64_t rbeg = (int64_t)(pos ? pos[t] : sa_at(ix, row));
+                SeedRec sd; sd.rbeg = rbeg; sd.qbeg = qb; sd.len = ql; sd.next = -1;
+                sd.score = bns_intv2rid(ix, rbeg, rbeg + ql);
+                raw[t] = sd;
+            });
             n_sa += total;
             const int n_ch = chain_seeds(raw, ct, ord, total, ix, o, n_dup);
             for (int k = 0; k < n_ch; ++k) ct[k].w = (uint32_t)chain_weight(raw, ct[k]);
@@ -341,13 +327,7 @@ __global__ void __launch_bounds__(CHAIN_THREADS) chain_build(ChainParams P, DevI
             int b = 0, e = 0;
             for (int i = 0; i < n_iv; ++i) {   // uniform across lanes (broadcast loads)
                 uint64_t x2 = iv[i].x2;
-                uint64_t cnt = x2;                       // step == 1 unless the interval is larger than max_occ
-                if (x2 > (uint64_t)o.max_occ) {
-                    const uint64_t step = x2 / (uint64_t)o.max_occ;
-                    cnt = (x2 + step - 1) / step;
-                    if (cnt > (uint64_t)o.max_occ) cnt = (uint64_t)o.max_occ;
-                }
-                total += (uint32_t)cnt;
+                total += occ_count(o, x2, nullptr);
                 if (x2 > (uint64_t)o.max_occ) {
                     int sb = (int)(iv[i].info >> 32), se = (int)(uint32_t)iv[i].info;
                     if (sb > e) { l_rep += e - b; b = sb; e = se; }
@@ -360,7 +340,7 @@ __global__ void __launch_bounds__(CHAIN_THREADS) chain_build(ChainParams P, DevI
         if (lane == 0 && total) base = atomicAdd(P.pool_top, total);
         base = __shfl_sync(FULL, base, 0);
         ReadBlock blk; blk.base = base; blk.n_alloc = total; blk.n_chains = 0; blk.n_seeds = 0;
-        if (total == 0 || (uint64_t)base + total > (uint64_t)P.pool_cap) {
+        if (total == 0 || (uint64_t)base + total > (uint64_t)P.pool_cap || (P.sa_pos && P.sa_pos_off[P.n_reads] > (uint64_t)P.pool_cap)) {
             if (total && lane == 0) atomicExch(P.overflow, 1u);
             blk.n_alloc = 0;
             if (lane == 0) P.blocks[r] = blk;
@@ -378,13 +358,7 @@ __global__ void __launch_bounds__(CHAIN_THREADS) chain_build(ChainParams P, DevI
                 if (i < n_iv) {
                     const Intv p = iv[i];
                     x0 = p.x0; info_lo = (uint32_t)p.info; info_hi = (uint32_t)(p.info >> 32);
-                    uint64_t c64 = p.x2;
-                    if (p.x2 > (uint64_t)o.max_occ) {
-                        step = p.x2 / (uint64_t)o.max_occ;
-                        c64 = (p.x2 + step - 1) / step;
-                        if (c64 > (uint64_t)o.max_occ) c64 = (uint64_t)o.max_occ;
-                    }
-                    cnt = (uint32_t)c64;
+                    cnt = occ_count(o, p.x2, &step);
                 }
                 uint32_t incl = cnt;
 #pragma unroll
@@ -401,7 +375,8 @@ __global__ void __launch_bounds__(CHAIN_THREADS) chain_build(ChainParams P, DevI
                     const uint32_t o_lo = __shfl_sync(FULL, info_lo, own), o_hi = __shfl_sync(FULL, info_hi, own);
                     if (t < chunk_total) {
                         const uint32_t c = t - (o_incl - o_cnt);
-                        const int64_t rbeg = (int64_t)sa_at(ix, o_x0 + (uint64_t)c * o_step);
+                        const uint64_t row = lookup_row(o_x0, o_step, c);
+                        const int64_t rbeg = (int64_t)(P.sa_pos ? P.sa_pos[P.sa_pos_off[r] + t0 + t] : sa_at(ix, row));
                         SeedRec sd; sd.rbeg = rbeg; sd.qbeg = (int)o_hi; sd.len = (int)(o_lo - o_hi); sd.next = -1;
                         sd.score = bns_intv2rid(ix, rbeg, rbeg + sd.len);   // rid parked in `score` until chaining
                         raw[t0 + t] = sd;

@@ -7,6 +7,7 @@
 //                        Chains are the gaps between sampled suffixes in text order (32 on average, with a long tail); lanes are
 //                        persistent and take the next sample as soon as their chain ends, from a pool of 32 samples per warp refilled
 //                        with one atomic ticket.  Every step reads one 64-byte Occ block at a random row and scatters one SA entry.
+//   k_sa_keep_samples    a compact load (the full suffix array does not fit): the samples stay as they are, range-checked.
 // A file that got past its checksums can still be wrong: a row outside [0, n], a sample above n or a chain longer than n stops the walk
 // and is reported, and no index the kernel computes is used before it has been range-checked.
 #include <cerrno>
@@ -19,6 +20,7 @@
 #include <unistd.h>
 #include "index_file.cuh"
 #include "common.cuh"
+#include "sa_lookup.cuh"
 
 const char* const kSectionName[SEC_COUNT] = {"pac", "occ", "sa_samples", "ann_offset", "ann_len", "ann_id", "host_state"};
 
@@ -58,40 +60,10 @@ struct SaRebuild {
     unsigned int* ticket;
     unsigned long long* stats;               // [0] error code, [1] where, [2] rows written, [3] LF steps, [4] warp iterations
 };
-enum { SA_ERR_SAMPLE = 1, SA_ERR_ROW = 2, SA_ERR_CHAIN = 3 };
+enum { SA_ERR_SAMPLE = 1, SA_ERR_ROW = 2, SA_ERR_CHAIN = 3, SA_ERR_SAMPLE0 = 4 };
 
 __device__ __forceinline__ void sa_fail(const SaRebuild& P, unsigned long long code, unsigned long long where) {
     if (atomicCAS(P.stats, 0ull, code) == 0ull) atomicExch(P.stats + 1, where);
-}
-
-// bwt_invPsi (libbwa bwt.h) for a row j in [0, n]: 0 for the primary row, else L2[c] + occ(j, c) with c = B0[j - (j > primary)] and occ
-// the count of c in B0[0 .. j - (j >= primary)] -- the checkpoint of j's 128-symbol block plus the popcounts of its symbols up to j.
-__device__ __forceinline__ uint64_t lf(const SaRebuild& P, uint64_t j) {
-    if (j == P.primary) return 0;
-    const uint64_t x = j - (j > P.primary);
-    const uint4* blk = reinterpret_cast<const uint4*>(P.occ + ((size_t)(x >> 7) << 4));
-    const uint4 ca = __ldg(blk), cb = __ldg(blk + 1), s0 = __ldg(blk + 2), s1 = __ldg(blk + 3);
-    const uint32_t w8[8] = {s0.x, s0.y, s0.z, s0.w, s1.x, s1.y, s1.z, s1.w};
-    const int wi = (int)((x >> 4) & 7);
-    uint32_t word = 0;
-#pragma unroll
-    for (int w = 0; w < 8; ++w) word = w == wi ? w8[w] : word;
-    const uint32_t c = (word >> ((15 - (uint32_t)(x & 15)) << 1)) & 3u;
-    const uint32_t rep = c * 0x55555555u;
-    const int within = (int)(x & 127) + 1;
-    uint32_t cnt = 0;
-#pragma unroll
-    for (int w = 0; w < 8; ++w) {
-        int nsym = within - (w << 4);
-        nsym = nsym < 0 ? 0 : (nsym > 16 ? 16 : nsym);
-        const uint32_t keep = __funnelshift_rc(0u, 0x55555555u, 2 * nsym);   // the first nsym symbols of the word (MSB first)
-        const uint32_t t = ~(w8[w] ^ rep);                                     // 11 where a symbol equals c
-        cnt += __popc(t & (t >> 1) & keep);
-    }
-    const uint64_t ck = c == 0 ? ((uint64_t)ca.y << 32 | ca.x) : c == 1 ? ((uint64_t)ca.w << 32 | ca.z)
-                      : c == 2 ? ((uint64_t)cb.y << 32 | cb.x) : ((uint64_t)cb.w << 32 | cb.z);
-    const uint64_t base = c == 0 ? P.L0 : c == 1 ? P.L1 : c == 2 ? P.L2 : P.L3;
-    return base + ck + cnt;
 }
 
 template <class SaT>
@@ -138,6 +110,18 @@ __global__ void __launch_bounds__(SA_THREADS) k_sa_from_samples(SaRebuild P, SaT
 #pragma unroll
     for (int o = 16; o; o >>= 1) { written += __shfl_xor_sync(FULL, written, o); steps += __shfl_xor_sync(FULL, steps, o); }
     if (lane == 0) { atomicAdd(P.stats + 2, (unsigned long long)written); atomicAdd(P.stats + 3, (unsigned long long)steps); atomicAdd(P.stats + 4, (unsigned long long)iters); }
+}
+
+// A compact load keeps the samples as they are (narrowed to the index's SA width): nothing downstream checks them again, so every one
+// must be <= n and sample 0 must be n (the row of the empty suffix).
+template <class SaT>
+__global__ void k_sa_keep_samples(SaRebuild P, SaT* __restrict__ out) {
+    for (uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; k < P.n_samples; k += (uint64_t)gridDim.x * blockDim.x) {
+        const uint64_t v = __ldg(P.samples + k);
+        if (v > P.n) sa_fail(P, SA_ERR_SAMPLE, k);
+        else if (k == 0 && v != P.n) sa_fail(P, SA_ERR_SAMPLE0, 0);
+        out[k] = (SaT)v;
+    }
 }
 
 // two pinned buffers: the file read of one chunk overlaps the copy of the other
@@ -340,7 +324,7 @@ int index_file_open(IndexFileReader& r, const char* path, const uint8_t* key, bs
     if (key && memcmp(key, h.key, 16) != 0) { bsq_set_error("bsq_index_load: %s: key mismatch (the file holds the index of other content)", path); return BSQ_ERR; }
     memset(m, 0, sizeof(*m));
     m->l_pac = h.l_pac; m->seq_len = n; m->primary = h.primary; memcpy(m->L2, h.L2, sizeof(m->L2)); m->n_anns = h.n_anns; m->sa_bytes = h.sa_bytes;
-    m->built = 1;
+    m->built = 1; m->sa_interval = 1;
     m->arr_bytes[BSQ_ARR_PAC] = want[SEC_PAC]; m->arr_bytes[BSQ_ARR_OCC] = want[SEC_OCC]; m->arr_bytes[BSQ_ARR_SA] = (n + 1) * h.sa_bytes;
     m->arr_bytes[BSQ_ARR_ANN_OFFSET] = want[SEC_ANN_OFFSET]; m->arr_bytes[BSQ_ARR_ANN_LEN] = want[SEC_ANN_LEN]; m->arr_bytes[BSQ_ARR_ANN_ID] = want[SEC_ANN_ID];
     m->build_ms = h.build_ms; m->build_launches = h.build_launches; m->sort_pass_bytes = h.sort_pass_bytes;
@@ -349,7 +333,7 @@ int index_file_open(IndexFileReader& r, const char* path, const uint8_t* key, bs
 
 void index_file_close(IndexFileReader& r) { if (r.fd >= 0) close(r.fd); r.fd = -1; }
 
-int index_file_fill(IndexFileReader& r, const IndexFileArrays& d, std::vector<uint8_t>& host_state, int device, cudaStream_t st,
+int index_file_fill(IndexFileReader& r, const IndexFileArrays& d, bool compact, std::vector<uint8_t>& host_state, int device, cudaStream_t st,
                     bsq_index_load_info* info) {
     typedef unsigned long long ull;
     const IndexFileHeader& h = r.hdr;
@@ -397,6 +381,23 @@ int index_file_fill(IndexFileReader& r, const IndexFileArrays& d, std::vector<ui
     P.occ = d.occ; P.samples = d_samples; P.n = n; P.primary = h.primary; P.L0 = h.L2[0]; P.L1 = h.L2[1]; P.L2 = h.L2[2]; P.L3 = h.L2[3];
     P.n_samples = (uint32_t)n_samples; P.ticket = reinterpret_cast<unsigned int*>(d_stats + 5); P.stats = d_stats;
     CUDA_CHECK(cudaMemsetAsync(d_stats, 0, 8 * 8, st));
+    if (compact) {   // the samples are the index: checked and narrowed, no walk
+        const unsigned grid = (unsigned)((n_samples + SA_THREADS - 1) / SA_THREADS < 148 * 8 ? (n_samples + SA_THREADS - 1) / SA_THREADS : 148 * 8);
+        CUDA_CHECK(cudaEventRecord(ev[2], st));
+        if (h.sa_bytes == 4) k_sa_keep_samples<uint32_t><<<grid, SA_THREADS, 0, st>>>(P, static_cast<uint32_t*>(d.sa));
+        else k_sa_keep_samples<uint64_t><<<grid, SA_THREADS, 0, st>>>(P, static_cast<uint64_t*>(d.sa));
+        CUDA_CHECK(cudaGetLastError());
+        CUDA_CHECK(cudaEventRecord(ev[3], st));
+        ull stats[2];
+        CUDA_CHECK(cudaMemcpyAsync(stats, d_stats, sizeof(stats), cudaMemcpyDeviceToHost, st));
+        CUDA_CHECK(cudaStreamSynchronize(st));
+        CUDA_CHECK(cudaEventElapsedTime(&info->sa_ms, ev[2], ev[3]));
+        switch (stats[0]) {
+            case 0: return BSQ_OK;
+            case SA_ERR_SAMPLE: bsq_set_error("bsq_index_load: SA sample %llu is larger than seq_len %llu", stats[1], (ull)n); return BSQ_ERR;
+            default: bsq_set_error("bsq_index_load: SA sample 0 is not seq_len %llu (the row of the empty suffix)", (ull)n); return BSQ_ERR;
+        }
+    }
     int sms = 0, per_sm = 0;
     CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
     if (h.sa_bytes == 4) CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sa_from_samples<uint32_t>, SA_THREADS, 0));

@@ -7,7 +7,8 @@
 //   ann_offset, ann_len, ann_id
 //   host_state   the blob of bsq_index_host_state_get (ambiguity holes and their rows)
 // The full suffix array (49.6 of 53.5 GB at 3.1 Gbp) is not stored: the load rebuilds it on the device from the samples by LF walks
-// (k_sa_from_samples).  Neither are the per-device derived arrays (inverse SA, prefix table): bsq_index_prepare builds them.
+// (k_sa_from_samples), or keeps only the samples when it does not fit (the compact layout, bsq_index_meta.sa_interval = 32; saving such
+// an index writes the same file).  Neither are the per-device derived arrays (inverse SA, prefix table): bsq_index_prepare builds them.
 #pragma once
 #include <cstdint>
 #include <string>
@@ -63,7 +64,8 @@ int index_file_save(const char* path, const bsq_index_meta& m, const IndexFileAr
 // Load, step 1: open the file, check the header against itself, the file size and `key`; *m = the meta of the index it holds.
 struct IndexFileReader { int fd = -1; uint64_t file_bytes = 0; IndexFileHeader hdr; std::string path; };
 int index_file_open(IndexFileReader& r, const char* path, const uint8_t* key, bsq_index_meta* m);
-// Load, step 2 (arrays allocated for *m): sections uploaded, checksummed on the device, full SA rebuilt; host_state = the blob.
-int index_file_fill(IndexFileReader& r, const IndexFileArrays& d, std::vector<uint8_t>& host_state, int device, cudaStream_t st,
+// Load, step 2 (arrays allocated for *m): sections uploaded, checksummed on the device, full SA rebuilt -- or, compact, d.sa = the
+// samples, checked and as wide as the index's SA entries; host_state = the blob.
+int index_file_fill(IndexFileReader& r, const IndexFileArrays& d, bool compact, std::vector<uint8_t>& host_state, int device, cudaStream_t st,
                     bsq_index_load_info* info);
 void index_file_close(IndexFileReader& r);

@@ -10,6 +10,8 @@
 //                                              blocks; first record zero; trailing record == L2 differences;
 //   * L2                                    -- L2[c+1] - L2[c] == occurrences of c in T, counted from pac (all bases).
 // "Sampled" means every row / block when n_samples covers them (small indexes, tests), else rows drawn by splitmix64.
+// A compact index (SA interval 32) holds SA[32 k] only: the sums, range and LF checks cover nothing it does not hold, order compares
+// consecutive samples, the BWT check runs on the sampled rows; Occ and L2 are checked as for a full index.
 #include <cstdint>
 #include <cuda_runtime.h>
 #include "common.cuh"
@@ -46,8 +48,7 @@ __device__ uint64_t occ_upto(const DevIndex& ix, uint64_t x, uint32_t c) {
 }
 
 // out: see IV_* in index_verify.cuh
-__global__ void k_verify_sa_sums(DevIndex ix, unsigned long long* out) {
-    const uint64_t rows = ix.seq_len + 1;
+__global__ void k_verify_sa_sums(DevIndex ix, uint64_t rows, unsigned long long* out) {
     unsigned long long s = 0, q = 0;
     for (uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; k < rows; k += (uint64_t)gridDim.x * blockDim.x) {
         const unsigned long long v = sa_at(ix, k);
@@ -70,14 +71,15 @@ __global__ void k_verify_text_counts(DevIndex ix, unsigned long long* out) {
     }
 }
 
-__global__ void k_verify_rows(DevIndex ix, uint64_t m, uint64_t seed, uint64_t max_lcp, unsigned long long* out) {
-    const uint64_t n = ix.seq_len;
+// entries k of ix.sa stand for rows k * iv; nk = entries held
+__global__ void k_verify_rows(DevIndex ix, uint32_t iv, uint64_t m, uint64_t seed, uint64_t max_lcp, unsigned long long* out) {
+    const uint64_t n = ix.seq_len, nk = (n + iv) / iv;
     unsigned long long ord_bad = 0, ord_und = 0, bwt_bad = 0, lf_bad = 0, n_ord = 0, n_row = 0;
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < m; i += (uint64_t)gridDim.x * blockDim.x) {
-        // ---- order: rows k, k + 1 (k in [0, n))
+        // ---- order: entries k, k + 1 (k in [0, nk - 1))
         {
-            const uint64_t k = sample_of(i, m, n, seed);
-            if (k < n) {
+            const uint64_t k = sample_of(i, m, nk - 1, seed);
+            if (k < nk - 1) {
                 const uint64_t a = sa_at(ix, k), b = sa_at(ix, k + 1);
                 ++n_ord;
                 if (a > n || b > n || a == b) ++ord_bad;
@@ -93,18 +95,20 @@ __global__ void k_verify_rows(DevIndex ix, uint64_t m, uint64_t seed, uint64_t m
                 }
             }
         }
-        // ---- BWT symbol and LF of row k (k in [0, n])
+        // ---- BWT symbol and LF of row k (entry e in [0, nk))
         {
-            const uint64_t k = sample_of(i, m, n + 1, seed ^ 0x5bd1e995u);
-            if (k <= n) {
+            const uint64_t e = sample_of(i, m, nk, seed ^ 0x5bd1e995u);
+            if (e < nk) {
+                const uint64_t k = e * iv;
                 ++n_row;
-                const uint64_t s = sa_at(ix, k);
-                if (k == ix.primary) { if (s != 0) { ++bwt_bad; ++lf_bad; } }
-                else if (s == 0 || s > n) { ++bwt_bad; ++lf_bad; }
+                const uint64_t s = sa_at(ix, e);
+                if (k == ix.primary) { if (s != 0) { ++bwt_bad; lf_bad += iv == 1; } }
+                else if (s == 0 || s > n) { ++bwt_bad; lf_bad += iv == 1; }
                 else {
                     const uint64_t x = k - (k > ix.primary);
                     const uint32_t c = b0_at(ix, x);
                     if (c != text_at(ix, s - 1)) ++bwt_bad;
+                    if (iv != 1) continue;
                     // bwt_invPsi: L2[c] + occ(k, c), occ counting B0[0 .. k - (k >= primary)]
                     const uint64_t r = ix.L2[c] + occ_upto(ix, k - (k >= ix.primary), c);
                     if (r > n || sa_at(ix, r) + 1 != s) ++lf_bad;
@@ -145,13 +149,13 @@ __global__ void k_verify_blocks(DevIndex ix, uint64_t m, uint64_t seed, unsigned
 
 }  // namespace
 
-void launch_index_verify(const DevIndex& ix, uint64_t n_samples, uint64_t seed, uint64_t max_lcp, unsigned long long* d_out, cudaStream_t st) {
+void launch_index_verify(const DevIndex& ix, uint32_t iv, uint64_t n_samples, uint64_t seed, uint64_t max_lcp, unsigned long long* d_out, cudaStream_t st) {
     cudaMemsetAsync(d_out, 0, IV_WORDS * 8, st);
     const unsigned grid = 148 * 8;
-    k_verify_sa_sums<<<grid, 256, 0, st>>>(ix, d_out);
+    const uint64_t rows = (ix.seq_len + iv) / iv, blocks = (ix.seq_len + 127) >> 7;
+    k_verify_sa_sums<<<grid, 256, 0, st>>>(ix, rows, d_out);
     k_verify_text_counts<<<grid, 256, 0, st>>>(ix, d_out);
-    const uint64_t rows = ix.seq_len + 1, blocks = (ix.seq_len + 127) >> 7;
     const uint64_t m_rows = n_samples >= rows ? rows : n_samples, m_blk = n_samples >= blocks ? blocks : n_samples;
-    k_verify_rows<<<grid, 256, 0, st>>>(ix, m_rows, seed, max_lcp, d_out);
+    k_verify_rows<<<grid, 256, 0, st>>>(ix, iv, m_rows, seed, max_lcp, d_out);
     k_verify_blocks<<<grid, 256, 0, st>>>(ix, m_blk, seed, d_out);
 }

@@ -30,9 +30,27 @@ struct ChainParams {
     const double* logtab;          // host-libm log(l) for l <= longest read; nullptr when no read is long enough for mem_flt_chained_seeds
     unsigned long long* sw_cells;  // optional: cells of the seed-filter local SW
     uint32_t* todo; uint32_t* todo_cnt;   // reads the thread-per-read pass left for the warp kernel (nullptr = the warp kernel takes every read)
+    // compact index: lookup t of read r (sa_lookup.cuh) has its text position at sa_pos[sa_pos_off[r] + t], pool_cap slots
+    // (sa_resolve.cu); sa_pos_off[n_reads] > pool_cap = the pass resolved nothing and every read overflows; nullptr = the full SA is
+    // resident and is read directly
+    const uint64_t* sa_pos; const uint64_t* sa_pos_off;
 };
 void launch_chain_thread(const ChainParams& p, const DevIndex& ix, const DevOpts& o, cudaStream_t st);
 void launch_chain(const ChainParams& p, const DevIndex& ix, const DevOpts& o, cudaStream_t st);
+
+// Position resolve pass of a compact index (sa_resolve.cu), between seeding and chaining
+struct SaResolveParams {
+    const Intv* intv; const uint32_t* intv_cnt; uint32_t intv_cap; uint32_t n_reads;
+    uint64_t* off;                 // n_reads + 1: lookups before read r; off[n_reads] = the batch's total
+    uint64_t* scan_tmp;            // prim::scan_tmp_elems(n_reads + 1)
+    uint64_t* pos; uint64_t pos_cap;   // one slot per lookup; a batch with more lookups than slots overflows the chain pool as well
+    uint32_t* ticket; uint32_t* err;   // err: 1 = a row outside [0, n], 2 = a walk longer than n
+    unsigned long long* lf_steps; unsigned long long* iters;   // += LF steps, += warp iterations (x 32 = lane slots); nullptr = not counted
+};
+void launch_sa_resolve_batch(const SaResolveParams& p, const DevIndex& ix, const DevOpts& o, cudaStream_t st, uint64_t* launches);
+// positions of the rows pos[0 .. *total), in place (ix.sa holds the samples of a compact index); nothing when *total > cap
+void launch_sa_resolve(const DevIndex& ix, uint64_t* pos, const uint64_t* total, uint64_t cap, uint32_t* ticket, uint32_t* err,
+                       unsigned long long* lf_steps, unsigned long long* iters, cudaStream_t st);
 
 // Result of one ksw_extend2 call computed ahead of sw_extend by the thread-per-extension kernels (extend_plan.cu).  sw_extend
 // uses `out` only when the parameters of the call it is about to make equal the recorded ones (the call is a pure function

@@ -46,7 +46,8 @@ template <class IdxT> struct Ctx {
     const uint4* kmer_tab;   // prefix table (x0, x1, x2, -) of all t-mers, t <= kk; nullptr when absent
     int kk;                  // depth of the prefix table
     int lane;                // the thread's lane, read from the special register ONCE (the compiler otherwise re-issues S2R in hot loops)
-    // unique-match shortcut: full SA, inverse SA and the 2-bit text; isa == nullptr disables it
+    // unique-match shortcut: full SA, inverse SA and the 2-bit text; isa == nullptr disables it and pass 3's speculative walk (a compact
+    // index has neither a full SA nor an inverse one)
     const IdxT* sa; const IdxT* isa; const uint8_t* pac; IdxT l_pac, n;
     IdxT primary;
     uint32_t sym_base;       // first symbol covered by this lane's word (symbol lanes), 1 << 20 for checkpoint lanes
@@ -529,7 +530,7 @@ __device__ __forceinline__ void collect_intv(const Ctx<IdxT>& C, const DevOpts& 
         // evaluates f(x + t L) on its own -- K-mer from the prefix table, then (unique K-mer) one text comparison of the
         // remaining L - K bases -- so the dependent loads of up to 32 starts are in flight together; the chain then consumes
         // the results in order for as long as each start is the predicted one and was decidable without Occ.
-        const bool spec_ok = C.kmer_tab != nullptr && pk != nullptr && !has_n &&
+        const bool spec_ok = C.kmer_tab != nullptr && C.isa != nullptr && pk != nullptr && !has_n &&
                              min_len >= C.kk && o.max_mem_intv > 1 && L <= 32;
         const int lane = C.lane;
         while (x < len) {
@@ -986,7 +987,7 @@ void launch_seed(const SeedParams& p, const DevIndex& ix, const DevOpts& o, cuda
 // The thread-per-read pass takes a batch when the prefix table (and with it the inverse SA) exists, seeds are longer than the table
 // is deep (so that an emitted match always carries its rows) and the reads fit its packed shared-memory copy and 9-bit sort key.
 bool seed_thread_usable(const SeedParams& p, const DevOpts& o, uint32_t max_len) {
-    return p.kmer_tab && p.todo && p.pk && o.min_seed_len > p.kmer_k && o.max_mem_intv > 1 && max_len <= 496 && p.cap / 2 >= 16 && p.cap / 2 <= 64;
+    return p.kmer_tab && p.isa && p.todo && p.pk && o.min_seed_len > p.kmer_k && o.max_mem_intv > 1 && max_len <= 496 && p.cap / 2 >= 16 && p.cap / 2 <= 64;
 }
 
 int seed_thread_words(uint32_t max_len) { return (int)(max_len >> 4) + 3; }

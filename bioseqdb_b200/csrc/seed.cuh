@@ -30,7 +30,8 @@ struct SeedParams {
     // extensions after passes 1 and 2
     uint32_t* pk; uint32_t* rflag; uint32_t* cnt12; uint32_t* ext12;
 };
-// thread-per-read pass: runs before launch_seed when seed_thread_usable(); appends the reads it declines to p.todo
+// thread-per-read pass: runs before launch_seed when seed_thread_usable() (it needs the inverse SA and the prefix table); appends the
+// reads it declines to p.todo
 bool seed_thread_usable(const SeedParams& p, const DevOpts& o, uint32_t max_len);
 int seed_thread_words(uint32_t max_len);
 int launch_seed_thread(const SeedParams& p, const DevIndex& ix, const DevOpts& o, uint32_t max_len, uint32_t* ticket, cudaStream_t st);

@@ -67,6 +67,18 @@ uint64_t BwaIndex::device_bytes() const {
     return b;
 }
 
+bool BwaIndex::compact() const {
+    bsq_index_meta m;
+    if (bsq_index_get_meta(index, &m) != BSQ_OK) fail();
+    return m.sa_interval == 32;
+}
+
+uint32_t BwaIndex::last_notes() const {
+    bsq_timing t;
+    if (bsq_last_timing(index, &t) != BSQ_OK) fail();
+    return t.notes;
+}
+
 // ---- BwaIndexCache
 static inline uint64_t mix64(uint64_t h, uint64_t v) {          // splitmix-style accumulate
     h ^= v + 0x9E3779B97F4A7C15ULL + (h << 6) + (h >> 2);
@@ -236,6 +248,13 @@ BwaMultiIndex::BwaMultiIndex(BwaIndex& ix_, const std::vector<int>& devices) : i
 }
 
 BwaMultiIndex::~BwaMultiIndex() { bsq_multi_free(multi); }
+
+uint32_t BwaMultiIndex::last_notes() const {
+    if (!multi) return 0;
+    bsq_timing t;
+    if (bsq_multi_last_timing(multi, &t) != BSQ_OK) fail();
+    return t.notes;
+}
 
 std::vector<std::vector<BwaMatch>> BwaMultiIndex::align_sequences(const std::vector<const NucleotideSequence*>& seqs) {
     if (!multi || seqs.empty()) return std::vector<std::vector<BwaMatch>>(seqs.size());

@@ -80,6 +80,10 @@ public:
     bsq_opts options;            // written by bwa_index_from_query before build()
     size_t ref_count() const { return offsets.size(); }
     uint64_t device_bytes() const;           // bsq_index_device_bytes
+    // true when the index keeps 1/32 of its suffix array only (bsq_index_meta.sa_interval == 32): the library compacts an index by
+    // itself when the full layout does not fit in device memory; rows are the same either way
+    bool compact() const;
+    uint32_t last_notes() const;             // BSQ_NOTE_* bits of the last alignment call (bsq_last_timing)
     uint64_t& session_lrand_state() { return lrand_state; }
 
 private:
@@ -110,6 +114,7 @@ public:
     std::vector<std::vector<BwaMatch>> align_sequences(const std::vector<const NucleotideSequence*>& seqs);
     // each device materialises the tuples of its own block from HBM (bsq_multi_result_tuples)
     BwaTupleBatch align_sequences_tuples(const std::vector<const NucleotideSequence*>& seqs, uint32_t flags = 0);
+    uint32_t last_notes() const;             // BSQ_NOTE_* bits of any device in the last call (bsq_multi_last_timing)
 
 private:
     BwaIndex& ix;

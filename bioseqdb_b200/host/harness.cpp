@@ -112,6 +112,9 @@ int main(int argc, char** argv) {
         for (auto& q : queries) ptrs.push_back(&q);
         const uint64_t ids_at = bwa.session_lrand_state();
         auto all = multi ? multi->align_sequences(ptrs) : bwa.align_sequences(ptrs);
+        // the layout of the built index (replicas start in it; a replica that compacts later says so in the multi call's notes)
+        const uint32_t notes = multi ? multi->last_notes() : bwa.last_notes();
+        fprintf(stderr, "index: layout=%s sa_compacted=%d\n", bwa.compact() ? "compact" : "full", (notes & BSQ_NOTE_SA_COMPACTED) ? 1 : 0);
         auto datum_of = [](const NucleotideSequence& s) {   // the datum as PostgreSQL stores it: length word + varlena payload
             std::vector<uint8_t> pl = s.varlena_payload();
             std::vector<uint8_t> d(4 + pl.size());

@@ -70,6 +70,8 @@ typedef struct bsq_result {
 /* per-stage device timings of the last bsq_align_batch / bsq_align_resident call, milliseconds */
 #define BSQ_NOTE_CHUNK_FALLBACK 1u /* bsq_align_batch: the result outgrew the chunk pipeline's estimate, the batch was re-run in one pass */
 #define BSQ_NOTE_TABLE_DOWNGRADED 2u /* device memory was short for the batch pools: the seeding prefix table gave up its deepest level */
+#define BSQ_NOTE_SA_COMPACTED 4u     /* device memory was short for the inverse SA or the batch pools: the index now keeps every 32nd SA entry
+                                      * only (bsq_index_meta.sa_interval = 32) and resolves positions by LF walks; rows are unchanged */
 typedef struct bsq_timing {
     float h2d, seed, chain, extend, finalize, d2h, total;
     uint32_t notes;    /* BSQ_NOTE_* bits: things a successful call wants its caller to know (never an error; see bsq_last_error for those) */
@@ -169,6 +171,11 @@ typedef struct bsq_index_meta {
     int64_t l_pac; uint64_t seq_len, primary, L2[5]; uint64_t n_anns; uint32_t sa_bytes; /* 4 or 8 per SA entry */
     uint32_t built; uint64_t arr_bytes[BSQ_ARR_COUNT]; double build_ms; uint64_t build_launches;
     uint64_t sort_pass_bytes; /* algorithmic bytes moved by the radix passes of the build */
+    /* 1: the full suffix array is resident (arr_bytes[BSQ_ARR_SA] = (seq_len + 1) * sa_bytes).  32: compact -- only SA[0], SA[32], ...
+     * ((seq_len + 32) / 32 entries of sa_bytes, entry 0 = seq_len) are held, and there is no inverse SA.  The library compacts an index
+     * by itself when the full layout cannot be allocated (BSQ_NOTE_SA_COMPACTED); it is never undone.  Rows are the same either way. */
+    uint32_t sa_interval;
+    uint32_t reserved;
 } bsq_index_meta;
 int bsq_index_get_meta(const bsq_index* h, bsq_index_meta* m);
 /* Device memory held by the index right now: pac / occ / sa / ann, the derived arrays of the seeding kernel (inverse SA,
@@ -193,7 +200,9 @@ int bsq_index_prepare(bsq_index* h, float* ms);   /* build the per-device derive
  * partial file).  key: 16 opaque bytes stored in the header (the index cache passes its digest), or NULL. */
 int bsq_index_save(bsq_index* h, const char* path, const uint8_t* key);
 /* Fills a FRESH handle (bsq_index_new, nothing added, not built) from a file written by bsq_index_save: header and sizes checked on the
- * host, sections uploaded and checksummed on the device, full SA rebuilt from its samples, host mirrors restored.  key != NULL: the
+ * host, sections uploaded and checksummed on the device, full SA rebuilt from its samples, host mirrors restored.  When the full SA
+ * cannot be allocated, the index is loaded compact (sa_interval = 32): the samples are kept as they are, after a device check that
+ * every one is <= seq_len and sample 0 == seq_len.  A compact index saves the same file it was loaded from.  key != NULL: the
  * file's key must match.  *ms = wall time of the call.  Options and flags are the handle's, as for any index.  On failure the handle is
  * left fresh. */
 int bsq_index_load(bsq_index* h, const char* path, const uint8_t* key, float* ms);
@@ -202,7 +211,7 @@ typedef struct bsq_index_load_info {
     uint64_t file_bytes;
     float read_ms;       /* wall: file read + upload of every section through the pinned staging buffers */
     float checksum_ms;   /* device: k_section_checksum over the uploaded sections */
-    float sa_ms;         /* device: k_sa_from_samples */
+    float sa_ms;         /* device: k_sa_from_samples (compact load: the check and narrowing of the samples) */
     float host_ms;       /* wall: host mirrors (pac, annotations, holes) restored */
     float total_ms;      /* wall: the whole call */
     uint64_t lf_steps;   /* LF steps of the suffix-array rebuild (seq_len + 1 for a sound file) */
@@ -220,7 +229,8 @@ void bsq_multi_free(bsq_multi* m);
 int bsq_multi_devices(const bsq_multi* m);
 int bsq_multi_align_batch(bsq_multi* m, const char* seqs, const uint64_t* offs, const int64_t* ids, uint64_t n, bsq_result** out);
 int bsq_multi_align_batch_datums(bsq_multi* m, const uint8_t* bytes, const uint64_t* off, const int64_t* ids, uint64_t n, bsq_result** out);
-int bsq_multi_last_timing(const bsq_multi* m, bsq_timing* t);   /* total = the slowest device's time from its first copy to the end of its download */
+int bsq_multi_last_timing(const bsq_multi* m, bsq_timing* t);   /* total = the slowest device's time from its first copy to the end of its download;
+                                                                 * notes = the BSQ_NOTE_* bits of every device */
 /* Row materialisation of a result on every device of `m`: the same tuples, byte for byte, as bsq_result_tuples(built, res, seqs, offs,
  * flags, ...), in one pinned block with the rows in read order, freed by bsq_tuples_free.  The reads are cut into the blocks of
  * bsq_multi_align_batch* (block d = reads [n d / D, n (d + 1) / D)) and device d builds the rows of block d.  A device whose batch still
@@ -233,7 +243,10 @@ int bsq_multi_result_tuples(bsq_multi* m, const bsq_result* res, const char* seq
  * kernels: SA is a permutation of 0..n (sum / sum of squares over all rows), adjacent suffixes are in order (text comparison), the BWT
  * string is T[SA[k]-1], bwt_invPsi(k) = L2[c] + occ(k, c) lands on the row of SA[k]-1 (what bwt_sa / bwt_extend rely on, libbwa bwt.c
  * behind reference bwa.cpp:149), the Occ checkpoints equal a recount of the blocks, L2 equals the symbol counts of the text.  Rows and
- * blocks are sampled (n_samples draws of each) unless n_samples covers them all.  Every *_bad must be 0 and *_ok 1 for a sound index. */
+ * blocks are sampled (n_samples draws of each) unless n_samples covers them all.  Every *_bad must be 0 and *_ok 1 for a sound index.
+ * On a compact index (sa_interval 32) the checks that need the full SA are not run: sa_permutation_ok and exhaustive are 0 and lf_bad
+ * stays 0; sa_out_of_range counts samples > seq_len, order_* compares the suffixes of consecutive samples, rows_checked / bwt_bad check
+ * the BWT symbol of sampled rows; Occ and L2 are checked as for a full index. */
 typedef struct bsq_index_check {
     uint64_t rows;                 /* n + 1 */
     uint64_t exhaustive;           /* 1: every row and block was checked */
@@ -251,6 +264,9 @@ int bsq_index_sa_sampled(const bsq_index* h, uint64_t* out, uint64_t n_sa); /* b
 /* Stage dumps for parity tests (device results copied to host): SMEM intervals after mem_collect_intv,
  * one record = 4 x u64 {x0,x1,x2,info}; cnt[n] = intervals per read, cap = records per read in `out`. */
 int bsq_debug_seed(bsq_index* h, const char* seqs, const uint64_t* offs, uint64_t n, uint64_t* out, uint32_t cap, uint32_t* cnt);
+/* out[i] = bwt_sa(rows[i]) for rows in [0, seq_len] (row 0 gives seq_len): SA[row] on a full index, the LF walk of the alignment
+ * pipeline's position resolve pass on a compact one.  n < 2^31. */
+int bsq_debug_sa_lookup(bsq_index* h, const uint64_t* rows, uint64_t n, uint64_t* out);
 /* Kernel-level entry points for parity tests of the DP kernels on explicit job lists.
  * ext jobs: query/target are nt4 bytes; out = 6 x int32 per job {score,qle,tle,gtle,gscore,max_off}. */
 int bsq_debug_ksw_extend(const bsq_opts* o, int device, uint64_t n_jobs, const uint8_t* q, const uint64_t* q_off, const uint8_t* t,
